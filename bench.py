@@ -25,6 +25,8 @@ src/dpg_slam/dpg_slam.cc:362-446) over one batch of synthetic Hokuyo-like scan p
   checks     in the run: records of the e2e arm == resident arm; the gathered buffer holds every rank's records;
              rank 0 re-aligns a strided sample of the GLOBAL batch on its one GPU and compares with the gathered
              records bit for bit (1 GPU == N GPUs); a strided sample equals the CPU oracle bit for bit.
+  outputs    --dump-outputs DIR (one GPU): the records of the last timed step, one DIR/<field>.npy per record field plus
+             index.npy (their positions in the batch); inputs are seeded, so two builds can be compared output for output.
 
 `--impl reference` times the reference's CPU algorithm on the host cores (the oracle port, oracle/dpg_oracle.c,
 OpenMP over pairs): PCL itself cannot be built in this image (DESIGN.md).
@@ -252,6 +254,31 @@ def algorithmic_flops(rec, counts_s, counts_t, sum_corr):
     icp = float(np.sum(it * (5.0 * ns * nt + 8.0 * ns)) + 14.0 * sum_corr)
     cov = float(np.sum(60.0 * k_last + 45.0 * np.minimum(k_last, 200.0)))
     return icp, cov
+
+
+DUMP_BUDGET_BYTES = 60_000_000         # under 64 MB with the .npy headers
+DUMP_FIELDS = (("tx", np.float32), ("ty", np.float32), ("theta", np.float32), ("rot_c", np.float32), ("rot_s", np.float32),
+               ("iterations", np.float64), ("status", np.float64), ("n_correspondences", np.float64),    # integers, exact in f64
+               ("mse", np.float64), ("cov", np.float64))
+DUMP_RECORD_BYTES = 8 + sum(np.dtype(t).itemsize * (9 if f == "cov" else 1) for f, t in DUMP_FIELDS)     # + the index
+
+
+def dump_sample(n_records: int) -> np.ndarray:
+    """Sorted indices of the records --dump-outputs writes: all of them when they fit the budget, else a fixed seeded
+    sample (the same for every run with the same arguments)."""
+    k = DUMP_BUDGET_BYTES // DUMP_RECORD_BYTES
+    if n_records <= k:
+        return np.arange(n_records, dtype=np.int64)
+    return np.sort(np.random.default_rng(0).choice(n_records, size=k, replace=False)).astype(np.int64)
+
+
+def dump_records(out_dir: str, rec, index) -> None:
+    """The records a caller of the timed path receives, one float32/float64 array per field: <out_dir>/<field>.npy, plus
+    index.npy, the position of each dumped record in the batch."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "index.npy"), np.asarray(index, np.float64))
+    for f, t in DUMP_FIELDS:
+        np.save(os.path.join(out_dir, f"{f}.npy"), np.ascontiguousarray(rec[f], dtype=t))
 
 
 def load_peaks():
@@ -723,6 +750,9 @@ def run_product_host_list(args):
                             "corridor_reference_default_params": ref_defaults}
         if world == 1 and rank == 0 and not args.no_latency:
             line["latency"] = latency_block(sm)                  # last: it replaces the scan store
+    if args.dump_outputs:                                        # one GPU: rec_local is the whole batch of the last timed step
+        keep = dump_sample(len(rec_local))
+        dump_records(args.dump_outputs, rec_local[keep], keep)
     if rank == 0:
         print(json.dumps(line), flush=True)
     cx.close()
@@ -839,7 +869,8 @@ def run_product_multisession(args):
         CH = 1 << 20
         pin = torch.empty(CH * sharded.RECORD_BYTES, dtype=torch.uint8).pin_memory()
 
-        def stream_records(fetch, n):
+        def stream_records(fetch, n, keep=None, kept=None):
+            """keep: sorted record indices to copy into the list kept"""
             it_sum, conv, it_max = 0.0, 0, 0
             for a in range(0, n, CH):
                 c = min(CH, n - a)
@@ -847,9 +878,14 @@ def run_product_multisession(args):
                 rec = np.frombuffer(pin.numpy(), dtype=sharded.RESULT_DTYPE, count=c)
                 it_sum += float(rec["iterations"].sum()); conv += int(((rec["status"] & FLAG_CONVERGED) != 0).sum())
                 it_max = max(it_max, int(rec["iterations"].max()))
+                if keep is not None:
+                    kept.append(rec[keep[np.searchsorted(keep, a):np.searchsorted(keep, a + c)] - a].copy())
             return it_sum, conv, it_max
 
-        it_sum, conv, it_max = stream_records(lambda a, c, ptr: sm.fetch_results_range(a, c, host_ptr=ptr), n_local)
+        keep, kept = (dump_sample(n_local), []) if args.dump_outputs else (None, None)
+        it_sum, conv, it_max = stream_records(lambda a, c, ptr: sm.fetch_results_range(a, c, host_ptr=ptr), n_local, keep, kept)
+        if args.dump_outputs:                     # one GPU: this rank's list is the whole batch of the last timed step
+            dump_records(args.dump_outputs, np.concatenate(kept), keep)
 
         # ---------------- end-to-end: node table H2D + enumeration on the device + ICP/cov + gather + records D2H ----------------
         e2e_steps = 1
@@ -970,7 +1006,15 @@ def main():
     ap.add_argument("--pairs", type=int, default=0, help="override the workload's pair count (per GPU for weak, global for strong scaling)")
     ap.add_argument("--scans-per-session", type=int, default=0, help="multisession: scans per session (default 50000)")
     ap.add_argument("--world-m", type=float, default=100.0, help="multisession: side of the square world in metres")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the records of the last step as DIR/<field>.npy (float32/float64; a "
+                         "fixed seeded sample when the batch exceeds 64 MB), so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "product" or args.gpus != 1):
+        # the reference arm times a sample of pairs sized by a timing pilot: its outputs are not comparable run to run
+        ap.error("--dump-outputs needs --impl product and --gpus 1")
     if args.impl == "reference":
         return run_reference(args)
     if args.workload == "multisession":
