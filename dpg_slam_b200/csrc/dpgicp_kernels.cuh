@@ -982,8 +982,9 @@ __device__ __forceinline__ void accumulate_pair(const SmemLayout &L, const KP &P
  * squared distances L.ad2[0 .. n_pad) (+inf = not accepted).  Exact block-wide radix select: four rounds of 8 bits over
  * the binary32 patterns (d2 >= +0, so the patterns order like the values), a 256-bin histogram in shared memory per
  * round.  Every thread of the CTA calls it between two __syncthreads-separated phases; all get the same tau
- * (+inf when fewer than 3 pairs were accepted: the pass stops anyway).  Scratch: L.dpart (free between the passes'
- * reductions) and L.ctl[5..7].
+ * (+inf only when no pair was accepted).  With 1 or 2 accepted pairs the rule still applies, as in the oracle and
+ * DESIGN §5.8: the pass then stops on K < 3 either way, but the kept set is what the parity hook returns and the
+ * record's n_correspondences counts.  Scratch: L.dpart (free between the passes' reductions) and L.ctl[5..7].
  * ---------------------------------------------------------------------------------------------- */
 __device__ __forceinline__ float select_tau(const SmemLayout &L, int n_pad, int mode, double param) {
   const float inf = __int_as_float(0x7f800000);
@@ -998,7 +999,7 @@ __device__ __forceinline__ float select_tau(const SmemLayout &L, int n_pad, int 
   if (lane == 0 && c) atomicAdd(&sel[0], c);
   __syncthreads();
   const int K = sel[0];
-  if (K < 3) return inf;
+  if (K < 1) return inf;
   int r;
   if (mode == DPGICP_OUTLIER_TRIMMED) {
     int keep = (int)floor(__dmul_rn(param, (double)K));

@@ -75,8 +75,21 @@ def test_sticky_rule_over_whole_runs_with_ties(gpu_matcher):
 
 
 # ---- outlier rejection ---------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("mode,param", [(OUTLIER_TRIMMED, 0.7), (OUTLIER_TRIMMED, 1.0), (OUTLIER_MEDIAN, 1.5), (OUTLIER_MEDIAN, 0.8)])
-def test_outlier_rejection_correspondences_bit_exact(gpu_matcher, mode, param):
+@pytest.mark.parametrize("mode,param,k_small", [(OUTLIER_TRIMMED, 0.7, None), (OUTLIER_TRIMMED, 1.0, None), (OUTLIER_MEDIAN, 1.5, None),
+                                                (OUTLIER_MEDIAN, 0.8, None), (OUTLIER_MEDIAN, 0.5, 1), (OUTLIER_MEDIAN, 0.5, 2)],
+                         ids=["1-0.7", "1-1.0", "2-1.5", "2-0.8", "2-0.5-K1", "2-0.5-K2"])
+def test_outlier_rejection_correspondences_bit_exact(gpu_matcher, mode, param, k_small):
+    if k_small:
+        # 3 target points, k_small accepted pairs: MEDIAN 0.5 keeps fewer than all of them (1 of 2, 0 of 1)
+        tgt = np.array([[0.0, 0.0], [0.0, 1.5], [0.0, 3.0]], np.float32)
+        src = (tgt[:k_small] + np.array([0.1, 0.0], np.float32) * np.arange(1, k_small + 1, dtype=np.float32)[:, None]).astype(np.float32)
+        Tm = np.array([1, 0, 0, 0], np.float32)
+        for search in (SEARCH_BRUTE, SEARCH_PRUNED, SEARCH_PROJECTIVE):
+            p = Params.defaults(downsample_divisor=1, search=search, outlier_mode=mode, outlier_param=param)
+            kk, want, _ = O.correspondences(src, tgt, p, src_orig=src, T=Tm)
+            got, _ = gpu_matcher.correspondences(src, tgt, Tm, p)
+            assert kk == k_small - 1 and np.array_equal(got, want), (search, got, want)
+        return
     wl = synth.config_corridor(n_pairs=6, seed=21)
     pts, off = O.clouds_from_ranges(wl.ranges, wl.scanner)
     for search in (SEARCH_BRUTE, SEARCH_PRUNED, SEARCH_PROJECTIVE):
