@@ -92,6 +92,11 @@ extern "C" {
 #define DPGICP_COV_REFERENCE_LIVE  0     /* diag(sx2, sy2, st2): cov_func_point_to_point.h:572-575 */
 #define DPGICP_COV_CENSI_INDEXPAIR 1     /* intended formula, clouds paired by index as dpg_slam.cc:430 */
 #define DPGICP_COV_CENSI_CORR      2     /* intended formula on the final ICP correspondences    */
+/* CENSI_CORR pair set: one correspondence pass at the FINAL pose (down-sampled source moved by the final transform),
+ * seeded with the last ICP pass's forward neighbours, then the reciprocal test and the outlier rejector (if any).  The
+ * kept pairs in source-index order, p = the untransformed down-sampled source point: the Hessian runs over all of them,
+ * the D-term over the first cov_cap (all when cov_cap = 0).  CENSI_INDEXPAIR: the full clouds paired by index,
+ * n_h = min(n_source, n_target), the D-term over the first min(n_h, cov_cap). */
 
 /* result.status: low byte = stop reason, higher bits = flags */
 #define DPGICP_STOP_MASK              0xffu
