@@ -14,7 +14,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 
 # ---- constants (include/dpgicp.h) -----------------------------------------------------------------
-ABI_VERSION = 3
+ABI_VERSION = 4
 METRIC_POINT_TO_POINT, METRIC_POINT_TO_LINE = 0, 1
 SEARCH_BRUTE, SEARCH_PRUNED, SEARCH_PROJECTIVE = 0, 1, 2
 COV_REFERENCE_LIVE, COV_CENSI_INDEXPAIR, COV_CENSI_CORR = 0, 1, 2
@@ -117,7 +117,7 @@ EXPORTS = [
     "dpgicp_correspondences_seeded", "dpgicp_set_nodes", "dpgicp_enumerate_pairs_device", "dpgicp_fetch_pairs",
     "dpgicp_convert_ranges_device", "dpgicp_gather_attach_local", "dpgicp_gather_set_root_only",
     "dpgicp_enable_stage_timing", "dpgicp_last_run_stage_ms", "dpgicp_run_range", "dpgicp_fetch_results_range",
-    "dpgicp_gather_fetch_range", "dpgicp_gather_declare",
+    "dpgicp_gather_fetch_range", "dpgicp_gather_declare", "dpgicp_append_ranges", "dpgicp_append_scans",
 ]
 
 _lib = None
@@ -152,6 +152,8 @@ def load_library() -> C.CDLL:
         "dpgicp_upload_scans": (C.c_int, [vp, vp, sz, vp, i32]),
         "dpgicp_upload_ranges": (C.c_int, [vp, vp, i32, i32] + [C.c_float] * 6),
         "dpgicp_upload_ranges_subset": (C.c_int, [vp, vp, i32, i32, vp, i32] + [C.c_float] * 6),
+        "dpgicp_append_ranges": (C.c_int, [vp, vp, i32, i32] + [C.c_float] * 6),
+        "dpgicp_append_scans": (C.c_int, [vp, vp, sz, vp, i32]),
         "dpgicp_scan_count": (C.c_int, [vp]),
         "dpgicp_download_scan": (C.c_int, [vp, i32, vp, C.POINTER(i32)]),
         "dpgicp_submit_pairs": (C.c_int, [vp, vp, vp, vp, i64, PP, vp]),

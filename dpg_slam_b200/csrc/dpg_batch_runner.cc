@@ -19,13 +19,18 @@
  * its round-robin shard kept, records gathered into device a's buffer by peer stores.  The CSV is identical for any N.
  * --caller online enumerates the pairs of one updatePoseGraphObsConstraints call for the newest node instead of a
  * whole reoptimize().
+ * --replay runs the reference's online loop instead of one batch (replay() below): every log scan becomes a node, is
+ * appended to the scan store and aligned with its predecessor and its loop-closure candidates; a reoptimize() runs at
+ * every pass boundary.  The CSV gains a leading column `update` (k, or reopt@k); the JSON line reports per-update times.
  */
+#include <algorithm>
 #include <chrono>
 #include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <stdexcept>
 #include <string>
 #include <vector>
 
@@ -152,6 +157,91 @@ void make_synthetic(const std::string &kind, int n_scans, int n_beams, int passe
   }
 }
 
+double percentile(std::vector<double> v, double q) {      /* nearest rank */
+  if (v.empty()) return 0.0;
+  std::sort(v.begin(), v.end());
+  return v[(size_t)std::lround(q * (double)(v.size() - 1))];
+}
+
+/* The reference's runtime shape, node by node (the data runner feeds scans one at a time, runner.cc:95-128):
+ *   for k = 0 .. n-1:
+ *     if k > 0 and pass[k] != pass[k-1]:   reoptimize() over nodes 0..k-1   (incrementPassNumber, slam.cc:25-33)
+ *     append scan k                        (createNode, dpg_slam.cc:462-513)
+ *     if k >= 1: pairs of node k           (updatePoseGraphObsConstraints, dpg_slam.cc:255-314)
+ * Each alignment batch is set_nodes -> enumerate on the device -> run -> records + factors back (the hand-off to
+ * addObservationConstraint).  Node estimates are the log's; a pose-graph optimiser would update them in between. */
+int replay(const ScanLog &L, const dpgicp_params &params, float r_same, float r_other, int device, const std::string &csv_out) {
+  dpgicp_shim::ScanMatcher sm(device);
+  dpgicp_ctx *ctx = sm.ctx();
+  auto check = [&](int rc, const char *what) {
+    if (rc != DPGICP_OK) throw std::runtime_error(std::string(what) + ": " + dpgicp_last_error(ctx));
+  };
+  std::vector<float> pose((size_t)L.n_scans * 3);
+  for (int s = 0; s < L.n_scans; ++s) {
+    pose[3 * (size_t)s] = L.est[(size_t)s].x; pose[3 * (size_t)s + 1] = L.est[(size_t)s].y; pose[3 * (size_t)s + 2] = L.est[(size_t)s].theta;
+  }
+  struct Row { int update; bool reopt; dpgicp_factor fac; dpgicp_result rec; };
+  std::vector<Row> rows;
+  std::vector<dpgicp_result> rec;
+  std::vector<dpgicp_factor> fac;
+  std::vector<double> t_append, t_nodes, t_erf, t_total;
+  int n_online = 0, n_reopt = 0;
+  size_t online_pairs = 0;
+  /* one alignment batch over nodes 0..n_nodes-1; returns the set_nodes and the enumerate + run + fetch times */
+  auto align = [&](int n_nodes, int mode, int update, double *dt_nodes, double *dt_erf) {
+    const double t0 = now_s();
+    check(dpgicp_set_nodes(ctx, pose.data(), L.pass.data(), n_nodes), "dpgicp_set_nodes");
+    const double t1 = now_s();
+    int64_t n = 0;
+    check(dpgicp_enumerate_pairs_device(ctx, mode, r_same, r_other, 0, 1, &n, nullptr), "dpgicp_enumerate_pairs_device");
+    check(dpgicp_run(ctx, &params), "dpgicp_run");
+    rec.resize((size_t)n); fac.resize((size_t)n);
+    check(dpgicp_fetch_results(ctx, rec.data(), n), "dpgicp_fetch_results");
+    check(dpgicp_fetch_factors(ctx, fac.data(), n), "dpgicp_fetch_factors");
+    const double t2 = now_s();
+    *dt_nodes = t1 - t0; *dt_erf = t2 - t1;
+    for (int64_t k = 0; k < n; ++k) rows.push_back({update, mode == DPGICP_ENUM_REOPTIMIZE, fac[(size_t)k], rec[(size_t)k]});
+    return (size_t)n;
+  };
+  const double t_start = now_s();
+  for (int k = 0; k < L.n_scans; ++k) {
+    double dn, de;
+    if (k > 0 && L.pass[(size_t)k] != L.pass[(size_t)k - 1]) { align(k, DPGICP_ENUM_REOPTIMIZE, k, &dn, &de); ++n_reopt; }
+    const double a0 = now_s();
+    sm.appendRanges(&L.ranges[(size_t)k * (size_t)L.n_beams], 1, L.n_beams, L.angle_min, L.angle_max, L.range_max, L.lx, L.ly, L.lt);
+    const double a1 = now_s();
+    if (k >= 1) {
+      online_pairs += align(k + 1, DPGICP_ENUM_ONLINE, k, &dn, &de);
+      t_append.push_back(a1 - a0); t_nodes.push_back(dn); t_erf.push_back(de); t_total.push_back(a1 - a0 + dn + de);
+      ++n_online;
+    }
+  }
+  const double replay_s = now_s() - t_start;
+  if (!csv_out.empty()) {
+    FILE *f = std::fopen(csv_out.c_str(), "w");
+    if (!f) { std::fprintf(stderr, "cannot write %s\n", csv_out.c_str()); return 1; }
+    std::fprintf(f, "update,src,tgt,tx,ty,theta,c00,c01,c02,c10,c11,c12,c20,c21,c22,iterations,status\n");
+    for (const Row &w : rows) {
+      const dpgicp_result &r = w.rec;
+      std::fprintf(f, w.reopt ? "reopt@%d," : "%d,", w.update);
+      std::fprintf(f, "%d,%d,%.9g,%.9g,%.9g", w.fac.to_node, w.fac.from_node, r.tx, r.ty, r.theta);
+      for (int c = 0; c < 9; ++c) std::fprintf(f, ",%.17g", r.cov[c]);
+      std::fprintf(f, ",%d,%u\n", r.iterations, r.status);
+    }
+    std::fclose(f);
+  }
+  auto ms = [](const std::vector<double> &v, double q) { return 1e3 * percentile(v, q); };
+  std::printf("{\"mode\": \"replay\", \"scans\": %d, \"beams\": %d, \"online_updates\": %d, \"reoptimize_batches\": %d, "
+              "\"pairs\": %zu, \"online_pairs\": %zu, "
+              "\"update_ms_median\": {\"append\": %.4f, \"set_nodes\": %.4f, \"enumerate_run_fetch\": %.4f, \"total\": %.4f}, "
+              "\"update_ms_p90\": {\"append\": %.4f, \"set_nodes\": %.4f, \"enumerate_run_fetch\": %.4f, \"total\": %.4f}, "
+              "\"replay_s\": %.6f}\n",
+              L.n_scans, L.n_beams, n_online, n_reopt, rows.size(), online_pairs,
+              ms(t_append, 0.5), ms(t_nodes, 0.5), ms(t_erf, 0.5), ms(t_total, 0.5),
+              ms(t_append, 0.9), ms(t_nodes, 0.9), ms(t_erf, 0.9), ms(t_total, 0.9), replay_s);
+  return 0;
+}
+
 }  // namespace
 
 int main(int argc, char **argv) {
@@ -159,7 +249,7 @@ int main(int argc, char **argv) {
   int n_scans = 501, n_beams = 1081, passes = 1, device = 0;
   std::vector<int> devices;
   int32_t caller = DPGICP_ENUM_REOPTIMIZE;
-  bool successive_only = false;
+  bool successive_only = false, replay_log = false;
   uint64_t seed = 2;
   dpgicp_params params;
   dpgicp_default_params(&params);
@@ -195,12 +285,14 @@ int main(int argc, char **argv) {
     else if (a == "--same-pass-radius") r_same = (float)std::atof(next("--same-pass-radius"));
     else if (a == "--other-pass-radius") r_other = (float)std::atof(next("--other-pass-radius"));
     else if (a == "--successive-only") successive_only = true;
+    else if (a == "--replay") replay_log = true;
     else {
       std::fprintf(stderr,
                    "usage: dpg_batch_runner [--synthetic corridor|office | --log FILE] [--scans N] [--beams N] [--passes N]\n"
                    "         [--seed S] [--divisor D] [--cov-mode 0|1|2] [--metric 0|1] [--search 0|1|2] [--window W] [--successive-only]\n"
                    "         [--same-pass-radius R] [--other-pass-radius R] [--write-log FILE] [--out FILE.csv] [--device K]\n"
-                   "         [--gpus N | --devices a,b,...] [--caller reoptimize|online] [--outlier-mode 0|1|2 --outlier-param X]\n");
+                   "         [--gpus N | --devices a,b,...] [--caller reoptimize|online] [--outlier-mode 0|1|2 --outlier-param X]\n"
+                   "         [--replay]\n");
       return a == "--help" ? 0 : 2;
     }
   }
@@ -213,7 +305,14 @@ int main(int argc, char **argv) {
   }
   if (!log_out.empty() && !write_log(log_out.c_str(), L)) { std::fprintf(stderr, "cannot write %s\n", log_out.c_str()); return 1; }
 
+  if (replay_log && !devices.empty()) {
+    std::fprintf(stderr, "dpg_batch_runner: --replay runs on one device (--device K); --gpus / --devices are not supported "
+                         "with it (online batches are tens of pairs)\n");
+    return 2;
+  }
+
   try {
+    if (replay_log) return replay(L, params, r_same, r_other, device, csv_out);
     std::vector<int32_t> src, tgt;
     std::vector<dpgicp_result> res;
     double t0, t1, t2, t3;

@@ -448,8 +448,9 @@ int finish_store(dpgicp_ctx *ctx, Store &st, int n_scans) {
   return DPGICP_OK;
 }
 
-int upload_scans_into(dpgicp_ctx *ctx, Store &st, const void *points, size_t stride, const int64_t *offsets,
-                      int32_t n_scans) {
+/* arguments of a ragged cloud upload (dpgicp_upload_scans / dpgicp_append_scans): the largest scan and the point total */
+int check_clouds(dpgicp_ctx *ctx, const void *points, size_t stride, const int64_t *offsets, int32_t n_scans,
+                 int64_t *max_count, int64_t *total) {
   if (n_scans < 0 || (n_scans > 0 && (!offsets))) return fail(ctx, DPGICP_E_INVALID, "bad scan arguments");
   if (stride < 8 || (stride % 4) != 0) return fail(ctx, DPGICP_E_INVALID, "stride_bytes must be >= 8 and a multiple of 4");
   int64_t maxc = 0;
@@ -459,10 +460,18 @@ int upload_scans_into(dpgicp_ctx *ctx, Store &st, const void *points, size_t str
     maxc = std::max(maxc, c);
   }
   if (maxc > DPGICP_MAX_POINTS) return fail(ctx, DPGICP_E_TOOBIG, "a scan has more than DPGICP_MAX_POINTS points");
-  const int64_t total = n_scans > 0 ? offsets[n_scans] : 0;
-  if (total > 0 && !points) return fail(ctx, DPGICP_E_INVALID, "points is NULL");
+  *max_count = maxc;
+  *total = n_scans > 0 ? offsets[n_scans] : 0;
+  if (*total > 0 && !points) return fail(ctx, DPGICP_E_INVALID, "points is NULL");
+  return DPGICP_OK;
+}
+
+int upload_scans_into(dpgicp_ctx *ctx, Store &st, const void *points, size_t stride, const int64_t *offsets,
+                      int32_t n_scans) {
+  int64_t maxc = 0, total = 0;
+  int rc = check_clouds(ctx, points, stride, offsets, n_scans, &maxc, &total);
+  if (rc) return rc;
   const int pitch = (int)std::max<int64_t>(2, (maxc + 1) & ~(int64_t)1);
-  int rc;
   if ((rc = reserve(ctx, st.rows, sizeof(float2) * (size_t)pitch * (size_t)std::max(n_scans, 1)))) return rc;
   if ((rc = reserve(ctx, st.count, sizeof(int32_t) * (size_t)std::max(n_scans, 1)))) return rc;
   if ((rc = reserve(ctx, ctx->stage, (size_t)total * stride + 16))) return rc;
@@ -759,6 +768,87 @@ int fetch_pairs_from(dpgicp_ctx *ctx, const Batch &b, int32_t *src, int32_t *tgt
   return DPGICP_OK;
 }
 
+/* Room for n_new more rows of at least need_pitch (even) points behind the rows of the store, every existing row kept
+ * (the append path).  Rows and counts grow by doubling, so n one-scan appends copy O(n) rows in total; a scan longer
+ * than the pitch re-pitches the kept rows on the device.  A buffer that moves is freed only after the stream has
+ * drained: the copy out of it, and any dpgicp_run enqueued before the append, read it.  On failure the store is as
+ * it was. */
+int grow_store(dpgicp_ctx *ctx, Store &st, int n_new, int need_pitch) {
+  const int n_old = st.n_scans;
+  const int64_t rows = (int64_t)n_old + n_new;
+  const int pitch = n_old > 0 ? std::max(st.pitch, need_pitch) : need_pitch;
+  const size_t row_bytes = sizeof(float2) * (size_t)pitch;
+  const bool move_rows = (n_old > 0 && pitch != st.pitch) || (size_t)rows * row_bytes > st.rows.cap;
+  const bool move_count = (size_t)rows * sizeof(int32_t) > st.count.cap;
+  DevBuf nr, nc;
+  auto alloc = [&](DevBuf &b, size_t bytes) {
+    cudaError_t e = cudaMalloc(&b.p, bytes);
+    if (e != cudaSuccess) {
+      b.p = nullptr;
+      return fail(ctx, e == cudaErrorMemoryAllocation ? DPGICP_E_NOMEM : DPGICP_E_CUDA,
+                  std::string("cudaMalloc (scan store growth): ") + cudaGetErrorString(e));
+    }
+    b.cap = bytes;
+    return (int)DPGICP_OK;
+  };
+  auto cuda = [&](cudaError_t e, const char *what) {
+    return e == cudaSuccess ? (int)DPGICP_OK : fail(ctx, DPGICP_E_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
+  };
+  int rc = DPGICP_OK;
+  if (move_rows) {
+    int64_t cap = st.pitch > 0 ? (int64_t)(st.rows.cap / (sizeof(float2) * (size_t)st.pitch)) : 0;
+    if (rows > cap) cap = std::max(rows, 2 * cap);
+    rc = alloc(nr, (size_t)cap * row_bytes);
+    if (!rc && n_old > 0 && pitch == st.pitch)
+      rc = cuda(cudaMemcpyAsync(nr.p, st.rows.p, (size_t)n_old * row_bytes, cudaMemcpyDeviceToDevice, ctx->stream),
+                "cudaMemcpyAsync (scan rows)");
+    if (!rc && n_old > 0 && pitch != st.pitch) {
+      const int threads = 128, blocks = (n_old + threads / 32 - 1) / (threads / 32);
+      repitch_rows_kernel<<<blocks, threads, 0, ctx->stream>>>((const float4 *)st.rows.p, n_old, st.pitch, pitch, (float4 *)nr.p);
+      ctx->launches++;
+      rc = cuda(cudaGetLastError(), "repitch_rows_kernel");
+    }
+  }
+  if (!rc && move_count) {
+    const int64_t cap = std::max(rows, 2 * (int64_t)(st.count.cap / sizeof(int32_t)));
+    rc = alloc(nc, (size_t)cap * sizeof(int32_t));
+    if (!rc && n_old > 0)
+      rc = cuda(cudaMemcpyAsync(nc.p, st.count.p, (size_t)n_old * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream),
+                "cudaMemcpyAsync (scan counts)");
+  }
+  if (!rc && (move_rows || move_count)) rc = cuda(cudaStreamSynchronize(ctx->stream), "cudaStreamSynchronize");
+  if (rc) {
+    cudaStreamSynchronize(ctx->stream);
+    release(nr); release(nc);
+    return rc;
+  }
+  if (move_rows) { release(st.rows); st.rows = nr; }
+  if (move_count) { release(st.count); st.count = nc; }
+  st.pitch = pitch;
+  return DPGICP_OK;
+}
+
+/* the counts of the n_new rows just converted behind the store back to the host (only those) + the range flag; the
+ * store takes them only when every point is in range */
+int finish_append(dpgicp_ctx *ctx, Store &st, int n_new) {
+  const size_t first = (size_t)st.n_scans;
+  st.h_count.resize(first + (size_t)n_new);
+  int bad = 0;
+  CU_TRY(ctx, cudaMemcpyAsync(st.h_count.data() + first, (const int32_t *)st.count.p + first, sizeof(int32_t) * (size_t)n_new,
+                              cudaMemcpyDeviceToHost, ctx->stream));
+  CU_TRY(ctx, cudaMemcpyAsync(&bad, ctx->d_bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  if (bad) {
+    st.h_count.resize(first);
+    return fail(ctx, DPGICP_E_RANGE, "appended scans hold a non-finite point or |coordinate| > DPGICP_MAX_ABS_COORD; "
+                                     "the store is unchanged");
+  }
+  if (first == 0) st.max_count = 0;
+  for (size_t k = first; k < st.h_count.size(); ++k) st.max_count = std::max(st.max_count, st.h_count[k]);
+  st.n_scans = (int32_t)st.h_count.size();
+  return DPGICP_OK;
+}
+
 }  // namespace
 
 /* ================================================================================================
@@ -991,6 +1081,65 @@ int dpgicp_upload_ranges_subset(dpgicp_ctx *ctx, const float *ranges, int32_t n_
   ctx->launches++;
   CU_TRY(ctx, cudaGetLastError());
   return finish_store(ctx, st, n_ids);
+}
+
+int dpgicp_append_ranges(dpgicp_ctx *ctx, const float *ranges, int32_t n_scans, int32_t n_beams, float angle_min,
+                         float angle_max, float range_max, float lx, float ly, float ltheta) {
+  if (!ctx) return DPGICP_E_INVALID;
+  NvtxRange range("dpgicp: append ranges + scan->cloud");
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  if (n_scans < 0 || n_beams < 2 || (n_scans > 0 && !ranges)) return fail(ctx, DPGICP_E_INVALID, "bad range-scan arguments");
+  if (n_beams > DPGICP_MAX_POINTS) return fail(ctx, DPGICP_E_TOOBIG, "n_beams exceeds DPGICP_MAX_POINTS");
+  Store &st = ctx->store;
+  if ((int64_t)st.n_scans + n_scans > INT32_MAX) return fail(ctx, DPGICP_E_INVALID, "the store would hold more than 2^31 - 1 scans");
+  if (n_scans == 0) return DPGICP_OK;
+  const int first = st.n_scans;
+  int rc;
+  if ((rc = grow_store(ctx, st, n_scans, (n_beams + 1) & ~1))) return rc;
+  if ((rc = reserve(ctx, ctx->stage, sizeof(float) * (size_t)n_scans * (size_t)n_beams + 16))) return rc;
+  CU_TRY(ctx, cudaMemsetAsync(ctx->d_bad, 0, sizeof(int), ctx->stream));
+  CU_TRY(ctx, cudaMemcpyAsync(ctx->stage.p, ranges, sizeof(float) * (size_t)n_scans * (size_t)n_beams,
+                              cudaMemcpyHostToDevice, ctx->stream));
+  /* the conversion of dpgicp_upload_ranges, writing rows first .. first + n_scans - 1 */
+  const float angle_inc = (float)(((double)(float)(angle_max - angle_min)) / ((double)n_beams - 1.0));
+  const float lc = cosf(ltheta), ls = sinf(ltheta);
+  const int threads = 128, warps_per_block = threads / 32;
+  const int blocks = (n_scans + warps_per_block - 1) / warps_per_block;
+  if ((rc = ensure_trig(ctx, n_beams, angle_min, angle_inc))) return rc;
+  ranges_to_rows_kernel<<<blocks, threads, 0, ctx->stream>>>((const float *)ctx->stage.p, nullptr, n_scans, n_beams,
+                                                            (const double2 *)ctx->trig.p, range_max, lx, ly, lc, ls, st.pitch,
+                                                            (float2 *)st.rows.p + (size_t)first * st.pitch,
+                                                            (int32_t *)st.count.p + first, ctx->d_bad);
+  ctx->launches++;
+  CU_TRY(ctx, cudaGetLastError());
+  return finish_append(ctx, st, n_scans);
+}
+
+int dpgicp_append_scans(dpgicp_ctx *ctx, const void *points, size_t stride, const int64_t *offsets, int32_t n_scans) {
+  if (!ctx) return DPGICP_E_INVALID;
+  NvtxRange range("dpgicp: append clouds");
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  int64_t maxc = 0, total = 0;
+  int rc = check_clouds(ctx, points, stride, offsets, n_scans, &maxc, &total);
+  if (rc) return rc;
+  Store &st = ctx->store;
+  if ((int64_t)st.n_scans + n_scans > INT32_MAX) return fail(ctx, DPGICP_E_INVALID, "the store would hold more than 2^31 - 1 scans");
+  if (n_scans == 0) return DPGICP_OK;
+  const int first = st.n_scans;
+  if ((rc = grow_store(ctx, st, n_scans, (int)std::max<int64_t>(2, (maxc + 1) & ~(int64_t)1)))) return rc;
+  if ((rc = reserve(ctx, ctx->stage, (size_t)total * stride + 16))) return rc;
+  if ((rc = reserve(ctx, ctx->offsets, sizeof(int64_t) * ((size_t)n_scans + 1)))) return rc;
+  CU_TRY(ctx, cudaMemsetAsync(ctx->d_bad, 0, sizeof(int), ctx->stream));
+  if (total > 0)
+    CU_TRY(ctx, cudaMemcpyAsync(ctx->stage.p, points, (size_t)total * stride, cudaMemcpyHostToDevice, ctx->stream));
+  CU_TRY(ctx, cudaMemcpyAsync(ctx->offsets.p, offsets, sizeof(int64_t) * ((size_t)n_scans + 1), cudaMemcpyHostToDevice,
+                              ctx->stream));
+  pack_rows_kernel<<<n_scans, 256, 0, ctx->stream>>>((const unsigned char *)ctx->stage.p, stride, (const long long *)ctx->offsets.p,
+                                                     n_scans, st.pitch, (float2 *)st.rows.p + (size_t)first * st.pitch,
+                                                     (int32_t *)st.count.p + first, ctx->d_bad);
+  ctx->launches++;
+  CU_TRY(ctx, cudaGetLastError());
+  return finish_append(ctx, st, n_scans);
 }
 
 int dpgicp_scan_count(const dpgicp_ctx *ctx) { return ctx ? ctx->store.n_scans : DPGICP_E_INVALID; }

@@ -1768,6 +1768,19 @@ __global__ void ranges_to_rows_kernel(const float *__restrict__ ranges, const in
   if (lane == 0) count[warp] = n;
 }
 
+/* rows of pitch `old_pitch` -> rows of the larger pitch `new_pitch` (both even, so every row starts on a 16-byte
+ * boundary and is a whole number of float4 = two points).  One warp per row, 16-byte loads and stores; the old
+ * row's padding is already zero, the new tail is zero-filled: every row keeps its contents and stays zero-padded. */
+__global__ void repitch_rows_kernel(const float4 *__restrict__ src, int n_rows, int old_pitch, int new_pitch,
+                                    float4 *__restrict__ dst) {
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  if (warp >= n_rows) return;
+  const int old_q = old_pitch >> 1, new_q = new_pitch >> 1;
+  const float4 *in = src + (size_t)warp * old_q;
+  float4 *out = dst + (size_t)warp * new_q;
+  for (int k = lane; k < new_q; k += 32) out[k] = k < old_q ? __ldg(in + k) : make_float4(0.f, 0.f, 0.f, 0.f);
+}
+
 /* ------------------------------------------------------------------------------------------------
  * Candidate-pair enumeration on the device (the callers of runIcp: reoptimize dpg_slam.cc:79-107 and
  * updatePoseGraphObsConstraints dpg_slam.cc:255-300), output left in device memory as the pair batch.

@@ -103,6 +103,22 @@ class ScanMatcher:
                                                    scanner.angle_min, scanner.angle_max, scanner.range_max,
                                                    scanner.laser_x, scanner.laser_y, scanner.laser_theta))
 
+    def append_scans(self, points: np.ndarray, offsets: np.ndarray):
+        """Append CSR clouds (layout of :meth:`upload_scans`) as the next rows of the store; earlier rows, the pair
+        batch and the node table stay.  A failed append leaves the store as it was."""
+        pts = _pts(points) if len(points) else np.zeros((0, 2), np.float32)
+        off = np.ascontiguousarray(offsets, np.int64)
+        self._check(self._lib.dpgicp_append_scans(self._h, pts.ctypes.data, pts.shape[1] * 4, off.ctypes.data,
+                                                  off.shape[0] - 1))
+
+    def append_ranges(self, ranges: np.ndarray, scanner):
+        """Append raw range scans (n_scans, n_beams) as the next rows of the store, converted on the device exactly as
+        :meth:`upload_ranges` does (createNode: one call per new node).  A failed append leaves the store as it was."""
+        r = np.ascontiguousarray(ranges, np.float32)
+        self._check(self._lib.dpgicp_append_ranges(self._h, r.ctypes.data, r.shape[0], r.shape[1],
+                                                   scanner.angle_min, scanner.angle_max, scanner.range_max,
+                                                   scanner.laser_x, scanner.laser_y, scanner.laser_theta))
+
     def upload_ranges_ptr(self, host_ptr: int, n_scans: int, n_beams: int, scanner):
         """Same, from a raw (e.g. pinned) host pointer."""
         self._check(self._lib.dpgicp_upload_ranges(self._h, C.c_void_p(host_ptr), n_scans, n_beams,

@@ -188,6 +188,23 @@ def config_corridor(n_pairs=5000, n_beams=1081, seed=2, step=1.0) -> Workload:
     return wl
 
 
+def config_corridor_passes(n_scans=1000, n_beams=1081, passes=2, seed=2) -> Workload:
+    """The config-2 corridor driven forth and back in `passes` passes, poses 1 m apart (odd passes face back), as an
+    online caller meets it node by node: node estimates = truth + noise N(0, 0.05 m; 0.02 rad), pass number per node.
+    The pair list is the successive pairs; an online replay enumerates its own."""
+    rng = np.random.default_rng(seed)
+    per = -(-n_scans // passes)
+    poses = np.zeros((n_scans, 3))
+    for s in range(n_scans):
+        k, back = s % per, (s // per) % 2 == 1
+        poses[s] = (5.0 + (per - 1 - k if back else k), rng.uniform(-0.3, 0.3),
+                    (math.pi if back else 0.0) + rng.uniform(-0.05, 0.05))
+    est = poses + rng.normal(0, [0.05, 0.05, 0.02], (n_scans, 3))
+    src = np.arange(1, n_scans)
+    return _finish("corridor_passes", Scanner(n_beams=n_beams), world_corridor(0.0, per + 10.0, seed=seed), poses, est,
+                   src, src - 1, seed, (np.arange(n_scans) // per).astype(np.int32))
+
+
 def _free_poses(segs, size, n, rng, margin=0.4):
     lib = _synth()
     out = np.empty((n, 3))

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define DPGICP_ABI_VERSION 3
+#define DPGICP_ABI_VERSION 4
 
 /* ---- error codes ------------------------------------------------------------------------- */
 #define DPGICP_OK            0
@@ -196,6 +196,25 @@ int  dpgicp_upload_ranges(dpgicp_ctx *ctx, const float *ranges, int32_t n_scans,
 int  dpgicp_upload_ranges_subset(dpgicp_ctx *ctx, const float *ranges, int32_t n_scans_total, int32_t n_beams,
                                  const int32_t *scan_ids, int32_t n_ids, float angle_min, float angle_max,
                                  float range_max, float laser_x, float laser_y, float laser_theta);
+
+/* Append n_scans range scans to the store: they become rows scan_count() .. scan_count() + n_scans - 1, so node k of
+ * an online caller can own row k without the earlier scans being sent again (createNode, dpg_slam.cc:462-513, one
+ * call per new node).  Same conversion and arguments as dpgicp_upload_ranges: every appended row and its count are bit
+ * for bit what one dpgicp_upload_ranges of all the scans would hold.  Existing rows, the current pair batch and the
+ * node table stay valid (indices only grow).  After dpgicp_upload_ranges_subset the appended scans take the next row
+ * numbers, whatever scans the subset's rows came from.  An empty (or never uploaded) store is started.
+ * Storage grows by doubling; a scan longer than the store's row pitch re-pitches the store on the device.
+ * Failure leaves the store as it was: a non-finite or out-of-range point gives DPGICP_E_RANGE with scan_count()
+ * unchanged and every earlier row intact (unlike a full upload, which empties the store); bad arguments give
+ * DPGICP_E_INVALID and n_beams > DPGICP_MAX_POINTS gives DPGICP_E_TOOBIG, both before any device work.  Stream-ordered
+ * with a dpgicp_run enqueued before it: the run reads the store as it was.                                        */
+int  dpgicp_append_ranges(dpgicp_ctx *ctx, const float *ranges, int32_t n_scans, int32_t n_beams,
+                          float angle_min, float angle_max, float range_max,
+                          float laser_x, float laser_y, float laser_theta);
+/* The same for point clouds, with the layout and offsets of dpgicp_upload_scans (a scan over DPGICP_MAX_POINTS points
+ * gives DPGICP_E_TOOBIG).                                                                                        */
+int  dpgicp_append_scans(dpgicp_ctx *ctx, const void *points, size_t stride_bytes,
+                         const int64_t *offsets, int32_t n_scans);
 
 int  dpgicp_scan_count(const dpgicp_ctx *ctx);
 /* copy scan k of the store back to the host (packed float2); *n_points in = capacity, out = count */

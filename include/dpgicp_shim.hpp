@@ -107,6 +107,20 @@ class ScanMatcher {
     check(dpgicp_upload_scans(ctx_, all.data(), sizeof(PointXYZ), off.data(), (int32_t)clouds.size()),
           "dpgicp_upload_scans");
   }
+  /* online form (createNode, dpg_slam.cc:462-513): the new node's scan(s) become the next rows of the store, earlier
+   * rows stay on the device; n_scans * n_beams floats at `ranges` */
+  void appendRanges(const float *ranges, int n_scans, int n_beams, float angle_min, float angle_max, float range_max,
+                    float lx = 0.2f, float ly = 0.0f, float ltheta = 0.0f) {
+    check(dpgicp_append_ranges(ctx_, ranges, n_scans, n_beams, angle_min, angle_max, range_max, lx, ly, ltheta),
+          "dpgicp_append_ranges");
+  }
+  void appendClouds(const std::vector<Cloud> &clouds) {
+    std::vector<PointXYZ> all;
+    std::vector<int64_t> off(1, 0);
+    for (const Cloud &c : clouds) { all.insert(all.end(), c.begin(), c.end()); off.push_back((int64_t)all.size()); }
+    check(dpgicp_append_scans(ctx_, all.data(), sizeof(PointXYZ), off.data(), (int32_t)clouds.size()),
+          "dpgicp_append_scans");
+  }
   /* node poses -> (source, target) list of one reoptimize() */
   void enumeratePairs(const std::vector<Pose2f> &poses, const std::vector<int32_t> &pass, float same_pass_radius,
                       float other_pass_radius, std::vector<int32_t> &src, std::vector<int32_t> &tgt) {
