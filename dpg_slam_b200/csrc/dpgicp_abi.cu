@@ -74,7 +74,9 @@ struct dpgicp_ctx {
   bool own_stream = true;
   Store store, scratch_store;
   Batch batch, scratch_batch;
-  Nodes nodes;
+  Nodes nodes;                               /* dpgicp_set_nodes: the table of dpgicp_enumerate_pairs_device */
+  Nodes list_nodes;                          /* dpgicp_enumerate_pairs: its own positions-only table */
+  DevBuf enum_amb;                           /* enumeration: pairs whose guess the host re-derives */
   DevBuf stage, offsets, misc, corr, trig, enum_cnt;
   /* per (kernel, warps, shared memory): resident CTAs per SM or clusters per device — queried once, not on every run */
   std::map<std::tuple<const void *, int, size_t>, int> occupancy;
@@ -622,9 +624,8 @@ int two_cloud_store(dpgicp_ctx *ctx, const void *a, int na, const void *b, int n
   return DPGICP_OK;
 }
 
-/* node estimates -> device, plus the index-order box hierarchy the enumeration walks */
-int set_nodes_impl(dpgicp_ctx *ctx, const float *pose, const int32_t *pass, int32_t n, bool pose_is_xy) {
-  Nodes &N = ctx->nodes;
+/* node estimates -> node table N on the device, plus the index-order box hierarchy the enumeration walks */
+int set_nodes_impl(dpgicp_ctx *ctx, Nodes &N, const float *pose, const int32_t *pass, int32_t n, bool pose_is_xy) {
   N.n = 0;
   if (n == 0) return DPGICP_OK;
   std::vector<float> xy((size_t)n * 2), aux((size_t)n * 4);
@@ -671,10 +672,10 @@ int set_nodes_impl(dpgicp_ctx *ctx, const float *pose, const int32_t *pass, int3
   return DPGICP_OK;
 }
 
-/* the caller's pair list of `mode` built on the device into batch b (this shard's part); host learns the counts */
-int enumerate_into(dpgicp_ctx *ctx, Batch &b, int mode, float r_same, float r_other, int rank, int world,
+/* the caller's pair list of `mode` over node table N built on the device into batch b (this shard's part); host learns
+ * the counts */
+int enumerate_into(dpgicp_ctx *ctx, const Nodes &N, Batch &b, int mode, float r_same, float r_other, int rank, int world,
                    int64_t *n_total, int64_t *n_local) {
-  Nodes &N = ctx->nodes;
   if (n_total) *n_total = 0;
   if (n_local) *n_local = 0;
   b.n_pairs = 0; b.has_order = false; b.max_scan = -1;
@@ -682,7 +683,8 @@ int enumerate_into(dpgicp_ctx *ctx, Batch &b, int mode, float r_same, float r_ot
   const int n = N.n;
   const int n_chunks = mode == DPGICP_ENUM_ONLINE ? std::max(1, (n - 3 + 31) / 32) : n;
   int rc;
-  if ((rc = reserve(ctx, ctx->enum_cnt, sizeof(unsigned long long) * ((size_t)n_chunks + 1) + 8 + sizeof(long long) * 4096))) return rc;
+  if ((rc = reserve(ctx, ctx->enum_cnt, sizeof(unsigned long long) * ((size_t)n_chunks + 2)))) return rc;
+  if ((rc = reserve(ctx, ctx->enum_amb, sizeof(AmbPair) * 4096))) return rc;
   EnumParams E;
   std::memset(&E, 0, sizeof(E));
   E.xy = (const float2 *)N.xy.p; E.pass = (const int32_t *)N.pass.p; E.aux = (const float4 *)N.aux.p;
@@ -690,9 +692,9 @@ int enumerate_into(dpgicp_ctx *ctx, Batch &b, int mode, float r_same, float r_ot
   for (int L = 0; L < N.levels; ++L) { E.level_off[L] = N.level_off[L]; E.level_cnt[L] = (int32_t)N.level_cnt[L]; }
   E.levels = N.levels; E.n = n; E.r_same = r_same; E.r_other = r_other;
   E.cnt = (unsigned long long *)ctx->enum_cnt.p;
-  E.amb_count = (unsigned int *)(E.cnt + n_chunks + 1);
-  E.amb_list = (long long *)(E.cnt + n_chunks + 2);
-  E.amb_cap = 4096;
+  E.amb_count = E.cnt + n_chunks + 1;
+  E.amb_list = (AmbPair *)ctx->enum_amb.p;
+  E.amb_cap = (long long)(ctx->enum_amb.cap / sizeof(AmbPair));
   E.rank = rank; E.world = world;
   const int blocks = (n_chunks + 3) / 4;
   if (mode == DPGICP_ENUM_ONLINE) enumerate_online_kernel<false><<<blocks, 128, 0, ctx->stream>>>(E, n_chunks);
@@ -702,7 +704,7 @@ int enumerate_into(dpgicp_ctx *ctx, Batch &b, int mode, float r_same, float r_ot
   CU_TRY(ctx, cudaGetLastError());
   unsigned long long total = 0;
   CU_TRY(ctx, cudaMemcpyAsync(&total, E.cnt + n_chunks, sizeof(total), cudaMemcpyDeviceToHost, ctx->stream));
-  CU_TRY(ctx, cudaMemsetAsync(E.amb_count, 0, sizeof(unsigned int), ctx->stream));
+  CU_TRY(ctx, cudaMemsetAsync(E.amb_count, 0, sizeof(*E.amb_count), ctx->stream));
   CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
   const int64_t local = (int64_t)total > rank ? ((int64_t)total - rank + world - 1) / world : 0;
   if (n_total) *n_total = (int64_t)total;
@@ -711,36 +713,41 @@ int enumerate_into(dpgicp_ctx *ctx, Batch &b, int mode, float r_same, float r_ot
   if ((rc = reserve(ctx, b.results, sizeof(dpgicp_result) * (size_t)std::max<int64_t>(local, 1)))) return rc;
   E.tasks = (PairTask *)b.tasks.p;
   E.n_local = local;
-  if (mode == DPGICP_ENUM_ONLINE) enumerate_online_kernel<true><<<blocks, 128, 0, ctx->stream>>>(E, n_chunks);
-  else enumerate_reopt_kernel<true><<<blocks, 128, 0, ctx->stream>>>(E);
-  ctx->launches++;
-  CU_TRY(ctx, cudaGetLastError());
   /* pairs whose cos/sin of the guess angle sit within a few binary64 ulps of a binary32 rounding boundary (about one
-   * in 10^7): the device's libm and the host's are not guaranteed to round them alike, so the host — whose libm defines
-   * the guess matrix everywhere else (set_pairs) — re-derives them */
-  unsigned int amb = 0;
-  CU_TRY(ctx, cudaMemcpyAsync(&amb, E.amb_count, sizeof(amb), cudaMemcpyDeviceToHost, ctx->stream));
-  CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  if (amb > (unsigned)E.amb_cap) return fail(ctx, DPGICP_E_STATE, "too many guess angles at a rounding boundary (internal limit)");
-  if (amb > 0) {
-    std::vector<long long> slots(amb);
-    CU_TRY(ctx, cudaMemcpyAsync(slots.data(), E.amb_list, sizeof(long long) * amb, cudaMemcpyDeviceToHost, ctx->stream));
+   * in 10^7 for random headings, but every pair of a recurring boundary heading difference): the device's libm and the
+   * host's are not guaranteed to round them alike, so the host — whose libm defines the guess matrix everywhere else
+   * (set_pairs) — re-derives them.  The fill pass lists them with their angles; when the list overflows, it grows to
+   * the count and the (deterministic) fill pass runs again.  Then one copy down, host libm, one copy up and a scatter:
+   * the number of synchronisations does not depend on the number of listed pairs. */
+  unsigned long long amb = 0;
+  for (int attempt = 0; attempt < 2; ++attempt) {
+    if (mode == DPGICP_ENUM_ONLINE) enumerate_online_kernel<true><<<blocks, 128, 0, ctx->stream>>>(E, n_chunks);
+    else enumerate_reopt_kernel<true><<<blocks, 128, 0, ctx->stream>>>(E);
+    ctx->launches++;
+    CU_TRY(ctx, cudaGetLastError());
+    CU_TRY(ctx, cudaMemcpyAsync(&amb, E.amb_count, sizeof(amb), cudaMemcpyDeviceToHost, ctx->stream));
     CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    for (long long slot : slots) {
-      PairTask t;
-      CU_TRY(ctx, cudaMemcpyAsync(&t, (PairTask *)b.tasks.p + slot, sizeof(t), cudaMemcpyDeviceToHost, ctx->stream));
-      CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-      float th[2];
-      CU_TRY(ctx, cudaMemcpyAsync(&th[0], (const float4 *)N.aux.p + t.tgt, sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-      CU_TRY(ctx, cudaMemcpyAsync(&th[1], (const float4 *)N.aux.p + t.src, sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-      CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-      double d = (double)(float)(th[1] - th[0]);
-      d -= (M_PI * 2.0) * rint(d / (M_PI * 2.0));
-      const float g2 = (float)d;
-      t.c = (float)std::cos((double)g2); t.s = (float)std::sin((double)g2);
-      CU_TRY(ctx, cudaMemcpyAsync((PairTask *)b.tasks.p + slot, &t, sizeof(t), cudaMemcpyHostToDevice, ctx->stream));
-      CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    if (amb <= (unsigned long long)E.amb_cap) break;
+    if ((rc = reserve(ctx, ctx->enum_amb, sizeof(AmbPair) * (size_t)amb))) return rc;
+    E.amb_list = (AmbPair *)ctx->enum_amb.p;
+    E.amb_cap = (long long)(ctx->enum_amb.cap / sizeof(AmbPair));
+    CU_TRY(ctx, cudaMemsetAsync(E.amb_count, 0, sizeof(*E.amb_count), ctx->stream));
+  }
+  if (amb > (unsigned long long)E.amb_cap)        /* the second fill pass lists exactly the pairs the first one counted */
+    return fail(ctx, DPGICP_E_STATE, "the guess re-derivation list changed between two identical fill passes");
+  if (amb > 0) {
+    std::vector<AmbPair> list(amb);
+    CU_TRY(ctx, cudaMemcpyAsync(list.data(), E.amb_list, sizeof(AmbPair) * amb, cudaMemcpyDeviceToHost, ctx->stream));
+    CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    for (AmbPair &p : list) {
+      const float g2 = p.a;                      /* AngleMod of the pair, as dpgicp_relative_guess computes it */
+      p.a = (float)std::cos((double)g2); p.b = (float)std::sin((double)g2);
     }
+    CU_TRY(ctx, cudaMemcpyAsync(E.amb_list, list.data(), sizeof(AmbPair) * amb, cudaMemcpyHostToDevice, ctx->stream));
+    amb_scatter_kernel<<<(unsigned)((amb + 255) / 256), 256, 0, ctx->stream>>>(E.amb_list, (long long)amb, E.tasks);
+    ctx->launches++;
+    CU_TRY(ctx, cudaGetLastError());
+    CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));   /* `list` goes out of scope */
   }
   b.n_pairs = local;
   b.max_scan = n - 1;
@@ -944,7 +951,8 @@ void dpgicp_destroy(dpgicp_ctx *ctx) {
   }
   for (cudaEvent_t e : ctx->stage_ev) if (e) cudaEventDestroy(e);
   release(ctx->nodes.xy); release(ctx->nodes.aux); release(ctx->nodes.pass); release(ctx->nodes.boxes);
-  release(ctx->enum_cnt); release(ctx->d_pair);
+  release(ctx->list_nodes.xy); release(ctx->list_nodes.aux); release(ctx->list_nodes.pass); release(ctx->list_nodes.boxes);
+  release(ctx->enum_cnt); release(ctx->enum_amb); release(ctx->d_pair);
   if (ctx->h_pair) cudaFreeHost(ctx->h_pair);
   gather_close(ctx);
   release(ctx->gather);
@@ -1609,15 +1617,16 @@ int dpgicp_enumerate_pairs(dpgicp_ctx *ctx, const float *node_xy, const int32_t 
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   if (n_nodes < 0 || !n_pairs || (n_nodes > 0 && (!node_xy || !node_pass)))
     return fail(ctx, DPGICP_E_INVALID, "bad node arguments");
+  if (!(r_same >= 0.0f) || !(r_other >= 0.0f)) return fail(ctx, DPGICP_E_INVALID, "radii must be >= 0");
   const int64_t capacity = *n_pairs;
   *n_pairs = 0;
   if (n_nodes < 2) return DPGICP_OK;
-  /* the device enumeration with the list copied out: positions only (theta = 0), scratch batch */
+  /* the device enumeration with the list copied out: its own positions-only table (theta = 0) and the scratch batch;
+   * the node table of dpgicp_set_nodes and the batch stay as they are */
   int rc;
-  if ((rc = set_nodes_impl(ctx, node_xy, node_pass, n_nodes, true))) return rc;
+  if ((rc = set_nodes_impl(ctx, ctx->list_nodes, node_xy, node_pass, n_nodes, true))) return rc;
   int64_t total = 0, local = 0;
-  rc = enumerate_into(ctx, ctx->scratch_batch, DPGICP_ENUM_REOPTIMIZE, r_same, r_other, 0, 1, &total, &local);
-  ctx->nodes.n = 0;                          /* positions only: not a node table dpgicp_enumerate_pairs_device may use */
+  rc = enumerate_into(ctx, ctx->list_nodes, ctx->scratch_batch, DPGICP_ENUM_REOPTIMIZE, r_same, r_other, 0, 1, &total, &local);
   if (rc) return rc;
   *n_pairs = total;
   if (total > capacity || (total > 0 && (!src || !tgt))) {
@@ -1633,7 +1642,7 @@ int dpgicp_set_nodes(dpgicp_ctx *ctx, const float *pose, const int32_t *pass, in
   if (!ctx) return DPGICP_E_INVALID;
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   if (n < 0 || (n > 0 && (!pose || !pass))) return fail(ctx, DPGICP_E_INVALID, "bad node arguments");
-  return set_nodes_impl(ctx, pose, pass, n, false);
+  return set_nodes_impl(ctx, ctx->nodes, pose, pass, n, false);
 }
 
 int dpgicp_enumerate_pairs_device(dpgicp_ctx *ctx, int32_t mode, float r_same, float r_other, int32_t rank, int32_t world,
@@ -1650,7 +1659,7 @@ int dpgicp_enumerate_pairs_device(dpgicp_ctx *ctx, int32_t mode, float r_same, f
     ctx->batch.n_pairs = 0;
     return DPGICP_OK;
   }
-  return enumerate_into(ctx, ctx->batch, mode, r_same, r_other, rank, world, n_total, n_local);
+  return enumerate_into(ctx, ctx->nodes, ctx->batch, mode, r_same, r_other, rank, world, n_total, n_local);
 }
 
 int dpgicp_fetch_pairs(dpgicp_ctx *ctx, int32_t *src, int32_t *tgt, float *T, int64_t n) {

@@ -1803,6 +1803,13 @@ struct NodeBox {               /* 32 bytes: bounding box + pass range of an inde
 constexpr int kEnumFan = 32;   /* children per box = lanes of the warp testing them */
 constexpr int kEnumMaxLevels = 7;
 
+/* a pair listed for the host: its slot in the shard's list and its guess angle; the host replaces (a, b) = (g2, 0)
+ * with its libm's (cos g2, sin g2) and amb_scatter_kernel writes them into the pair */
+struct AmbPair {
+  long long slot;
+  float a, b;
+};
+
 struct EnumParams {
   const float2 *xy;            /* node positions                                          */
   const int32_t *pass;         /* node pass numbers                                       */
@@ -1817,9 +1824,9 @@ struct EnumParams {
   PairTask *tasks;             /* fill pass: this shard's pair list                         */
   int32_t rank, world;
   long long n_local;           /* capacity of tasks: this shard's pair count                 */
-  unsigned int *amb_count;     /* pairs whose cos/sin sit too close to a binary32 rounding boundary for two */
-  long long *amb_list;         /* libm implementations to be guaranteed to agree: the host re-derives these */
-  int32_t amb_cap;
+  unsigned long long *amb_count; /* pairs whose cos/sin sit too close to a binary32 rounding boundary for two */
+  AmbPair *amb_list;           /* libm implementations to be guaranteed to agree: the host re-derives these */
+  long long amb_cap;           /* entries of amb_list; the count goes on past it (the host then grows the list) */
 };
 
 /* the reference's gate: float distance between two node estimates against the same-pass / other-pass radius */
@@ -1897,10 +1904,19 @@ __device__ __forceinline__ PairTask make_pair_task(const EnumParams &E, int src,
   sincos(g2, &sd, &cd);
   t.c = (float)cd; t.s = (float)sd;
   if (near_f32_rounding_boundary(cd) || near_f32_rounding_boundary(sd)) {
-    const unsigned k = atomicAdd(E.amb_count, 1u);
-    if (k < (unsigned)E.amb_cap) E.amb_list[k] = slot;
+    const unsigned long long k = atomicAdd(E.amb_count, 1ull);
+    if (k < (unsigned long long)E.amb_cap) { AmbPair p; p.slot = slot; p.a = (float)g2; p.b = 0.f; E.amb_list[k] = p; }
   }
   return t;
+}
+
+/* the host's cos / sin of the listed pairs' guess angles into their pair tasks */
+__global__ void amb_scatter_kernel(const AmbPair *__restrict__ list, long long n, PairTask *__restrict__ tasks) {
+  const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const AmbPair p = list[k];
+  tasks[p.slot].c = p.a;
+  tasks[p.slot].s = p.b;
 }
 
 /* DPGICP_ENUM_REOPTIMIZE: one warp per node i.  FILL = false counts node i's pairs into cnt[i]; FILL = true writes

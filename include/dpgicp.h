@@ -326,7 +326,9 @@ int  dpgicp_correspondences_seeded(dpgicp_ctx *ctx,
 /* For node i (ascending) and every j < i-1 ... emits (src=i, tgt=j) when the node positions are
  * within same_pass_radius (same pass) or other_pass_radius (different pass), plus every
  * successive pair (src=i, tgt=i-1) — the pair set of one DpgSLAM::reoptimize().  Output order is
- * the reference's loop order.  *n_pairs in = capacity, out = count (DPGICP_E_TOOBIG if short).  */
+ * the reference's loop order.  *n_pairs in = capacity, out = count (DPGICP_E_TOOBIG if short).
+ * Radii must be >= 0 (NaN: DPGICP_E_INVALID).  This form is independent of the device-resident one below: it uses a
+ * node table of its own and leaves the table of dpgicp_set_nodes and the current batch as they were.            */
 int  dpgicp_enumerate_pairs(dpgicp_ctx *ctx, const float *node_xy, const int32_t *node_pass,
                             int32_t n_nodes, float same_pass_radius, float other_pass_radius,
                             int32_t *src_idx, int32_t *tgt_idx, int64_t *n_pairs);
@@ -345,7 +347,9 @@ int  dpgicp_enumerate_pairs(dpgicp_ctx *ctx, const float *node_xy, const int32_t
  *                           loop runs to dpg_nodes_.size() - 2 exclusive, dpg_slam.cc:275-299].
  * Sharding: of the global list only the pairs with (global index % shard_world) == shard_rank become this context's
  * batch (round-robin, as the multi-GPU path shards); local pair k is global pair shard_rank + k * shard_world.
- * n_pairs_total / n_pairs_local (may be NULL) receive the global and the local count.                          */
+ * n_pairs_total / n_pairs_local (may be NULL) receive the global and the local count.  Radii must be >= 0
+ * (NaN: DPGICP_E_INVALID).  Any legal node table enumerates: guesses whose cos / sin lie next to a binary32 rounding
+ * boundary are re-derived with the host's libm, however many pairs share one (e.g. a recurring heading difference). */
 #define DPGICP_ENUM_REOPTIMIZE 0
 #define DPGICP_ENUM_ONLINE     1
 int  dpgicp_set_nodes(dpgicp_ctx *ctx, const float *node_pose_xytheta, const int32_t *node_pass, int32_t n_nodes);
