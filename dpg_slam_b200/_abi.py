@@ -14,7 +14,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 
 # ---- constants (include/dpgicp.h) -----------------------------------------------------------------
-ABI_VERSION = 4
+ABI_VERSION = 5
 METRIC_POINT_TO_POINT, METRIC_POINT_TO_LINE = 0, 1
 SEARCH_BRUTE, SEARCH_PRUNED, SEARCH_PROJECTIVE = 0, 1, 2
 COV_REFERENCE_LIVE, COV_CENSI_INDEXPAIR, COV_CENSI_CORR = 0, 1, 2
@@ -118,6 +118,10 @@ EXPORTS = [
     "dpgicp_convert_ranges_device", "dpgicp_gather_attach_local", "dpgicp_gather_set_root_only",
     "dpgicp_enable_stage_timing", "dpgicp_last_run_stage_ms", "dpgicp_run_range", "dpgicp_fetch_results_range",
     "dpgicp_gather_fetch_range", "dpgicp_gather_declare", "dpgicp_append_ranges", "dpgicp_append_scans",
+    "dpgicp_slot_create", "dpgicp_slot_destroy", "dpgicp_slot_set_pairs", "dpgicp_slot_set_pair_cost_hints",
+    "dpgicp_slot_run", "dpgicp_slot_run_range", "dpgicp_slot_fetch_results", "dpgicp_slot_fetch_results_range",
+    "dpgicp_slot_fetch_factors", "dpgicp_slot_fetch_pairs", "dpgicp_slot_last_run_counters", "dpgicp_slot_synchronize",
+    "dpgicp_slot_query", "dpgicp_slot_enumerate_pairs_device",
 ]
 
 _lib = None
@@ -191,6 +195,21 @@ def load_library() -> C.CDLL:
         "dpgicp_run_range": (C.c_int, [vp, PP, i64, i64]),
         "dpgicp_fetch_results_range": (C.c_int, [vp, vp, i64, i64]),
         "dpgicp_gather_fetch_range": (C.c_int, [vp, vp, i64, i64]),
+        "dpgicp_slot_create": (C.c_int, [vp, C.POINTER(vp)]),
+        "dpgicp_slot_destroy": (C.c_int, [vp]),
+        "dpgicp_slot_set_pairs": (C.c_int, [vp, vp, vp, vp, i64]),
+        "dpgicp_slot_set_pair_cost_hints": (C.c_int, [vp, vp, i64]),
+        "dpgicp_slot_run": (C.c_int, [vp, PP]),
+        "dpgicp_slot_run_range": (C.c_int, [vp, PP, i64, i64]),
+        "dpgicp_slot_fetch_results": (C.c_int, [vp, vp, i64]),
+        "dpgicp_slot_fetch_results_range": (C.c_int, [vp, vp, i64, i64]),
+        "dpgicp_slot_fetch_factors": (C.c_int, [vp, vp, i64]),
+        "dpgicp_slot_fetch_pairs": (C.c_int, [vp, vp, vp, vp, i64]),
+        "dpgicp_slot_last_run_counters": (C.c_int, [vp, C.POINTER(C.c_uint64 * 8)]),
+        "dpgicp_slot_synchronize": (C.c_int, [vp]),
+        "dpgicp_slot_query": (C.c_int, [vp]),
+        "dpgicp_slot_enumerate_pairs_device": (C.c_int, [vp, i32, C.c_float, C.c_float, i32, i32, C.POINTER(i64),
+                                                         C.POINTER(i64)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)      # AttributeError if the symbol is not exported

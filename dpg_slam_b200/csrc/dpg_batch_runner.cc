@@ -22,6 +22,9 @@
  * --replay runs the reference's online loop instead of one batch (replay() below): every log scan becomes a node, is
  * appended to the scan store and aligned with its predecessor and its loop-closure candidates; a reoptimize() runs at
  * every pass boundary.  The CSV gains a leading column `update` (k, or reopt@k); the JSON line reports per-update times.
+ * --inflight K (K >= 2) enumerates the pair list into K batch slots of one context and runs it in batches of
+ * --batch-pairs pairs with K batches in flight (batch b on slot b % K, launched once that slot's previous batch is
+ * fetched).  The CSV is identical to --inflight 1.
  */
 #include <algorithm>
 #include <chrono>
@@ -30,6 +33,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <stdexcept>
 #include <string>
 #include <vector>
@@ -250,6 +254,8 @@ int main(int argc, char **argv) {
   std::vector<int> devices;
   int32_t caller = DPGICP_ENUM_REOPTIMIZE;
   bool successive_only = false, replay_log = false;
+  int inflight = 1;
+  int64_t batch_pairs = 5000;
   uint64_t seed = 2;
   dpgicp_params params;
   dpgicp_default_params(&params);
@@ -286,13 +292,15 @@ int main(int argc, char **argv) {
     else if (a == "--other-pass-radius") r_other = (float)std::atof(next("--other-pass-radius"));
     else if (a == "--successive-only") successive_only = true;
     else if (a == "--replay") replay_log = true;
+    else if (a == "--inflight") inflight = std::atoi(next("--inflight"));
+    else if (a == "--batch-pairs") batch_pairs = std::atoll(next("--batch-pairs"));
     else {
       std::fprintf(stderr,
                    "usage: dpg_batch_runner [--synthetic corridor|office | --log FILE] [--scans N] [--beams N] [--passes N]\n"
                    "         [--seed S] [--divisor D] [--cov-mode 0|1|2] [--metric 0|1] [--search 0|1|2] [--window W] [--successive-only]\n"
                    "         [--same-pass-radius R] [--other-pass-radius R] [--write-log FILE] [--out FILE.csv] [--device K]\n"
                    "         [--gpus N | --devices a,b,...] [--caller reoptimize|online] [--outlier-mode 0|1|2 --outlier-param X]\n"
-                   "         [--replay]\n");
+                   "         [--replay] [--inflight K [--batch-pairs N]]\n");
       return a == "--help" ? 0 : 2;
     }
   }
@@ -305,6 +313,12 @@ int main(int argc, char **argv) {
   }
   if (!log_out.empty() && !write_log(log_out.c_str(), L)) { std::fprintf(stderr, "cannot write %s\n", log_out.c_str()); return 1; }
 
+  if (inflight < 1 || batch_pairs < 1) { std::fprintf(stderr, "dpg_batch_runner: --inflight and --batch-pairs must be >= 1\n"); return 2; }
+  if (inflight > 1 && (replay_log || successive_only || !devices.empty())) {
+    std::fprintf(stderr, "dpg_batch_runner: --inflight K > 1 runs the enumerated batch of one context (--device K); it is not "
+                         "supported with --replay, --successive-only, --gpus or --devices\n");
+    return 2;
+  }
   if (replay_log && !devices.empty()) {
     std::fprintf(stderr, "dpg_batch_runner: --replay runs on one device (--device K); --gpus / --devices are not supported "
                          "with it (online batches are tens of pairs)\n");
@@ -327,6 +341,39 @@ int main(int argc, char **argv) {
       t2 = now_s();
       res = sm.runIcpBatch(L.est, src, tgt);
       t3 = now_s();
+    } else if (inflight > 1) {
+      dpgicp_shim::ScanMatcher sm(devices[0]);
+      sm.params() = params;
+      t0 = now_s();
+      sm.uploadRanges(L.ranges, L.n_scans, L.n_beams, L.angle_min, L.angle_max, L.range_max, L.lx, L.ly, L.lt);
+      t1 = now_s();
+      std::vector<float> flat((size_t)L.n_scans * 3);
+      for (int i = 0; i < L.n_scans; ++i) { flat[3 * (size_t)i] = L.est[(size_t)i].x; flat[3 * (size_t)i + 1] = L.est[(size_t)i].y; flat[3 * (size_t)i + 2] = L.est[(size_t)i].theta; }
+      if (dpgicp_set_nodes(sm.ctx(), flat.data(), L.pass.data(), L.n_scans) != DPGICP_OK)
+        throw std::runtime_error(std::string("dpgicp_set_nodes: ") + sm.last_error());
+      std::vector<std::unique_ptr<dpgicp_shim::ScanMatcher::Slot>> slots;
+      int64_t n = 0;
+      for (int k = 0; k < inflight; ++k) {
+        slots.emplace_back(new dpgicp_shim::ScanMatcher::Slot(sm));
+        n = slots.back()->enumeratePairs(caller, r_same, r_other);
+      }
+      t2 = now_s();
+      res.resize((size_t)n);
+      std::vector<int64_t> pending((size_t)inflight, -1);         /* first pair of the batch each slot has in flight */
+      auto fetch = [&](int k) {
+        const int64_t f = pending[(size_t)k];
+        if (f >= 0) slots[(size_t)k]->fetchResults(&res[(size_t)f], f, std::min(batch_pairs, n - f));
+        pending[(size_t)k] = -1;
+      };
+      for (int64_t first = 0, b = 0; first < n; first += batch_pairs, ++b) {
+        const int k = (int)(b % inflight);
+        fetch(k);
+        slots[(size_t)k]->runRange(first, std::min(batch_pairs, n - first));
+        pending[(size_t)k] = first;
+      }
+      for (int k = 0; k < inflight; ++k) fetch(k);
+      t3 = now_s();
+      slots[0]->pairs(src, tgt, n);
     } else {
       /* the callers' form: nodes in, pair list enumerated and kept on the device(s), records gathered back */
       dpgicp_shim::MultiGpuScanMatcher sm(devices);
@@ -360,10 +407,10 @@ int main(int argc, char **argv) {
       }
       std::fclose(f);
     }
-    std::printf("{\"scans\": %d, \"beams\": %d, \"gpus\": %zu, \"pairs\": %zu, \"converged\": %zu, \"cov_singular\": %zu, "
+    std::printf("{\"scans\": %d, \"beams\": %d, \"gpus\": %zu, \"inflight\": %d, \"pairs\": %zu, \"converged\": %zu, \"cov_singular\": %zu, "
                 "\"mean_iterations\": %.2f, \"upload_s\": %.6f, \"enumerate_s\": %.6f, \"icp_cov_s\": %.6f, "
                 "\"pairs_per_s\": %.1f}\n",
-                L.n_scans, L.n_beams, devices.size(), res.size(), converged, singular, res.empty() ? 0.0 : it_sum / (double)res.size(),
+                L.n_scans, L.n_beams, devices.size(), inflight, res.size(), converged, singular, res.empty() ? 0.0 : it_sum / (double)res.size(),
                 t1 - t0, t2 - t1, t3 - t2, res.empty() ? 0.0 : (double)res.size() / (t3 - t2));
   } catch (const std::exception &e) {
     std::fprintf(stderr, "dpg_batch_runner: %s\n", e.what());

@@ -17,6 +17,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <new>
+#include <set>
 #include <string>
 #include <vector>
 
@@ -67,22 +68,37 @@ struct Nodes {                   /* pose-graph node estimates on the device (dpg
 
 }  // namespace
 
+/* One pair batch of a context and the per-run cells of its stage chain.  The context holds the default slot (the batch of
+ * dpgicp_set_pairs / dpgicp_run / dpgicp_fetch_*), which runs on the context's stream; dpgicp_slot_create adds slots with
+ * a stream of their own, so several batches can be in flight over the one scan store. */
+struct dpgicp_slot {
+  dpgicp_ctx *ctx = nullptr;
+  cudaStream_t own = nullptr;                /* nullptr: the default slot, on the context's stream */
+  Batch batch;
+  DevBuf state[2], susp[2];                  /* suspended-pair state slots + pair lists, ping-pong between stages */
+  unsigned long long *d_queue = nullptr;     /* [0..4] stage queue heads, [6],[7] suspended counts, [8..15] counters, [16..23] development phase timers, [24..28] pairs finished per stage */
+  cudaEvent_t stage_ev[9] = {nullptr};
+  bool stage_timing = false;
+  int last_stages = 0;
+};
+
 struct dpgicp_ctx {
   int device = 0;
   int sm_count = 148;
   cudaStream_t stream = nullptr;
   bool own_stream = true;
   Store store, scratch_store;
-  Batch batch, scratch_batch;
+  dpgicp_slot main;                          /* the default slot */
+  std::vector<dpgicp_slot *> slots;          /* the live slots of dpgicp_slot_create */
+  cudaEvent_t written = nullptr;             /* recorded on the context's stream behind every write a later slot run reads
+                                              * (store rows and counts, an enumerated pair list): slot streams wait on it */
+  Batch scratch_batch;
   Nodes nodes;                               /* dpgicp_set_nodes: the table of dpgicp_enumerate_pairs_device */
   Nodes list_nodes;                          /* dpgicp_enumerate_pairs: its own positions-only table */
   DevBuf enum_amb;                           /* enumeration: pairs whose guess the host re-derives */
   DevBuf stage, offsets, misc, corr, trig, enum_cnt;
   /* per (kernel, warps, shared memory): resident CTAs per SM or clusters per device — queried once, not on every run */
   std::map<std::tuple<const void *, int, size_t>, int> occupancy;
-  cudaEvent_t stage_ev[9] = {nullptr};
-  bool stage_timing = false;
-  int last_stages = 0;
   void *h_pair = nullptr;                    /* pinned scratch of the single-pair call shapes */
   size_t h_pair_cap = 0;
   DevBuf d_pair;
@@ -90,8 +106,6 @@ struct dpgicp_ctx {
   bool gather_local = false;                 /* peers attached by dpgicp_gather_attach_local (no IPC mappings to close) */
   int trig_n = 0;
   float trig_min = 0.f, trig_inc = 0.f;
-  DevBuf state[2], susp[2];                  /* suspended-pair state slots + pair lists, ping-pong between stages */
-  unsigned long long *d_queue = nullptr;     /* [0..4] stage queue heads, [6],[7] suspended counts, [8..15] counters, [16..23] development phase timers, [24..28] pairs finished per stage */
   DevBuf gather;                             /* this rank's copy of the whole batch's records (fused gather)  */
   int64_t gather_n = 0;
   int gather_world = 0, gather_rank = 0;
@@ -124,6 +138,31 @@ int fail(dpgicp_ctx *ctx, int code, const std::string &msg) {
                   std::string(#expr) + ": " + cudaGetErrorString(e__));                           \
     }                                                                                             \
   } while (0)
+
+cudaStream_t stream_of(const dpgicp_slot *s) { return s->own ? s->own : s->ctx->stream; }
+
+/* a buffer the runs of every slot may read is about to be overwritten or freed: wait until the slots' streams have
+ * drained (the default slot's runs are ordered on the context's stream) */
+int drain_slots(dpgicp_ctx *ctx) {
+  for (dpgicp_slot *s : ctx->slots) CU_TRY(ctx, cudaStreamSynchronize(s->own));
+  return DPGICP_OK;
+}
+
+/* the store is about to be replaced: every slot's runs have read it, and every batch is emptied (its indices referred to
+ * the old store) */
+int replace_store(dpgicp_ctx *ctx) {
+  int rc = drain_slots(ctx);
+  if (rc) return rc;
+  ctx->main.batch.n_pairs = 0;
+  for (dpgicp_slot *s : ctx->slots) s->batch.n_pairs = std::min<int64_t>(s->batch.n_pairs, 0);
+  return DPGICP_OK;
+}
+
+/* the context's stream has written what a slot's later runs read (store rows and counts, an enumerated list) */
+int mark_written(dpgicp_ctx *ctx) {
+  CU_TRY(ctx, cudaEventRecord(ctx->written, ctx->stream));
+  return DPGICP_OK;
+}
 
 int reserve(dpgicp_ctx *ctx, DevBuf &b, size_t bytes) {
   if (bytes <= b.cap) return DPGICP_OK;
@@ -181,7 +220,7 @@ float gate_threshold(const dpgicp_params *p) {
 }
 
 template <int WARPS, int SEARCH, int CSIZE>
-int launch_icp_t(dpgicp_ctx *ctx, const KernelParams &kp, size_t smem, int64_t max_items, int nw, int *grid_out) {
+int launch_icp_t(dpgicp_ctx *ctx, cudaStream_t stream, const KernelParams &kp, size_t smem, int64_t max_items, int nw, int *grid_out) {
   auto kern = icp_pairs_kernel<WARPS, SEARCH, CSIZE>;
   const void *kfn = reinterpret_cast<const void *>(kern);
   /* the dynamic shared-memory opt-in and the occupancy of a shape do not change between runs: set / query once */
@@ -198,7 +237,7 @@ int launch_icp_t(dpgicp_ctx *ctx, const KernelParams &kp, size_t smem, int64_t m
   cudaLaunchConfig_t cfg = {};
   cfg.blockDim = dim3((unsigned)nw * 32, 1, 1);
   cfg.dynamicSmemBytes = smem;
-  cfg.stream = ctx->stream;
+  cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
   attr[0].val.clusterDim.x = CSIZE; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
@@ -242,26 +281,26 @@ int launch_icp_t(dpgicp_ctx *ctx, const KernelParams &kp, size_t smem, int64_t m
 /* nw warps per CTA run on the instantiation with the next power-of-two register budget; clusters (the last
  * stage only) use the 16-warp budget */
 template <int SEARCH>
-int launch_icp_w(dpgicp_ctx *ctx, int nw, int csize, const KernelParams &kp, size_t smem, int64_t n, int *grid_out) {
+int launch_icp_w(dpgicp_ctx *ctx, cudaStream_t stream, int nw, int csize, const KernelParams &kp, size_t smem, int64_t n, int *grid_out) {
   nw = std::max(1, std::min(nw, 16));
   /* first stage of large scans: 12 warps with the 80-register budget so that two CTAs share an SM */
-  if (csize == 1 && !kp.resume && nw > 8 && nw <= 12) return launch_icp_t<12, SEARCH, 1>(ctx, kp, smem, n, nw, grid_out);
-  if (csize == 2) return launch_icp_t<16, SEARCH, 2>(ctx, kp, smem, n, nw, grid_out);
-  if (csize == 4) return launch_icp_t<16, SEARCH, 4>(ctx, kp, smem, n, nw, grid_out);
-  if (nw <= 1) return launch_icp_t<1, SEARCH, 1>(ctx, kp, smem, n, 1, grid_out);
-  if (nw <= 2) return launch_icp_t<2, SEARCH, 1>(ctx, kp, smem, n, nw, grid_out);
-  if (nw <= 4) return launch_icp_t<4, SEARCH, 1>(ctx, kp, smem, n, nw, grid_out);
-  if (nw <= 8) return launch_icp_t<8, SEARCH, 1>(ctx, kp, smem, n, nw, grid_out);
-  return launch_icp_t<16, SEARCH, 1>(ctx, kp, smem, n, nw, grid_out);
+  if (csize == 1 && !kp.resume && nw > 8 && nw <= 12) return launch_icp_t<12, SEARCH, 1>(ctx, stream, kp, smem, n, nw, grid_out);
+  if (csize == 2) return launch_icp_t<16, SEARCH, 2>(ctx, stream, kp, smem, n, nw, grid_out);
+  if (csize == 4) return launch_icp_t<16, SEARCH, 4>(ctx, stream, kp, smem, n, nw, grid_out);
+  if (nw <= 1) return launch_icp_t<1, SEARCH, 1>(ctx, stream, kp, smem, n, 1, grid_out);
+  if (nw <= 2) return launch_icp_t<2, SEARCH, 1>(ctx, stream, kp, smem, n, nw, grid_out);
+  if (nw <= 4) return launch_icp_t<4, SEARCH, 1>(ctx, stream, kp, smem, n, nw, grid_out);
+  if (nw <= 8) return launch_icp_t<8, SEARCH, 1>(ctx, stream, kp, smem, n, nw, grid_out);
+  return launch_icp_t<16, SEARCH, 1>(ctx, stream, kp, smem, n, nw, grid_out);
 }
 
-int launch_stage(dpgicp_ctx *ctx, int search, int nw, int csize, const KernelParams &kp, size_t smem, int64_t n, int *grid_out) {
-  if (search == DPGICP_SEARCH_PROJECTIVE) return launch_icp_w<DPGICP_SEARCH_PROJECTIVE>(ctx, nw, csize, kp, smem, n, grid_out);
-  if (search == DPGICP_SEARCH_PRUNED) return launch_icp_w<DPGICP_SEARCH_PRUNED>(ctx, nw, csize, kp, smem, n, grid_out);
-  if (search == kSearchPrunedFlat) return launch_icp_w<kSearchPrunedFlat>(ctx, nw, csize, kp, smem, n, grid_out);
-  if (search == kSearchPrunedStock) return launch_icp_w<kSearchPrunedStock>(ctx, nw, csize, kp, smem, n, grid_out);
-  if (search == kSearchPrunedFlatStock) return launch_icp_w<kSearchPrunedFlatStock>(ctx, nw, csize, kp, smem, n, grid_out);
-  return launch_icp_w<DPGICP_SEARCH_BRUTE>(ctx, nw, csize, kp, smem, n, grid_out);
+int launch_stage(dpgicp_ctx *ctx, cudaStream_t stream, int search, int nw, int csize, const KernelParams &kp, size_t smem, int64_t n, int *grid_out) {
+  if (search == DPGICP_SEARCH_PROJECTIVE) return launch_icp_w<DPGICP_SEARCH_PROJECTIVE>(ctx, stream, nw, csize, kp, smem, n, grid_out);
+  if (search == DPGICP_SEARCH_PRUNED) return launch_icp_w<DPGICP_SEARCH_PRUNED>(ctx, stream, nw, csize, kp, smem, n, grid_out);
+  if (search == kSearchPrunedFlat) return launch_icp_w<kSearchPrunedFlat>(ctx, stream, nw, csize, kp, smem, n, grid_out);
+  if (search == kSearchPrunedStock) return launch_icp_w<kSearchPrunedStock>(ctx, stream, nw, csize, kp, smem, n, grid_out);
+  if (search == kSearchPrunedFlatStock) return launch_icp_w<kSearchPrunedFlatStock>(ctx, stream, nw, csize, kp, smem, n, grid_out);
+  return launch_icp_w<DPGICP_SEARCH_BRUTE>(ctx, stream, nw, csize, kp, smem, n, grid_out);
 }
 
 /* warps per CTA close to `target` that split `tiles` 32-point tiles evenly (every warp gets
@@ -274,10 +313,14 @@ int balanced_warps(int tiles, int target, int csize = 1) {
   return std::max(1, (warps_total + csize - 1) / csize);
 }
 
-int launch_icp(dpgicp_ctx *ctx, const Store &st, const Batch &b, const dpgicp_params *p, int32_t *corr_out,
+/* the stage chain of batch b over store st, on slot s's stream with s's queue cells and state buffers (b is s's batch, or
+ * the context's scratch batch for the single-pair shapes on the default slot) */
+int launch_icp(dpgicp_slot *s, const Store &st, const Batch &b, const dpgicp_params *p, int32_t *corr_out,
                float *corr_d2, const int32_t *corr_seed = nullptr, int32_t *corr_nn_out = nullptr, int64_t first = 0,
                int64_t count = -1) {
   NvtxRange range("dpgicp: ICP + covariance stage chain");
+  dpgicp_ctx *ctx = s->ctx;
+  cudaStream_t stream = stream_of(s);
   const int div = p->downsample_divisor;
   int n_max = (st.max_count + div - 1) / div;
   int n_cap = ((std::max(n_max, 1) + kTile - 1) / kTile) * kTile;
@@ -294,7 +337,7 @@ int launch_icp(dpgicp_ctx *ctx, const Store &st, const Batch &b, const dpgicp_pa
   kp.order = (b.has_order && whole) ? (const long long *)b.order.p : nullptr;
   kp.results = (dpgicp_result *)b.results.p + first;
   kp.pair_base = first;
-  kp.counters = ctx->d_queue + 8;
+  kp.counters = s->d_queue + 8;
   kp.n_pairs = count;
   kp.n_cap = n_cap;
   kp.max_iterations = p->max_iterations;
@@ -316,7 +359,7 @@ int launch_icp(dpgicp_ctx *ctx, const Store &st, const Batch &b, const dpgicp_pa
   kp.outlier_mode = p->outlier_mode;
   kp.outlier_param = p->outlier_param;
   kp.slot_bytes = (long long)kStateHeader + 12ll * n_cap;
-  if (ctx->gather_world > 1 && corr_out == nullptr && &b == &ctx->batch) {
+  if (ctx->gather_world > 1 && corr_out == nullptr && &b == &ctx->main.batch) {
     if ((b.n_pairs - 1) * (int64_t)ctx->gather_world + ctx->gather_rank >= ctx->gather_n)
       return fail(ctx, DPGICP_E_STATE, "the attached gather buffers are too small for this shard");
     kp.gather_world = ctx->gather_world;
@@ -374,60 +417,60 @@ int launch_icp(dpgicp_ctx *ctx, const Store &st, const Batch &b, const dpgicp_pa
     int next_units = -1;
     KernelParams kq = kp;
     kq.resume = 1;
-    int rcq = launch_stage(ctx, search, shapes[1].warps, shapes[1].csize, kq, smem_of(shapes[1].warps), (int64_t)1 << 40, &next_units);
+    int rcq = launch_stage(ctx, stream, search, shapes[1].warps, shapes[1].csize, kq, smem_of(shapes[1].warps), (int64_t)1 << 40, &next_units);
     if (rcq) return rcq;
     const long long bound = (long long)std::ceil((shapes[1].csize > 1 ? ctx->handover_cluster : ctx->handover_factor) * (double)next_units);
     if (count > bound) break;
     for (int k = 1; k < n_stages; ++k) shapes[k - 1] = shapes[k];
     --n_stages;
   }
-  CU_TRY(ctx, cudaMemsetAsync(ctx->d_queue, 0, 32 * sizeof(unsigned long long), ctx->stream));
+  CU_TRY(ctx, cudaMemsetAsync(s->d_queue, 0, 32 * sizeof(unsigned long long), stream));
   int grid_prev = 0;
-  const bool timing = ctx->stage_timing && corr_out == nullptr;
-  if (timing) { ctx->last_stages = n_stages; CU_TRY(ctx, cudaEventRecord(ctx->stage_ev[0], ctx->stream)); }
+  const bool timing = s->stage_timing && corr_out == nullptr;
+  if (timing) { s->last_stages = n_stages; CU_TRY(ctx, cudaEventRecord(s->stage_ev[0], stream)); }
   if (n_stages > 1) {
     /* every stage can suspend at most one pair per CTA: size the state slots for stage 0's grid */
     int g0 = -1;
-    int rc = launch_stage(ctx, search, shapes[0].warps, shapes[0].csize, kp, smem_of(shapes[0].warps), count, &g0);
+    int rc = launch_stage(ctx, stream, search, shapes[0].warps, shapes[0].csize, kp, smem_of(shapes[0].warps), count, &g0);
     if (rc) return rc;
     for (int k = 0; k < 2; ++k) {
-      if ((rc = reserve(ctx, ctx->state[k], (size_t)g0 * (size_t)kp.slot_bytes))) return rc;
-      if ((rc = reserve(ctx, ctx->susp[k], (size_t)g0 * sizeof(long long)))) return rc;
+      if ((rc = reserve(ctx, s->state[k], (size_t)g0 * (size_t)kp.slot_bytes))) return rc;
+      if ((rc = reserve(ctx, s->susp[k], (size_t)g0 * sizeof(long long)))) return rc;
     }
     kp.slot_cap = g0;
   }
   for (int sidx = 0; sidx < n_stages; ++sidx) {
     KernelParams ks = kp;
-    ks.queue = ctx->d_queue + sidx;
+    ks.queue = s->d_queue + sidx;
     ks.resume = sidx > 0 ? 1 : 0;
     if (sidx > 0) {
-      ks.in_count = reinterpret_cast<const unsigned int *>(ctx->d_queue + 6 + ((sidx - 1) & 1));
-      ks.susp_in = (const long long *)ctx->susp[(sidx - 1) & 1].p;
-      ks.state_in = (const unsigned char *)ctx->state[(sidx - 1) & 1].p;
+      ks.in_count = reinterpret_cast<const unsigned int *>(s->d_queue + 6 + ((sidx - 1) & 1));
+      ks.susp_in = (const long long *)s->susp[(sidx - 1) & 1].p;
+      ks.state_in = (const unsigned char *)s->state[(sidx - 1) & 1].p;
     }
-    ks.finished = ctx->d_queue + 24 + sidx;
+    ks.finished = s->d_queue + 24 + sidx;
     if (sidx + 1 < n_stages) {
       /* hand over once the next stage could run all that is left at once (clusters: exactly; CTAs: a third more,
        * the next stage's own queue-dry rule then takes over) */
       int next_units = -1;
       KernelParams kq = kp;
       kq.resume = 1;                        /* occupancy query for the shape the next stage will really use */
-      int rcq = launch_stage(ctx, search, shapes[sidx + 1].warps, shapes[sidx + 1].csize, kq, smem_of(shapes[sidx + 1].warps), (int64_t)1 << 40, &next_units);
+      int rcq = launch_stage(ctx, stream, search, shapes[sidx + 1].warps, shapes[sidx + 1].csize, kq, smem_of(shapes[sidx + 1].warps), (int64_t)1 << 40, &next_units);
       if (rcq) return rcq;
       ks.handover = (long long)std::ceil((shapes[sidx + 1].csize > 1 ? ctx->handover_cluster : ctx->handover_factor) * (double)next_units);
       if (ctx->handover_factor <= 0.0) ks.handover = (long long)1 << 40;      /* development: the plain queue-dry rule */
-      ks.out_count = reinterpret_cast<unsigned int *>(ctx->d_queue + 6 + (sidx & 1));
-      ks.susp_out = (long long *)ctx->susp[sidx & 1].p;
-      ks.state_out = (unsigned char *)ctx->state[sidx & 1].p;
+      ks.out_count = reinterpret_cast<unsigned int *>(s->d_queue + 6 + (sidx & 1));
+      ks.susp_out = (long long *)s->susp[sidx & 1].p;
+      ks.state_out = (unsigned char *)s->state[sidx & 1].p;
       if (sidx >= 2)      /* the count cell is reused by stage sidx: clear it after stage sidx-1 consumed it */
-        CU_TRY(ctx, cudaMemsetAsync(ctx->d_queue + 6 + (sidx & 1), 0, sizeof(unsigned long long), ctx->stream));
+        CU_TRY(ctx, cudaMemsetAsync(s->d_queue + 6 + (sidx & 1), 0, sizeof(unsigned long long), stream));
     }
     int grid = 0;
     const int64_t max_items = sidx == 0 ? count : (int64_t)grid_prev;
-    int rc = launch_stage(ctx, search, shapes[sidx].warps, shapes[sidx].csize, ks, smem_of(shapes[sidx].warps), max_items, &grid);
+    int rc = launch_stage(ctx, stream, search, shapes[sidx].warps, shapes[sidx].csize, ks, smem_of(shapes[sidx].warps), max_items, &grid);
     if (rc) return rc;
     grid_prev = grid;
-    if (timing) CU_TRY(ctx, cudaEventRecord(ctx->stage_ev[sidx + 1], ctx->stream));
+    if (timing) CU_TRY(ctx, cudaEventRecord(s->stage_ev[sidx + 1], stream));
   }
   return DPGICP_OK;
 }
@@ -447,7 +490,7 @@ int finish_store(dpgicp_ctx *ctx, Store &st, int n_scans) {
     st.n_scans = 0;
     return fail(ctx, DPGICP_E_RANGE, "scan store holds a non-finite point or |coordinate| > DPGICP_MAX_ABS_COORD");
   }
-  return DPGICP_OK;
+  return mark_written(ctx);
 }
 
 /* arguments of a ragged cloud upload (dpgicp_upload_scans / dpgicp_append_scans): the largest scan and the point total */
@@ -494,7 +537,7 @@ int upload_scans_into(dpgicp_ctx *ctx, Store &st, const void *points, size_t str
   return finish_store(ctx, st, n_scans);
 }
 
-int set_pairs_into(dpgicp_ctx *ctx, const Store &st, Batch &b, const int32_t *src, const int32_t *tgt,
+int set_pairs_into(dpgicp_ctx *ctx, cudaStream_t stream, const Store &st, Batch &b, const int32_t *src, const int32_t *tgt,
                    const float *guess, const float *T_direct, int64_t n) {
   if (n < 0 || (n > 0 && (!src || !tgt || (!guess && !T_direct))))
     return fail(ctx, DPGICP_E_INVALID, "bad pair arguments");
@@ -535,8 +578,8 @@ int set_pairs_into(dpgicp_ctx *ctx, const Store &st, Batch &b, const int32_t *sr
   if ((rc = reserve(ctx, b.tasks, sizeof(PairTask) * (size_t)std::max<int64_t>(n, 1)))) return rc;
   if ((rc = reserve(ctx, b.results, sizeof(dpgicp_result) * (size_t)std::max<int64_t>(n, 1)))) return rc;
   if (n > 0)
-    CU_TRY(ctx, cudaMemcpyAsync(b.tasks.p, b.h_tasks, sizeof(PairTask) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-  CU_TRY(ctx, cudaEventRecord(b.h_tasks_free, ctx->stream));
+    CU_TRY(ctx, cudaMemcpyAsync(b.tasks.p, b.h_tasks, sizeof(PairTask) * (size_t)n, cudaMemcpyHostToDevice, stream));
+  CU_TRY(ctx, cudaEventRecord(b.h_tasks_free, stream));
   b.n_pairs = n;
   b.has_order = false;
   b.max_scan = -1;
@@ -755,7 +798,7 @@ int enumerate_into(dpgicp_ctx *ctx, const Nodes &N, Batch &b, int mode, float r_
 }
 
 /* the pair list of a batch back on the host */
-int fetch_pairs_from(dpgicp_ctx *ctx, const Batch &b, int32_t *src, int32_t *tgt, float *T, int64_t n) {
+int fetch_pairs_from(dpgicp_ctx *ctx, cudaStream_t stream, const Batch &b, int32_t *src, int32_t *tgt, float *T, int64_t n) {
   if (n < 0 || n > b.n_pairs) return fail(ctx, DPGICP_E_INVALID, "bad fetch arguments");
   if (n == 0) return DPGICP_OK;
   int rc;
@@ -764,21 +807,21 @@ int fetch_pairs_from(dpgicp_ctx *ctx, const Batch &b, int32_t *src, int32_t *tgt
   float4 *d_T = (float4 *)((char *)ctx->stage.p + (((size_t)n * 8 + 15) & ~(size_t)15));
   const int threads = 256;
   const long long blocks = (n + threads - 1) / threads;
-  unpack_tasks_kernel<<<(unsigned)blocks, threads, 0, ctx->stream>>>((const PairTask *)b.tasks.p, (long long)n, src ? d_src : nullptr,
+  unpack_tasks_kernel<<<(unsigned)blocks, threads, 0, stream>>>((const PairTask *)b.tasks.p, (long long)n, src ? d_src : nullptr,
                                                                    tgt ? d_tgt : nullptr, T ? d_T : nullptr);
   ctx->launches++;
   CU_TRY(ctx, cudaGetLastError());
-  if (src) CU_TRY(ctx, cudaMemcpyAsync(src, d_src, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (tgt) CU_TRY(ctx, cudaMemcpyAsync(tgt, d_tgt, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (T) CU_TRY(ctx, cudaMemcpyAsync(T, d_T, (size_t)n * 16, cudaMemcpyDeviceToHost, ctx->stream));
-  CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  if (src) CU_TRY(ctx, cudaMemcpyAsync(src, d_src, (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
+  if (tgt) CU_TRY(ctx, cudaMemcpyAsync(tgt, d_tgt, (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
+  if (T) CU_TRY(ctx, cudaMemcpyAsync(T, d_T, (size_t)n * 16, cudaMemcpyDeviceToHost, stream));
+  CU_TRY(ctx, cudaStreamSynchronize(stream));
   return DPGICP_OK;
 }
 
 /* Room for n_new more rows of at least need_pitch (even) points behind the rows of the store, every existing row kept
  * (the append path).  Rows and counts grow by doubling, so n one-scan appends copy O(n) rows in total; a scan longer
- * than the pitch re-pitches the kept rows on the device.  A buffer that moves is freed only after the stream has
- * drained: the copy out of it, and any dpgicp_run enqueued before the append, read it.  On failure the store is as
+ * than the pitch re-pitches the kept rows on the device.  A buffer that moves is freed only after the context's stream
+ * and every slot's stream have drained: the copy out of it, and any run enqueued before the append, read it.  On failure the store is as
  * it was. */
 int grow_store(dpgicp_ctx *ctx, Store &st, int n_new, int need_pitch) {
   const int n_old = st.n_scans;
@@ -824,6 +867,7 @@ int grow_store(dpgicp_ctx *ctx, Store &st, int n_new, int need_pitch) {
                 "cudaMemcpyAsync (scan counts)");
   }
   if (!rc && (move_rows || move_count)) rc = cuda(cudaStreamSynchronize(ctx->stream), "cudaStreamSynchronize");
+  if (!rc && (move_rows || move_count)) rc = drain_slots(ctx);
   if (rc) {
     cudaStreamSynchronize(ctx->stream);
     release(nr); release(nc);
@@ -853,7 +897,42 @@ int finish_append(dpgicp_ctx *ctx, Store &st, int n_new) {
   if (first == 0) st.max_count = 0;
   for (size_t k = first; k < st.h_count.size(); ++k) st.max_count = std::max(st.max_count, st.h_count[k]);
   st.n_scans = (int32_t)st.h_count.size();
-  return DPGICP_OK;
+  return mark_written(ctx);
+}
+
+/* the device cells and events of a slot (own_stream: a stream of its own, else the context's) */
+cudaError_t slot_init(dpgicp_slot *s, dpgicp_ctx *ctx, bool own_stream) {
+  s->ctx = ctx;
+  cudaError_t e = cudaMalloc((void **)&s->d_queue, 32 * sizeof(unsigned long long));
+  for (cudaEvent_t &ev : s->stage_ev)
+    if (e == cudaSuccess) e = cudaEventCreate(&ev);
+  if (e == cudaSuccess && own_stream) e = cudaStreamCreateWithFlags(&s->own, cudaStreamNonBlocking);
+  return e;
+}
+
+void release_batch(Batch &b) {
+  release(b.tasks); release(b.results); release(b.order);
+  if (b.h_tasks) cudaFreeHost(b.h_tasks);
+  if (b.h_tasks_free) cudaEventDestroy(b.h_tasks_free);
+  b.h_tasks = nullptr; b.h_tasks_free = nullptr;
+}
+
+/* after the slot's stream has drained */
+void slot_release(dpgicp_slot *s) {
+  release_batch(s->batch);
+  for (int k = 0; k < 2; ++k) { release(s->state[k]); release(s->susp[k]); }
+  if (s->d_queue) cudaFree(s->d_queue);
+  for (cudaEvent_t e : s->stage_ev) if (e) cudaEventDestroy(e);
+  if (s->own) cudaStreamDestroy(s->own);
+}
+
+/* slot handles a caller holds: a destroyed (or never created) handle is refused, not followed */
+std::mutex g_slots_mutex;
+std::set<const dpgicp_slot *> g_slots;
+
+dpgicp_slot *live(dpgicp_slot *s) {
+  std::lock_guard<std::mutex> lock(g_slots_mutex);
+  return s && g_slots.count(s) ? s : nullptr;
 }
 
 }  // namespace
@@ -912,13 +991,12 @@ int dpgicp_create(int device, dpgicp_ctx **out) {
   }
   ctx->sm_count = prop.multiProcessorCount;
   if ((e = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking)) != cudaSuccess ||
-      (e = cudaMalloc((void **)&ctx->d_queue, 32 * sizeof(unsigned long long))) != cudaSuccess ||
-      (e = cudaMalloc((void **)&ctx->d_bad, sizeof(int))) != cudaSuccess) {
+      (e = cudaMalloc((void **)&ctx->d_bad, sizeof(int))) != cudaSuccess ||
+      (e = cudaEventCreateWithFlags(&ctx->written, cudaEventDisableTiming)) != cudaSuccess ||
+      (e = slot_init(&ctx->main, ctx, false)) != cudaSuccess) {
     delete ctx;
     return fail(nullptr, DPGICP_E_CUDA, cudaGetErrorString(e));
   }
-  for (cudaEvent_t &ev : ctx->stage_ev)
-    if ((e = cudaEventCreate(&ev)) != cudaSuccess) { delete ctx; return fail(nullptr, DPGICP_E_CUDA, cudaGetErrorString(e)); }
   if (const char *w = std::getenv("DPGICP_WARPS")) ctx->force_warps = std::atoi(w);
   if (const char *c = std::getenv("DPGICP_CTAS_PER_SM")) ctx->force_ctas_per_sm = std::atoi(c);
   if (const char *c = std::getenv("DPGICP_HANDOVER")) {
@@ -942,14 +1020,12 @@ int dpgicp_create(int device, dpgicp_ctx **out) {
 void dpgicp_destroy(dpgicp_ctx *ctx) {
   if (!ctx) return;
   cudaSetDevice(ctx->device);
+  while (!ctx->slots.empty()) dpgicp_slot_destroy(ctx->slots.back());
   cudaStreamSynchronize(ctx->stream);
   for (Store *s : {&ctx->store, &ctx->scratch_store}) { release(s->rows); release(s->count); }
-  for (Batch *b : {&ctx->batch, &ctx->scratch_batch}) {
-    release(b->tasks); release(b->results); release(b->order);
-    if (b->h_tasks) cudaFreeHost(b->h_tasks);
-    if (b->h_tasks_free) cudaEventDestroy(b->h_tasks_free);
-  }
-  for (cudaEvent_t e : ctx->stage_ev) if (e) cudaEventDestroy(e);
+  release_batch(ctx->scratch_batch);
+  slot_release(&ctx->main);
+  if (ctx->written) cudaEventDestroy(ctx->written);
   release(ctx->nodes.xy); release(ctx->nodes.aux); release(ctx->nodes.pass); release(ctx->nodes.boxes);
   release(ctx->list_nodes.xy); release(ctx->list_nodes.aux); release(ctx->list_nodes.pass); release(ctx->list_nodes.boxes);
   release(ctx->enum_cnt); release(ctx->enum_amb); release(ctx->d_pair);
@@ -957,8 +1033,6 @@ void dpgicp_destroy(dpgicp_ctx *ctx) {
   gather_close(ctx);
   release(ctx->gather);
   release(ctx->stage); release(ctx->offsets); release(ctx->misc); release(ctx->corr); release(ctx->trig);
-  for (int k = 0; k < 2; ++k) { release(ctx->state[k]); release(ctx->susp[k]); }
-  if (ctx->d_queue) cudaFree(ctx->d_queue);
   if (ctx->d_bad) cudaFree(ctx->d_bad);
   if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
   if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -992,7 +1066,8 @@ int dpgicp_synchronize(dpgicp_ctx *ctx) {
 int dpgicp_upload_scans(dpgicp_ctx *ctx, const void *points, size_t stride, const int64_t *offsets, int32_t n_scans) {
   if (!ctx) return DPGICP_E_INVALID;
   CU_TRY(ctx, cudaSetDevice(ctx->device));
-  ctx->batch.n_pairs = 0;
+  int rc = replace_store(ctx);
+  if (rc) return rc;
   return upload_scans_into(ctx, ctx->store, points, stride, offsets, n_scans);
 }
 
@@ -1004,9 +1079,9 @@ int dpgicp_upload_ranges(dpgicp_ctx *ctx, const float *ranges, int32_t n_scans, 
   if (n_scans < 0 || n_beams < 2 || (n_scans > 0 && !ranges)) return fail(ctx, DPGICP_E_INVALID, "bad range-scan arguments");
   if (n_beams > DPGICP_MAX_POINTS) return fail(ctx, DPGICP_E_TOOBIG, "n_beams exceeds DPGICP_MAX_POINTS");
   Store &st = ctx->store;
-  ctx->batch.n_pairs = 0;
+  int rc = replace_store(ctx);
+  if (rc) return rc;
   const int pitch = (n_beams + 1) & ~1;
-  int rc;
   if ((rc = reserve(ctx, st.rows, sizeof(float2) * (size_t)pitch * (size_t)std::max(n_scans, 1)))) return rc;
   if ((rc = reserve(ctx, st.count, sizeof(int32_t) * (size_t)std::max(n_scans, 1)))) return rc;
   if ((rc = reserve(ctx, ctx->stage, sizeof(float) * (size_t)n_scans * (size_t)n_beams + 16))) return rc;
@@ -1042,9 +1117,9 @@ int dpgicp_upload_ranges_subset(dpgicp_ctx *ctx, const float *ranges, int32_t n_
     if (scan_ids[k] < 0 || scan_ids[k] >= n_scans_total)
       return fail(ctx, DPGICP_E_INVALID, "scan id out of range at position " + std::to_string(k));
   Store &st = ctx->store;
-  ctx->batch.n_pairs = 0;
+  int rc = replace_store(ctx);
+  if (rc) return rc;
   const int pitch = (n_beams + 1) & ~1;
-  int rc;
   if ((rc = reserve(ctx, st.rows, sizeof(float2) * (size_t)pitch * (size_t)std::max(n_ids, 1)))) return rc;
   if ((rc = reserve(ctx, st.count, sizeof(int32_t) * (size_t)std::max(n_ids, 1)))) return rc;
   st.pitch = pitch;
@@ -1168,17 +1243,22 @@ int dpgicp_download_scan(dpgicp_ctx *ctx, int32_t scan, float *xy, int32_t *n_po
   return DPGICP_OK;
 }
 
-int dpgicp_set_pairs(dpgicp_ctx *ctx, const int32_t *src, const int32_t *tgt, const float *guess, int64_t n) {
-  if (!ctx) return DPGICP_E_INVALID;
+static int set_pairs_slot(dpgicp_slot *s, const int32_t *src, const int32_t *tgt, const float *guess, int64_t n) {
+  dpgicp_ctx *ctx = s->ctx;
   NvtxRange range("dpgicp: pair list");
   CU_TRY(ctx, cudaSetDevice(ctx->device));
-  return set_pairs_into(ctx, ctx->store, ctx->batch, src, tgt, guess, nullptr, n);
+  return set_pairs_into(ctx, stream_of(s), ctx->store, s->batch, src, tgt, guess, nullptr, n);
 }
 
-int dpgicp_set_pair_cost_hints(dpgicp_ctx *ctx, const float *hints, int64_t n) {
+int dpgicp_set_pairs(dpgicp_ctx *ctx, const int32_t *src, const int32_t *tgt, const float *guess, int64_t n) {
   if (!ctx) return DPGICP_E_INVALID;
+  return set_pairs_slot(&ctx->main, src, tgt, guess, n);
+}
+
+static int set_pair_cost_hints_slot(dpgicp_slot *s, const float *hints, int64_t n) {
+  dpgicp_ctx *ctx = s->ctx;
   CU_TRY(ctx, cudaSetDevice(ctx->device));
-  Batch &b = ctx->batch;
+  Batch &b = s->batch;
   if (!hints) { b.has_order = false; return DPGICP_OK; }
   if (n != b.n_pairs) return fail(ctx, DPGICP_E_INVALID, "hint count differs from the pair list");
   if (n == 0) return DPGICP_OK;
@@ -1198,47 +1278,63 @@ int dpgicp_set_pair_cost_hints(dpgicp_ctx *ctx, const float *hints, int64_t n) {
   std::sort(order.begin() + head, order.end());
   int rc;
   if ((rc = reserve(ctx, b.order, sizeof(long long) * (size_t)n))) return rc;
-  CU_TRY(ctx, cudaMemcpyAsync(b.order.p, order.data(), sizeof(long long) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-  CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));        /* `order` goes out of scope */
+  CU_TRY(ctx, cudaMemcpyAsync(b.order.p, order.data(), sizeof(long long) * (size_t)n, cudaMemcpyHostToDevice, stream_of(s)));
+  CU_TRY(ctx, cudaStreamSynchronize(stream_of(s)));        /* `order` goes out of scope */
   b.has_order = true;
   return DPGICP_OK;
 }
 
+int dpgicp_set_pair_cost_hints(dpgicp_ctx *ctx, const float *hints, int64_t n) {
+  if (!ctx) return DPGICP_E_INVALID;
+  return set_pair_cost_hints_slot(&ctx->main, hints, n);
+}
+
+/* slot s's whole batch, or its pairs [first, first + count); a slot with a stream of its own first waits
+ * for the context's writes enqueued before (store, enumerated list) */
+static int run_slot(dpgicp_slot *s, const dpgicp_params *params, bool whole, int64_t first, int64_t count) {
+  dpgicp_ctx *ctx = s->ctx;
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  const int rc = check_params(ctx, params);
+  if (rc) return rc;
+  const Batch &b = s->batch;
+  if (whole && b.n_pairs == 0) return DPGICP_OK;           /* an empty batch is valid and does nothing */
+  if (b.n_pairs < 0) return fail(ctx, DPGICP_E_STATE, "no pair list set");
+  if (!whole) {
+    if (first < 0 || count < 0 || first + count > b.n_pairs) return fail(ctx, DPGICP_E_INVALID, "pair range outside the batch");
+    if (count == 0) return DPGICP_OK;
+  }
+  if (ctx->store.n_scans <= 0) return fail(ctx, DPGICP_E_STATE, "no scans uploaded");
+  if (b.max_scan >= ctx->store.n_scans)
+    return fail(ctx, DPGICP_E_STATE, "the enumerated pair list refers to nodes without a scan in the store (node k owns scan k)");
+  if (s->own) CU_TRY(ctx, cudaStreamWaitEvent(s->own, ctx->written, 0));
+  return whole ? launch_icp(s, ctx->store, b, params, nullptr, nullptr)
+               : launch_icp(s, ctx->store, b, params, nullptr, nullptr, nullptr, nullptr, first, count);
+}
+
 int dpgicp_run(dpgicp_ctx *ctx, const dpgicp_params *params) {
   if (!ctx) return DPGICP_E_INVALID;
-  CU_TRY(ctx, cudaSetDevice(ctx->device));
-  int rc = check_params(ctx, params);
-  if (rc) return rc;
-  if (ctx->batch.n_pairs == 0) return DPGICP_OK;               /* an empty batch is valid and does nothing */
-  if (ctx->batch.n_pairs < 0) return fail(ctx, DPGICP_E_STATE, "no pair list set");
-  if (ctx->store.n_scans <= 0) return fail(ctx, DPGICP_E_STATE, "no scans uploaded");
-  if (ctx->batch.max_scan >= ctx->store.n_scans)
-    return fail(ctx, DPGICP_E_STATE, "the enumerated pair list refers to nodes without a scan in the store (node k owns scan k)");
-  return launch_icp(ctx, ctx->store, ctx->batch, params, nullptr, nullptr);
+  return run_slot(&ctx->main, params, true, 0, 0);
 }
 
 int dpgicp_run_range(dpgicp_ctx *ctx, const dpgicp_params *params, int64_t first, int64_t count) {
   if (!ctx) return DPGICP_E_INVALID;
+  return run_slot(&ctx->main, params, false, first, count);
+}
+
+static int fetch_results_slot(dpgicp_slot *s, dpgicp_result *out, int64_t first, int64_t count) {
+  dpgicp_ctx *ctx = s->ctx;
   CU_TRY(ctx, cudaSetDevice(ctx->device));
-  int rc = check_params(ctx, params);
-  if (rc) return rc;
-  if (first < 0 || count < 0 || first + count > ctx->batch.n_pairs) return fail(ctx, DPGICP_E_INVALID, "pair range outside the batch");
-  if (count == 0) return DPGICP_OK;
-  if (ctx->store.n_scans <= 0) return fail(ctx, DPGICP_E_STATE, "no scans uploaded");
-  if (ctx->batch.max_scan >= ctx->store.n_scans)
-    return fail(ctx, DPGICP_E_STATE, "the enumerated pair list refers to nodes without a scan in the store (node k owns scan k)");
-  return launch_icp(ctx, ctx->store, ctx->batch, params, nullptr, nullptr, nullptr, nullptr, first, count);
+  if (first < 0 || count < 0 || first + count > s->batch.n_pairs || (count > 0 && !out)) return fail(ctx, DPGICP_E_INVALID, "bad fetch arguments");
+  if (count > 0)
+    CU_TRY(ctx, cudaMemcpyAsync(out, (const dpgicp_result *)s->batch.results.p + first, sizeof(dpgicp_result) * (size_t)count,
+                                cudaMemcpyDeviceToHost, stream_of(s)));
+  CU_TRY(ctx, cudaStreamSynchronize(stream_of(s)));
+  return DPGICP_OK;
 }
 
 int dpgicp_fetch_results_range(dpgicp_ctx *ctx, dpgicp_result *out, int64_t first, int64_t count) {
   if (!ctx) return DPGICP_E_INVALID;
-  CU_TRY(ctx, cudaSetDevice(ctx->device));
-  if (first < 0 || count < 0 || first + count > ctx->batch.n_pairs || (count > 0 && !out)) return fail(ctx, DPGICP_E_INVALID, "bad fetch arguments");
-  if (count > 0)
-    CU_TRY(ctx, cudaMemcpyAsync(out, (const dpgicp_result *)ctx->batch.results.p + first, sizeof(dpgicp_result) * (size_t)count,
-                                cudaMemcpyDeviceToHost, ctx->stream));
-  CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  return DPGICP_OK;
+  return fetch_results_slot(&ctx->main, out, first, count);
 }
 
 int dpgicp_gather_fetch_range(dpgicp_ctx *ctx, dpgicp_result *out, int64_t first, int64_t count) {
@@ -1257,32 +1353,31 @@ int dpgicp_gather_fetch_range(dpgicp_ctx *ctx, dpgicp_result *out, int64_t first
 int dpgicp_fetch_results(dpgicp_ctx *ctx, dpgicp_result *out, int64_t n) {
   if (!ctx) return DPGICP_E_INVALID;
   NvtxRange range("dpgicp: fetch records");
+  return fetch_results_slot(&ctx->main, out, 0, n);
+}
+
+static int fetch_factors_slot(dpgicp_slot *s, dpgicp_factor *out, int64_t n) {
+  dpgicp_ctx *ctx = s->ctx;
   CU_TRY(ctx, cudaSetDevice(ctx->device));
-  if (n < 0 || n > ctx->batch.n_pairs || (n > 0 && !out)) return fail(ctx, DPGICP_E_INVALID, "bad fetch arguments");
-  if (n > 0)
-    CU_TRY(ctx, cudaMemcpyAsync(out, ctx->batch.results.p, sizeof(dpgicp_result) * (size_t)n, cudaMemcpyDeviceToHost,
-                                ctx->stream));
-  CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  if (n < 0 || n > s->batch.n_pairs || (n > 0 && !out)) return fail(ctx, DPGICP_E_INVALID, "bad fetch arguments");
+  if (n == 0) { CU_TRY(ctx, cudaStreamSynchronize(stream_of(s))); return DPGICP_OK; }
+  int rc;
+  if ((rc = reserve(ctx, ctx->stage, sizeof(dpgicp_factor) * (size_t)n))) return rc;
+  const int threads = 128;
+  const long long blocks = (n + threads - 1) / threads;
+  factors_kernel<<<(unsigned)blocks, threads, 0, stream_of(s)>>>((const dpgicp_result *)s->batch.results.p,
+                                                              (const PairTask *)s->batch.tasks.p, (long long)n,
+                                                              (dpgicp_factor *)ctx->stage.p);
+  ctx->launches++;
+  CU_TRY(ctx, cudaGetLastError());
+  CU_TRY(ctx, cudaMemcpyAsync(out, ctx->stage.p, sizeof(dpgicp_factor) * (size_t)n, cudaMemcpyDeviceToHost, stream_of(s)));
+  CU_TRY(ctx, cudaStreamSynchronize(stream_of(s)));
   return DPGICP_OK;
 }
 
 int dpgicp_fetch_factors(dpgicp_ctx *ctx, dpgicp_factor *out, int64_t n) {
   if (!ctx) return DPGICP_E_INVALID;
-  CU_TRY(ctx, cudaSetDevice(ctx->device));
-  if (n < 0 || n > ctx->batch.n_pairs || (n > 0 && !out)) return fail(ctx, DPGICP_E_INVALID, "bad fetch arguments");
-  if (n == 0) { CU_TRY(ctx, cudaStreamSynchronize(ctx->stream)); return DPGICP_OK; }
-  int rc;
-  if ((rc = reserve(ctx, ctx->stage, sizeof(dpgicp_factor) * (size_t)n))) return rc;
-  const int threads = 128;
-  const long long blocks = (n + threads - 1) / threads;
-  factors_kernel<<<(unsigned)blocks, threads, 0, ctx->stream>>>((const dpgicp_result *)ctx->batch.results.p,
-                                                              (const PairTask *)ctx->batch.tasks.p, (long long)n,
-                                                              (dpgicp_factor *)ctx->stage.p);
-  ctx->launches++;
-  CU_TRY(ctx, cudaGetLastError());
-  CU_TRY(ctx, cudaMemcpyAsync(out, ctx->stage.p, sizeof(dpgicp_factor) * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
-  CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  return DPGICP_OK;
+  return fetch_factors_slot(&ctx->main, out, n);
 }
 
 static int gather_export_impl(dpgicp_ctx *ctx, int64_t n_global, int64_t n_alloc, unsigned char *handle_out) {
@@ -1408,27 +1503,32 @@ int dpgicp_gather_device_ptr(dpgicp_ctx *ctx, void **out_ptr, int64_t *out_n) {
 
 int dpgicp_results_device_ptr(dpgicp_ctx *ctx, void **out_ptr, int64_t *out_n) {
   if (!ctx || !out_ptr || !out_n) return DPGICP_E_INVALID;
-  *out_ptr = ctx->batch.results.p;
-  *out_n = ctx->batch.n_pairs;
+  *out_ptr = ctx->main.batch.results.p;
+  *out_n = ctx->main.batch.n_pairs;
+  return DPGICP_OK;
+}
+
+static int last_run_counters_slot(dpgicp_slot *s, uint64_t counters[8]) {
+  dpgicp_ctx *ctx = s->ctx;
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  unsigned long long h[8];
+  CU_TRY(ctx, cudaMemcpyAsync(h, s->d_queue + 8, sizeof(h), cudaMemcpyDeviceToHost, stream_of(s)));
+  CU_TRY(ctx, cudaStreamSynchronize(stream_of(s)));
+  for (int k = 0; k < 8; ++k) counters[k] = h[k];
+  counters[4] = ctx->launches;
   return DPGICP_OK;
 }
 
 int dpgicp_last_run_counters(dpgicp_ctx *ctx, uint64_t counters[8]) {
   if (!ctx || !counters) return DPGICP_E_INVALID;
-  CU_TRY(ctx, cudaSetDevice(ctx->device));
-  unsigned long long h[8];
-  CU_TRY(ctx, cudaMemcpyAsync(h, ctx->d_queue + 8, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-  CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  for (int k = 0; k < 8; ++k) counters[k] = h[k];
-  counters[4] = ctx->launches;
-  return DPGICP_OK;
+  return last_run_counters_slot(&ctx->main, counters);
 }
 
 #ifdef DPGICP_PHASE_TIMING
 /* development builds only: cycles thread 0 spent in each phase of the pass loop, summed over pairs */
 int dpgicp_debug_phase_counters(dpgicp_ctx *ctx, uint64_t out[8]) {
   unsigned long long h[8];
-  CU_TRY(ctx, cudaMemcpyAsync(h, ctx->d_queue + 16, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+  CU_TRY(ctx, cudaMemcpyAsync(h, ctx->main.d_queue + 16, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
   CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
   for (int k = 0; k < 8; ++k) out[k] = h[k];
   return DPGICP_OK;
@@ -1466,8 +1566,8 @@ int dpgicp_single_pair(dpgicp_ctx *ctx, const void *source, int32_t n_source, co
   if (!guess || !out) return fail(ctx, DPGICP_E_INVALID, "guess/out is NULL");
   if ((rc = two_cloud_store(ctx, source, n_source, target, n_target, stride))) return rc;
   const int32_t s = 0, t = 1;
-  if ((rc = set_pairs_into(ctx, ctx->scratch_store, ctx->scratch_batch, &s, &t, guess, nullptr, 1))) return rc;
-  if ((rc = launch_icp(ctx, ctx->scratch_store, ctx->scratch_batch, params, nullptr, nullptr))) return rc;
+  if ((rc = set_pairs_into(ctx, ctx->stream, ctx->scratch_store, ctx->scratch_batch, &s, &t, guess, nullptr, 1))) return rc;
+  if ((rc = launch_icp(&ctx->main, ctx->scratch_store, ctx->scratch_batch, params, nullptr, nullptr))) return rc;
   CU_TRY(ctx, cudaMemcpyAsync(out, ctx->scratch_batch.results.p, sizeof(dpgicp_result), cudaMemcpyDeviceToHost,
                               ctx->stream));
   CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1487,7 +1587,7 @@ int dpgicp_correspondences_seeded(dpgicp_ctx *ctx, const void *source, int32_t n
       if (prev_nn[i] < -1 || prev_nn[i] >= n_target) return fail(ctx, DPGICP_E_INVALID, "prev_nn out of range at point " + std::to_string(i));
   if ((rc = two_cloud_store(ctx, source, n_source, target, n_target, stride))) return rc;
   const int32_t s = 0, t = 1;
-  if ((rc = set_pairs_into(ctx, ctx->scratch_store, ctx->scratch_batch, &s, &t, nullptr, T, 1))) return rc;
+  if ((rc = set_pairs_into(ctx, ctx->stream, ctx->scratch_store, ctx->scratch_batch, &s, &t, nullptr, T, 1))) return rc;
   const size_t n = (size_t)std::max(n_source, 1);
   if ((rc = reserve(ctx, ctx->corr, n * 16))) return rc;
   dpgicp_params p = *params;
@@ -1498,7 +1598,7 @@ int dpgicp_correspondences_seeded(dpgicp_ctx *ctx, const void *source, int32_t n
   int32_t *d_nn = (int32_t *)((char *)ctx->corr.p + n * 12);
   if (prev_nn && n_source > 0)
     CU_TRY(ctx, cudaMemcpyAsync(d_seed, prev_nn, sizeof(int32_t) * (size_t)n_source, cudaMemcpyHostToDevice, ctx->stream));
-  if ((rc = launch_icp(ctx, ctx->scratch_store, ctx->scratch_batch, &p, d_corr, d_d2, prev_nn ? d_seed : nullptr, nn_out ? d_nn : nullptr))) return rc;
+  if ((rc = launch_icp(&ctx->main, ctx->scratch_store, ctx->scratch_batch, &p, d_corr, d_d2, prev_nn ? d_seed : nullptr, nn_out ? d_nn : nullptr))) return rc;
   if (n_source > 0) {
     CU_TRY(ctx, cudaMemcpyAsync(corr_tgt, d_corr, sizeof(int32_t) * (size_t)n_source, cudaMemcpyDeviceToHost, ctx->stream));
     CU_TRY(ctx, cudaMemcpyAsync(corr_d2, d_d2, sizeof(float) * (size_t)n_source, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1633,7 +1733,7 @@ int dpgicp_enumerate_pairs(dpgicp_ctx *ctx, const float *node_xy, const int32_t 
     ctx->scratch_batch.n_pairs = 0;
     return fail(ctx, DPGICP_E_TOOBIG, "pair capacity too small; required count returned in *n_pairs");
   }
-  rc = fetch_pairs_from(ctx, ctx->scratch_batch, src, tgt, nullptr, total);
+  rc = fetch_pairs_from(ctx, ctx->stream, ctx->scratch_batch, src, tgt, nullptr, total);
   ctx->scratch_batch.n_pairs = 0;
   return rc;
 }
@@ -1645,27 +1745,38 @@ int dpgicp_set_nodes(dpgicp_ctx *ctx, const float *pose, const int32_t *pass, in
   return set_nodes_impl(ctx, ctx->nodes, pose, pass, n, false);
 }
 
-int dpgicp_enumerate_pairs_device(dpgicp_ctx *ctx, int32_t mode, float r_same, float r_other, int32_t rank, int32_t world,
-                                  int64_t *n_total, int64_t *n_local) {
-  if (!ctx) return DPGICP_E_INVALID;
+/* enumeration into slot s: on the context's stream (synchronous, as the host re-derives guesses), after the slot's own
+ * work has drained (its list and records are rewritten); the slot's later runs follow it through ctx->written */
+static int enumerate_slot(dpgicp_slot *s, int32_t mode, float r_same, float r_other, int32_t rank, int32_t world,
+                          int64_t *n_total, int64_t *n_local) {
+  dpgicp_ctx *ctx = s->ctx;
   NvtxRange range("dpgicp: enumerate pairs (device)");
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   if (mode != DPGICP_ENUM_REOPTIMIZE && mode != DPGICP_ENUM_ONLINE) return fail(ctx, DPGICP_E_INVALID, "mode must be DPGICP_ENUM_REOPTIMIZE or DPGICP_ENUM_ONLINE");
   if (world < 1 || rank < 0 || rank >= world) return fail(ctx, DPGICP_E_INVALID, "bad shard arguments");
   if (!(r_same >= 0.0f) || !(r_other >= 0.0f)) return fail(ctx, DPGICP_E_INVALID, "radii must be >= 0");
+  if (s->own) CU_TRY(ctx, cudaStreamSynchronize(s->own));
   if (ctx->nodes.n <= 0) {
     if (n_total) *n_total = 0;
     if (n_local) *n_local = 0;
-    ctx->batch.n_pairs = 0;
+    s->batch.n_pairs = 0;
     return DPGICP_OK;
   }
-  return enumerate_into(ctx, ctx->nodes, ctx->batch, mode, r_same, r_other, rank, world, n_total, n_local);
+  int rc = enumerate_into(ctx, ctx->nodes, s->batch, mode, r_same, r_other, rank, world, n_total, n_local);
+  if (rc) return rc;
+  return s->own ? mark_written(ctx) : DPGICP_OK;
+}
+
+int dpgicp_enumerate_pairs_device(dpgicp_ctx *ctx, int32_t mode, float r_same, float r_other, int32_t rank, int32_t world,
+                                  int64_t *n_total, int64_t *n_local) {
+  if (!ctx) return DPGICP_E_INVALID;
+  return enumerate_slot(&ctx->main, mode, r_same, r_other, rank, world, n_total, n_local);
 }
 
 int dpgicp_fetch_pairs(dpgicp_ctx *ctx, int32_t *src, int32_t *tgt, float *T, int64_t n) {
   if (!ctx) return DPGICP_E_INVALID;
   CU_TRY(ctx, cudaSetDevice(ctx->device));
-  return fetch_pairs_from(ctx, ctx->batch, src, tgt, T, n);
+  return fetch_pairs_from(ctx, ctx->stream, ctx->main.batch, src, tgt, T, n);
 }
 
 int dpgicp_convert_ranges_device(dpgicp_ctx *ctx, const float *d_ranges, int32_t n_scans, int32_t n_beams, float angle_min,
@@ -1675,9 +1786,9 @@ int dpgicp_convert_ranges_device(dpgicp_ctx *ctx, const float *d_ranges, int32_t
   if (n_scans < 0 || n_beams < 2 || (n_scans > 0 && !d_ranges)) return fail(ctx, DPGICP_E_INVALID, "bad range-scan arguments");
   if (n_beams > DPGICP_MAX_POINTS) return fail(ctx, DPGICP_E_TOOBIG, "n_beams exceeds DPGICP_MAX_POINTS");
   Store &st = ctx->store;
-  ctx->batch.n_pairs = 0;
+  int rc = replace_store(ctx);
+  if (rc) return rc;
   const int pitch = (n_beams + 1) & ~1;
-  int rc;
   if ((rc = reserve(ctx, st.rows, sizeof(float2) * (size_t)pitch * (size_t)std::max(n_scans, 1)))) return rc;
   if ((rc = reserve(ctx, st.count, sizeof(int32_t) * (size_t)std::max(n_scans, 1)))) return rc;
   st.pitch = pitch;
@@ -1699,8 +1810,8 @@ int dpgicp_convert_ranges_device(dpgicp_ctx *ctx, const float *d_ranges, int32_t
 
 int dpgicp_enable_stage_timing(dpgicp_ctx *ctx, int32_t on) {
   if (!ctx) return DPGICP_E_INVALID;
-  ctx->stage_timing = on != 0;
-  ctx->last_stages = 0;
+  ctx->main.stage_timing = on != 0;
+  ctx->main.last_stages = 0;
   return DPGICP_OK;
 }
 
@@ -1709,10 +1820,10 @@ int dpgicp_last_run_stage_ms(dpgicp_ctx *ctx, float stage_ms[8], int32_t *n_stag
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   *n_stages = 0;
   for (int k = 0; k < 8; ++k) stage_ms[k] = 0.f;
-  if (!ctx->stage_timing || ctx->last_stages <= 0) return fail(ctx, DPGICP_E_STATE, "stage timing is off (dpgicp_enable_stage_timing) or nothing has run");
-  CU_TRY(ctx, cudaEventSynchronize(ctx->stage_ev[ctx->last_stages]));
-  for (int k = 0; k < ctx->last_stages; ++k) CU_TRY(ctx, cudaEventElapsedTime(&stage_ms[k], ctx->stage_ev[k], ctx->stage_ev[k + 1]));
-  *n_stages = ctx->last_stages;
+  if (!ctx->main.stage_timing || ctx->main.last_stages <= 0) return fail(ctx, DPGICP_E_STATE, "stage timing is off (dpgicp_enable_stage_timing) or nothing has run");
+  CU_TRY(ctx, cudaEventSynchronize(ctx->main.stage_ev[ctx->main.last_stages]));
+  for (int k = 0; k < ctx->main.last_stages; ++k) CU_TRY(ctx, cudaEventElapsedTime(&stage_ms[k], ctx->main.stage_ev[k], ctx->main.stage_ev[k + 1]));
+  *n_stages = ctx->main.last_stages;
   return DPGICP_OK;
 }
 
@@ -1771,6 +1882,116 @@ int dpgicp_fp32x2_probe(dpgicp_ctx *ctx, double *mul_add_packed) {
   cudaEventDestroy(e0); cudaEventDestroy(e1);
   *mul_add_packed = best;
   return DPGICP_OK;
+}
+
+/* ---- batch slots ------------------------------------------------------------------------------------------------ */
+int dpgicp_slot_create(dpgicp_ctx *ctx, dpgicp_slot **out) {
+  if (!ctx || !out) return DPGICP_E_INVALID;
+  *out = nullptr;
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  dpgicp_slot *s = new (std::nothrow) dpgicp_slot();
+  if (!s) return fail(ctx, DPGICP_E_NOMEM, "out of host memory");
+  s->batch.n_pairs = -1;                     /* no pair list yet: a run is refused */
+  cudaError_t e = slot_init(s, ctx, true);
+  if (e != cudaSuccess) {
+    slot_release(s);
+    delete s;
+    return fail(ctx, e == cudaErrorMemoryAllocation ? DPGICP_E_NOMEM : DPGICP_E_CUDA, std::string("dpgicp_slot_create: ") + cudaGetErrorString(e));
+  }
+  ctx->slots.push_back(s);
+  {
+    std::lock_guard<std::mutex> lock(g_slots_mutex);
+    g_slots.insert(s);
+  }
+  *out = s;
+  return DPGICP_OK;
+}
+
+int dpgicp_slot_destroy(dpgicp_slot *slot) {
+  dpgicp_slot *s = live(slot);
+  if (!s) return DPGICP_E_INVALID;
+  {
+    std::lock_guard<std::mutex> lock(g_slots_mutex);
+    g_slots.erase(s);
+  }
+  dpgicp_ctx *ctx = s->ctx;
+  cudaSetDevice(ctx->device);
+  cudaStreamSynchronize(s->own);
+  ctx->slots.erase(std::find(ctx->slots.begin(), ctx->slots.end(), s));
+  slot_release(s);
+  delete s;
+  return DPGICP_OK;
+}
+
+int dpgicp_slot_set_pairs(dpgicp_slot *slot, const int32_t *src, const int32_t *tgt, const float *guess, int64_t n) {
+  dpgicp_slot *s = live(slot);
+  return s ? set_pairs_slot(s, src, tgt, guess, n) : DPGICP_E_INVALID;
+}
+
+int dpgicp_slot_set_pair_cost_hints(dpgicp_slot *slot, const float *hints, int64_t n) {
+  dpgicp_slot *s = live(slot);
+  return s ? set_pair_cost_hints_slot(s, hints, n) : DPGICP_E_INVALID;
+}
+
+int dpgicp_slot_run(dpgicp_slot *slot, const dpgicp_params *params) {
+  dpgicp_slot *s = live(slot);
+  return s ? run_slot(s, params, true, 0, 0) : DPGICP_E_INVALID;
+}
+
+int dpgicp_slot_run_range(dpgicp_slot *slot, const dpgicp_params *params, int64_t first, int64_t count) {
+  dpgicp_slot *s = live(slot);
+  return s ? run_slot(s, params, false, first, count) : DPGICP_E_INVALID;
+}
+
+int dpgicp_slot_fetch_results(dpgicp_slot *slot, dpgicp_result *out, int64_t n) {
+  dpgicp_slot *s = live(slot);
+  return s ? fetch_results_slot(s, out, 0, n) : DPGICP_E_INVALID;
+}
+
+int dpgicp_slot_fetch_results_range(dpgicp_slot *slot, dpgicp_result *out, int64_t first, int64_t count) {
+  dpgicp_slot *s = live(slot);
+  return s ? fetch_results_slot(s, out, first, count) : DPGICP_E_INVALID;
+}
+
+int dpgicp_slot_fetch_factors(dpgicp_slot *slot, dpgicp_factor *out, int64_t n) {
+  dpgicp_slot *s = live(slot);
+  return s ? fetch_factors_slot(s, out, n) : DPGICP_E_INVALID;
+}
+
+int dpgicp_slot_fetch_pairs(dpgicp_slot *slot, int32_t *src, int32_t *tgt, float *T, int64_t n) {
+  dpgicp_slot *s = live(slot);
+  if (!s) return DPGICP_E_INVALID;
+  CU_TRY(s->ctx, cudaSetDevice(s->ctx->device));
+  return fetch_pairs_from(s->ctx, stream_of(s), s->batch, src, tgt, T, n);
+}
+
+int dpgicp_slot_last_run_counters(dpgicp_slot *slot, uint64_t counters[8]) {
+  dpgicp_slot *s = live(slot);
+  return s && counters ? last_run_counters_slot(s, counters) : DPGICP_E_INVALID;
+}
+
+int dpgicp_slot_synchronize(dpgicp_slot *slot) {
+  dpgicp_slot *s = live(slot);
+  if (!s) return DPGICP_E_INVALID;
+  CU_TRY(s->ctx, cudaSetDevice(s->ctx->device));
+  CU_TRY(s->ctx, cudaStreamSynchronize(s->own));
+  return DPGICP_OK;
+}
+
+int dpgicp_slot_query(dpgicp_slot *slot) {
+  dpgicp_slot *s = live(slot);
+  if (!s) return DPGICP_E_INVALID;
+  CU_TRY(s->ctx, cudaSetDevice(s->ctx->device));
+  const cudaError_t e = cudaStreamQuery(s->own);
+  if (e == cudaErrorNotReady) { cudaGetLastError(); return 0; }
+  CU_TRY(s->ctx, e);
+  return 1;
+}
+
+int dpgicp_slot_enumerate_pairs_device(dpgicp_slot *slot, int32_t mode, float r_same, float r_other, int32_t rank,
+                                       int32_t world, int64_t *n_total, int64_t *n_local) {
+  dpgicp_slot *s = live(slot);
+  return s ? enumerate_slot(s, mode, r_same, r_other, rank, world, n_total, n_local) : DPGICP_E_INVALID;
 }
 
 }  /* extern "C" */

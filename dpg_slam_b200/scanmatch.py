@@ -396,6 +396,11 @@ class ScanMatcher:
         self._check(self._lib.dpgicp_last_run_stage_ms(self._h, C.byref(ms), C.byref(n)))
         return [float(ms[k]) for k in range(n.value)]
 
+    def slot(self) -> "BatchSlot":
+        """A batch slot on this context: a pair batch of its own, run on a CUDA stream of its own over this context's scan
+        store, so that several batches can be in flight (``dpgicp_slot_*``; ordering rules in include/dpgicp.h)."""
+        return BatchSlot(self)
+
     def enumerate_pairs(self, node_xy, node_pass, same_pass_radius=5.0, other_pass_radius=2.0):
         """Pair list of one ``reoptimize()`` in the reference's loop order (parameters.h:212,224)."""
         xy = np.ascontiguousarray(node_xy, np.float32)
@@ -412,3 +417,107 @@ class ScanMatcher:
                                                          same_pass_radius, other_pass_radius, src.ctypes.data,
                                                          tgt.ctypes.data, C.byref(n)))
         return src, tgt
+
+
+class BatchSlot:
+    """One batch in flight on a :class:`ScanMatcher`'s context, with the batch methods of the context's default batch.
+    ``run`` returns at once; ``query`` tells without blocking whether the slot's work is done.  Destroyed by ``close``
+    (which waits for the slot's work) or together with its context."""
+
+    def __init__(self, sm: ScanMatcher):
+        self._sm = sm
+        self._lib = sm._lib
+        h = C.c_void_p()
+        sm._check(self._lib.dpgicp_slot_create(sm._h, C.byref(h)))
+        self._h = h
+        self._n_pairs = 0
+
+    def _check(self, rc: int):
+        if rc < 0:
+            self._sm._check(rc)
+
+    def close(self):
+        if getattr(self, "_h", None) and getattr(self._sm, "_h", None):
+            self._lib.dpgicp_slot_destroy(self._h)
+        self._h = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def set_pairs(self, src_idx, tgt_idx, guess):
+        s = np.ascontiguousarray(src_idx, np.int32)
+        t = np.ascontiguousarray(tgt_idx, np.int32)
+        g = np.ascontiguousarray(guess, np.float32).reshape(-1, 3)
+        if not (s.shape[0] == t.shape[0] == g.shape[0]):
+            raise ValueError("src_idx, tgt_idx and guess must have the same length")
+        self._n_pairs = s.shape[0]
+        self._check(self._lib.dpgicp_slot_set_pairs(self._h, s.ctypes.data, t.ctypes.data, g.ctypes.data, s.shape[0]))
+
+    def set_pair_cost_hints(self, hints):
+        if hints is None:
+            self._check(self._lib.dpgicp_slot_set_pair_cost_hints(self._h, None, 0))
+            return
+        h = np.ascontiguousarray(hints, np.float32)
+        self._check(self._lib.dpgicp_slot_set_pair_cost_hints(self._h, h.ctypes.data, h.shape[0]))
+
+    def run(self, params: Params):
+        """Launch the slot's batch asynchronously on the slot's stream."""
+        self._check(self._lib.dpgicp_slot_run(self._h, C.byref(params)))
+
+    def run_range(self, params: Params, first: int, count: int):
+        self._check(self._lib.dpgicp_slot_run_range(self._h, C.byref(params), first, count))
+
+    def fetch_results(self, n: Optional[int] = None, out: Optional[np.ndarray] = None) -> np.ndarray:
+        n = self._n_pairs if n is None else n
+        if out is None:
+            out = np.zeros(n, RESULT_DTYPE)
+        elif out.dtype != RESULT_DTYPE or not out.flags.c_contiguous or out.shape[0] < n:
+            raise ValueError("out must be a contiguous RESULT_DTYPE array of at least n records")
+        self._check(self._lib.dpgicp_slot_fetch_results(self._h, out.ctypes.data, n))
+        return out
+
+    def fetch_results_range(self, first: int, count: int) -> np.ndarray:
+        out = np.zeros(count, RESULT_DTYPE)
+        self._check(self._lib.dpgicp_slot_fetch_results_range(self._h, out.ctypes.data, first, count))
+        return out
+
+    def fetch_factors(self, n: Optional[int] = None) -> np.ndarray:
+        n = self._n_pairs if n is None else n
+        out = np.zeros(n, FACTOR_DTYPE)
+        self._check(self._lib.dpgicp_slot_fetch_factors(self._h, out.ctypes.data, n))
+        return out
+
+    def fetch_pairs(self, n: Optional[int] = None):
+        n = self._n_pairs if n is None else n
+        src = np.zeros(n, np.int32)
+        tgt = np.zeros(n, np.int32)
+        T = np.zeros((n, 4), np.float32)
+        self._check(self._lib.dpgicp_slot_fetch_pairs(self._h, src.ctypes.data, tgt.ctypes.data, T.ctypes.data, n))
+        return src, tgt, T
+
+    def enumerate_pairs_device(self, mode=_abi.ENUM_REOPTIMIZE, same_pass_radius=5.0, other_pass_radius=2.0,
+                               shard_rank=0, shard_world=1) -> Tuple[int, int]:
+        tot, loc = C.c_int64(0), C.c_int64(0)
+        self._check(self._lib.dpgicp_slot_enumerate_pairs_device(self._h, mode, same_pass_radius, other_pass_radius,
+                                                                 shard_rank, shard_world, C.byref(tot), C.byref(loc)))
+        self._n_pairs = int(loc.value)
+        return int(tot.value), int(loc.value)
+
+    def last_run_counters(self) -> dict:
+        c = (C.c_uint64 * 8)()
+        self._check(self._lib.dpgicp_slot_last_run_counters(self._h, C.byref(c)))
+        return {"iterations": int(c[0]), "correspondences": int(c[1]), "distance_evals": int(c[2]),
+                "box_tests": int(c[3]), "kernel_launches": int(c[4]),
+                "dev_candidates": int(c[5]), "dev_loose_searches": int(c[6]), "dev_searches": int(c[7])}
+
+    def synchronize(self):
+        self._check(self._lib.dpgicp_slot_synchronize(self._h))
+
+    def query(self) -> bool:
+        """True when the slot's enqueued work is done (does not block)."""
+        rc = self._lib.dpgicp_slot_query(self._h)
+        self._check(rc)
+        return rc == 1

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define DPGICP_ABI_VERSION 4
+#define DPGICP_ABI_VERSION 5
 
 /* ---- error codes ------------------------------------------------------------------------- */
 #define DPGICP_OK            0
@@ -161,6 +161,7 @@ typedef struct dpgicp_factor {          /* 96 bytes */
 } dpgicp_factor;
 
 typedef struct dpgicp_ctx dpgicp_ctx;
+typedef struct dpgicp_slot dpgicp_slot;
 
 /* ---- lifetime ------------------------------------------------------------------------------ */
 int  dpgicp_abi_version(void);
@@ -388,6 +389,57 @@ int  dpgicp_fp32_probe(dpgicp_ctx *ctx, double *ops_per_s_mul_add, double *ops_p
  * second, one packed instruction = 2 operations.  Measured equal to the scalar rate: a packed instruction takes two
  * pipe cycles, so packing saves issue slots, not FP32 time.                                         */
 int  dpgicp_fp32x2_probe(dpgicp_ctx *ctx, double *ops_per_s_mul_add_packed);
+
+/* ---- batch slots: several pair batches in flight on one context ------------------------------------------------
+ * The batch calls above (dpgicp_set_pairs, _run, _fetch_*, dpgicp_enumerate_pairs_device, stage timing, the fused
+ * gather) act on the context's DEFAULT slot, which runs on the context's stream (dpgicp_set_stream).  A slot created
+ * here holds a batch of its own (pair list, cost hints, records, counters) and runs it on a CUDA stream of its own on
+ * the context's device, so a caller can prepare and launch batch k+1 while batch k still runs.  Every slot shares the
+ * context's scan store and node table: one copy of the store serves every batch in flight.
+ *   for (k = 0; k < n_batches; ++k) {
+ *     dpgicp_slot *s = slot[k % K];
+ *     if (k >= K) dpgicp_slot_fetch_results(s, out[k - K], n[k - K]);     // waits for that batch only
+ *     dpgicp_slot_set_pairs(s, src[k], tgt[k], guess[k], n[k]);
+ *     dpgicp_slot_run(s, &params);                                        // returns at once
+ *   }
+ * Ordering rules (enforced by the library with stream events and synchronisations):
+ *   - a slot's run reads the store as it was when the run was enqueued, and waits for the store writes (upload, append,
+ *     convert) and the enumeration into that slot enqueued before it;
+ *   - dpgicp_upload_scans / _upload_ranges / _upload_ranges_subset / _convert_ranges_device replace the store: they wait
+ *     for every slot's enqueued work and empty every slot's batch.  dpgicp_append_* writes only rows no enqueued run
+ *     reads and does not wait, unless the store has to move (growth, re-pitch): the old buffers are then freed only
+ *     after every slot's stream has drained;
+ *   - dpgicp_set_nodes does not wait: no run reads the node table (the enumeration does, and it is synchronous);
+ *   - dpgicp_slot_enumerate_pairs_device runs on the context's stream and returns when the list is on the device, as
+ *     dpgicp_enumerate_pairs_device does; it first waits for the slot's own enqueued work;
+ *   - the fused multi-GPU gather (dpgicp_gather_attach*) applies to the default slot only: a slot's run writes its
+ *     local records only, whether or not a gather is attached;
+ *   - records do not depend on what runs concurrently (bit-equal to the same batch run alone).
+ * Returns: DPGICP_E_INVALID for a NULL or destroyed slot (as for bad arguments), DPGICP_E_STATE for a run before the
+ * slot's first pair list.  Errors are reported through dpgicp_last_error of the slot's context.  A slot belongs to the
+ * thread that owns its context.                                                                                  */
+int  dpgicp_slot_create(dpgicp_ctx *ctx, dpgicp_slot **out_slot);
+/* waits for the slot's work, then frees it; dpgicp_destroy destroys the slots of the context still alive */
+int  dpgicp_slot_destroy(dpgicp_slot *slot);
+/* the slot forms of dpgicp_set_pairs, _set_pair_cost_hints, _run, _run_range, _fetch_results, _fetch_results_range,
+ * _fetch_factors, _fetch_pairs, _last_run_counters ([4] counts the launches of the whole context) and _synchronize */
+int  dpgicp_slot_set_pairs(dpgicp_slot *slot, const int32_t *src_idx, const int32_t *tgt_idx, const float *guess,
+                           int64_t n_pairs);
+int  dpgicp_slot_set_pair_cost_hints(dpgicp_slot *slot, const float *hints, int64_t n_pairs);
+int  dpgicp_slot_run(dpgicp_slot *slot, const dpgicp_params *params);
+int  dpgicp_slot_run_range(dpgicp_slot *slot, const dpgicp_params *params, int64_t first, int64_t count);
+int  dpgicp_slot_fetch_results(dpgicp_slot *slot, dpgicp_result *out, int64_t n_pairs);
+int  dpgicp_slot_fetch_results_range(dpgicp_slot *slot, dpgicp_result *out, int64_t first, int64_t count);
+int  dpgicp_slot_fetch_factors(dpgicp_slot *slot, dpgicp_factor *out, int64_t n_pairs);
+int  dpgicp_slot_fetch_pairs(dpgicp_slot *slot, int32_t *src_idx, int32_t *tgt_idx, float *T, int64_t n_pairs);
+int  dpgicp_slot_last_run_counters(dpgicp_slot *slot, uint64_t counters[8]);
+int  dpgicp_slot_synchronize(dpgicp_slot *slot);
+/* non-blocking: 1 when the slot's enqueued work is done, 0 while it runs, < 0 on error */
+int  dpgicp_slot_query(dpgicp_slot *slot);
+/* dpgicp_enumerate_pairs_device with the list and guesses left as the slot's batch */
+int  dpgicp_slot_enumerate_pairs_device(dpgicp_slot *slot, int32_t mode, float same_pass_radius, float other_pass_radius,
+                                        int32_t shard_rank, int32_t shard_world, int64_t *n_pairs_total,
+                                        int64_t *n_pairs_local);
 
 #ifdef __cplusplus
 }

@@ -157,6 +157,55 @@ class ScanMatcher {
     return out;
   }
 
+  /* One more batch in flight over this matcher's scan store (dpgicp_slot_*): run() returns at once, the fetches wait
+   * for this slot's batch only.  Must not outlive its ScanMatcher. */
+  class Slot {
+   public:
+    explicit Slot(ScanMatcher &sm) : sm_(sm) { sm_.check(dpgicp_slot_create(sm_.ctx_, &slot_), "dpgicp_slot_create"); }
+    ~Slot() { dpgicp_slot_destroy(slot_); }
+    Slot(const Slot &) = delete;
+    Slot &operator=(const Slot &) = delete;
+
+    dpgicp_slot *get() { return slot_; }
+    void setPairs(const std::vector<int32_t> &src, const std::vector<int32_t> &tgt, const std::vector<float> &guess) {
+      if (tgt.size() != src.size() || guess.size() != 3 * src.size()) throw std::runtime_error("Slot::setPairs: length mismatch");
+      sm_.check(dpgicp_slot_set_pairs(slot_, src.data(), tgt.data(), guess.data(), (int64_t)src.size()), "dpgicp_slot_set_pairs");
+    }
+    /* the caller's pair list built on the device into this slot; returns the local pair count */
+    int64_t enumeratePairs(int32_t mode, float same_pass_radius, float other_pass_radius) {
+      int64_t n = 0;
+      sm_.check(dpgicp_slot_enumerate_pairs_device(slot_, mode, same_pass_radius, other_pass_radius, 0, 1, nullptr, &n),
+                "dpgicp_slot_enumerate_pairs_device");
+      return n;
+    }
+    void run() { sm_.check(dpgicp_slot_run(slot_, &sm_.params_), "dpgicp_slot_run"); }
+    void runRange(int64_t first, int64_t count) {
+      sm_.check(dpgicp_slot_run_range(slot_, &sm_.params_, first, count), "dpgicp_slot_run_range");
+    }
+    void fetchResults(dpgicp_result *out, int64_t first, int64_t count) {
+      sm_.check(dpgicp_slot_fetch_results_range(slot_, out, first, count), "dpgicp_slot_fetch_results_range");
+    }
+    std::vector<dpgicp_factor> factors(size_t n) {
+      std::vector<dpgicp_factor> out(n);
+      sm_.check(dpgicp_slot_fetch_factors(slot_, out.data(), (int64_t)n), "dpgicp_slot_fetch_factors");
+      return out;
+    }
+    void pairs(std::vector<int32_t> &src, std::vector<int32_t> &tgt, int64_t n) {
+      src.assign((size_t)n, 0); tgt.assign((size_t)n, 0);
+      sm_.check(dpgicp_slot_fetch_pairs(slot_, src.data(), tgt.data(), nullptr, n), "dpgicp_slot_fetch_pairs");
+    }
+    bool done() {
+      const int rc = dpgicp_slot_query(slot_);
+      if (rc < 0) sm_.check(rc, "dpgicp_slot_query");
+      return rc == 1;
+    }
+    void synchronize() { sm_.check(dpgicp_slot_synchronize(slot_), "dpgicp_slot_synchronize"); }
+
+   private:
+    ScanMatcher &sm_;
+    dpgicp_slot *slot_ = nullptr;
+  };
+
  private:
   void check(int rc, const char *what) {
     if (rc != DPGICP_OK) throw std::runtime_error(std::string(what) + ": " + last_error());
