@@ -19,6 +19,7 @@
 #include <new>
 #include <set>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "dpgicp.h"
@@ -37,12 +38,52 @@ std::string g_create_error;
 std::mutex g_optin_mutex;
 std::map<std::pair<int, const void *>, size_t> g_smem_optin;   /* (device, kernel) -> dynamic shared memory opted in */
 
-struct DevBuf {
+/* Device memory (cudaMalloc) or page-locked host memory (cudaMallocHost), freed by its owner.  An owner whose memory a
+ * stream may still read lets it go only after that stream has drained. */
+template <cudaError_t (*Alloc)(void **, size_t), cudaError_t (*Free)(void *)>
+struct Buf {
   void *p = nullptr;
   size_t cap = 0;
+  Buf() = default;
+  Buf(const Buf &) = delete;
+  Buf &operator=(const Buf &) = delete;
+  Buf &operator=(Buf &&o) noexcept { release(); std::swap(p, o.p); std::swap(cap, o.cap); return *this; }
+  ~Buf() { release(); }
+  void release() {
+    if (p) Free(p);
+    p = nullptr; cap = 0;
+  }
+  cudaError_t alloc(size_t bytes) {      /* exactly `bytes`; the old buffer is freed first */
+    release();
+    void *q = nullptr;
+    const cudaError_t e = Alloc(&q, bytes);
+    if (e == cudaSuccess) { p = q; cap = bytes; }
+    return e;
+  }
 };
+using DevBuf = Buf<cudaMalloc, cudaFree>;
+using HostBuf = Buf<cudaMallocHost, cudaFreeHost>;
 
-struct Store {                 /* padded rows + counts on the device, counts mirrored on the host */
+/* a CUDA event or stream, destroyed by its owner */
+template <class T, cudaError_t (*Destroy)(T)>
+struct Handle {
+  T h = nullptr;
+  Handle() = default;
+  Handle(const Handle &) = delete;
+  Handle &operator=(const Handle &) = delete;
+  ~Handle() { reset(); }
+  void reset() {
+    if (h) Destroy(h);
+    h = nullptr;
+  }
+  operator T() const { return h; }
+};
+using Event = Handle<cudaEvent_t, cudaEventDestroy>;
+using Stream = Handle<cudaStream_t, cudaStreamDestroy>;
+
+/* padded rows + counts on the device, counts mirrored on the host.  A write of the scan store fills the rows behind
+ * n_scans and only then advances it (commit_rows). */
+struct Store {
   DevBuf rows, count;
   int32_t pitch = 0, n_scans = 0, max_count = 0;
   std::vector<int32_t> h_count;
@@ -51,9 +92,8 @@ struct Store {                 /* padded rows + counts on the device, counts mir
 struct Batch {
   DevBuf tasks, results, order;
   bool has_order = false;
-  PairTask *h_tasks = nullptr;   /* pinned */
-  size_t h_tasks_cap = 0;
-  cudaEvent_t h_tasks_free = nullptr;   /* recorded after the H2D copy out of h_tasks: the buffer may be rewritten */
+  HostBuf h_tasks;               /* PairTask staging of set_pairs */
+  Event h_tasks_free;            /* recorded after the H2D copy out of h_tasks: the buffer may be rewritten */
   int64_t n_pairs = 0;
   int32_t max_scan = -1;         /* device-enumerated lists: highest scan (= node) index used; -1 = validated on the host */
 };
@@ -70,27 +110,29 @@ struct Nodes {                   /* pose-graph node estimates on the device (dpg
 
 /* One pair batch of a context and the per-run cells of its stage chain.  The context holds the default slot (the batch of
  * dpgicp_set_pairs / dpgicp_run / dpgicp_fetch_*), which runs on the context's stream; dpgicp_slot_create adds slots with
- * a stream of their own, so several batches can be in flight over the one scan store. */
+ * a stream of their own, so several batches can be in flight over the one scan store.  Its members free themselves: a
+ * slot is deleted only after its stream has drained. */
 struct dpgicp_slot {
   dpgicp_ctx *ctx = nullptr;
-  cudaStream_t own = nullptr;                /* nullptr: the default slot, on the context's stream */
+  Stream own;                                /* null: the default slot, on the context's stream */
   Batch batch;
   DevBuf state[2], susp[2];                  /* suspended-pair state slots + pair lists, ping-pong between stages */
-  unsigned long long *d_queue = nullptr;     /* [0..4] stage queue heads, [6],[7] suspended counts, [8..15] counters, [16..23] development phase timers, [24..28] pairs finished per stage */
-  cudaEvent_t stage_ev[9] = {nullptr};
+  DevBuf d_queue;                            /* unsigned long long [0..4] stage queue heads, [6],[7] suspended counts, [8..15] counters, [16..23] development phase timers, [24..28] pairs finished per stage */
+  Event stage_ev[9];
   bool stage_timing = false;
   int last_stages = 0;
 };
 
+/* Its members free themselves: a context is deleted only after its slots are destroyed and its stream has drained. */
 struct dpgicp_ctx {
   int device = 0;
   int sm_count = 148;
-  cudaStream_t stream = nullptr;
-  bool own_stream = true;
+  Stream own_stream;                         /* the stream the context made; null while a caller's stream is in use */
+  cudaStream_t stream = nullptr;             /* the stream in use: own_stream or the one of dpgicp_set_stream */
   Store store, scratch_store;
   dpgicp_slot main;                          /* the default slot */
   std::vector<dpgicp_slot *> slots;          /* the live slots of dpgicp_slot_create */
-  cudaEvent_t written = nullptr;             /* recorded on the context's stream behind every write a later slot run reads
+  Event written;                             /* recorded on the context's stream behind every write a later slot run reads
                                               * (store rows and counts, an enumerated pair list): slot streams wait on it */
   Batch scratch_batch;
   Nodes nodes;                               /* dpgicp_set_nodes: the table of dpgicp_enumerate_pairs_device */
@@ -99,9 +141,7 @@ struct dpgicp_ctx {
   DevBuf stage, offsets, misc, corr, trig, enum_cnt;
   /* per (kernel, warps, shared memory): resident CTAs per SM or clusters per device — queried once, not on every run */
   std::map<std::tuple<const void *, int, size_t>, int> occupancy;
-  void *h_pair = nullptr;                    /* pinned scratch of the single-pair call shapes */
-  size_t h_pair_cap = 0;
-  DevBuf d_pair;
+  HostBuf h_pair;                            /* scratch of the single-pair call shapes */
   int gather_root_only = 0;
   bool gather_local = false;                 /* peers attached by dpgicp_gather_attach_local (no IPC mappings to close) */
   int trig_n = 0;
@@ -112,9 +152,8 @@ struct dpgicp_ctx {
   void *gather_peer[DPGICP_MAX_GATHER_RANKS] = {nullptr};
   int max_stages = 5;
   std::vector<int> chain, chain_cluster;     /* DPGICP_CHAIN: target warps (and "x<cluster size>") per stage (development knob) */
-  int *d_bad = nullptr;
-  void *h_stage = nullptr;                   /* pinned staging for subset uploads from pageable memory */
-  size_t h_stage_cap = 0;
+  DevBuf d_bad;                              /* int: range flag of the store writes */
+  HostBuf h_stage;                           /* staging for subset uploads from pageable memory */
   double handover_factor = 2.0;              /* DPGICP_HANDOVER="f[,fc]": a stage hands over once at most f x (CTAs of the next stage) pairs are */
   double handover_cluster = 1.0;             /* left; fc x (clusters) when the next stage runs clusters (development knob; 0 = plain queue-dry rule) */
   int force_warps = 0;
@@ -139,7 +178,7 @@ int fail(dpgicp_ctx *ctx, int code, const std::string &msg) {
     }                                                                                             \
   } while (0)
 
-cudaStream_t stream_of(const dpgicp_slot *s) { return s->own ? s->own : s->ctx->stream; }
+cudaStream_t stream_of(const dpgicp_slot *s) { return s->own ? s->own.h : s->ctx->stream; }
 
 /* a buffer the runs of every slot may read is about to be overwritten or freed: wait until the slots' streams have
  * drained (the default slot's runs are ordered on the context's stream) */
@@ -148,8 +187,8 @@ int drain_slots(dpgicp_ctx *ctx) {
   return DPGICP_OK;
 }
 
-/* the store is about to be replaced: every slot's runs have read it, and every batch is emptied (its indices referred to
- * the old store) */
+/* the store is about to be replaced (make_room): every slot's runs have read it, and every batch is emptied (its indices
+ * referred to the old store) */
 int replace_store(dpgicp_ctx *ctx) {
   int rc = drain_slots(ctx);
   if (rc) return rc;
@@ -164,18 +203,12 @@ int mark_written(dpgicp_ctx *ctx) {
   return DPGICP_OK;
 }
 
-int reserve(dpgicp_ctx *ctx, DevBuf &b, size_t bytes) {
+/* at least `bytes` in b, its contents not kept; a pinned buffer's caller first waits for any copy still queued out of it */
+template <class B>
+int reserve(dpgicp_ctx *ctx, B &b, size_t bytes) {
   if (bytes <= b.cap) return DPGICP_OK;
-  if (b.p) { CU_TRY(ctx, cudaFree(b.p)); b.p = nullptr; b.cap = 0; }
-  size_t want = std::max(bytes, (size_t)256);
-  CU_TRY(ctx, cudaMalloc(&b.p, want));
-  b.cap = want;
+  CU_TRY(ctx, b.alloc(std::max(bytes, (size_t)256)));
   return DPGICP_OK;
-}
-
-void release(DevBuf &b) {
-  if (b.p) cudaFree(b.p);
-  b.p = nullptr; b.cap = 0;
 }
 
 int check_params(dpgicp_ctx *ctx, const dpgicp_params *p) {
@@ -337,7 +370,8 @@ int launch_icp(dpgicp_slot *s, const Store &st, const Batch &b, const dpgicp_par
   kp.order = (b.has_order && whole) ? (const long long *)b.order.p : nullptr;
   kp.results = (dpgicp_result *)b.results.p + first;
   kp.pair_base = first;
-  kp.counters = s->d_queue + 8;
+  unsigned long long *const q = (unsigned long long *)s->d_queue.p;
+  kp.counters = q + 8;
   kp.n_pairs = count;
   kp.n_cap = n_cap;
   kp.max_iterations = p->max_iterations;
@@ -424,7 +458,7 @@ int launch_icp(dpgicp_slot *s, const Store &st, const Batch &b, const dpgicp_par
     for (int k = 1; k < n_stages; ++k) shapes[k - 1] = shapes[k];
     --n_stages;
   }
-  CU_TRY(ctx, cudaMemsetAsync(s->d_queue, 0, 32 * sizeof(unsigned long long), stream));
+  CU_TRY(ctx, cudaMemsetAsync(q, 0, 32 * sizeof(unsigned long long), stream));
   int grid_prev = 0;
   const bool timing = s->stage_timing && corr_out == nullptr;
   if (timing) { s->last_stages = n_stages; CU_TRY(ctx, cudaEventRecord(s->stage_ev[0], stream)); }
@@ -441,14 +475,14 @@ int launch_icp(dpgicp_slot *s, const Store &st, const Batch &b, const dpgicp_par
   }
   for (int sidx = 0; sidx < n_stages; ++sidx) {
     KernelParams ks = kp;
-    ks.queue = s->d_queue + sidx;
+    ks.queue = q + sidx;
     ks.resume = sidx > 0 ? 1 : 0;
     if (sidx > 0) {
-      ks.in_count = reinterpret_cast<const unsigned int *>(s->d_queue + 6 + ((sidx - 1) & 1));
+      ks.in_count = reinterpret_cast<const unsigned int *>(q + 6 + ((sidx - 1) & 1));
       ks.susp_in = (const long long *)s->susp[(sidx - 1) & 1].p;
       ks.state_in = (const unsigned char *)s->state[(sidx - 1) & 1].p;
     }
-    ks.finished = s->d_queue + 24 + sidx;
+    ks.finished = q + 24 + sidx;
     if (sidx + 1 < n_stages) {
       /* hand over once the next stage could run all that is left at once (clusters: exactly; CTAs: a third more,
        * the next stage's own queue-dry rule then takes over) */
@@ -459,11 +493,11 @@ int launch_icp(dpgicp_slot *s, const Store &st, const Batch &b, const dpgicp_par
       if (rcq) return rcq;
       ks.handover = (long long)std::ceil((shapes[sidx + 1].csize > 1 ? ctx->handover_cluster : ctx->handover_factor) * (double)next_units);
       if (ctx->handover_factor <= 0.0) ks.handover = (long long)1 << 40;      /* development: the plain queue-dry rule */
-      ks.out_count = reinterpret_cast<unsigned int *>(s->d_queue + 6 + (sidx & 1));
+      ks.out_count = reinterpret_cast<unsigned int *>(q + 6 + (sidx & 1));
       ks.susp_out = (long long *)s->susp[sidx & 1].p;
       ks.state_out = (unsigned char *)s->state[sidx & 1].p;
       if (sidx >= 2)      /* the count cell is reused by stage sidx: clear it after stage sidx-1 consumed it */
-        CU_TRY(ctx, cudaMemsetAsync(s->d_queue + 6 + (sidx & 1), 0, sizeof(unsigned long long), stream));
+        CU_TRY(ctx, cudaMemsetAsync(q + 6 + (sidx & 1), 0, sizeof(unsigned long long), stream));
     }
     int grid = 0;
     const int64_t max_items = sidx == 0 ? count : (int64_t)grid_prev;
@@ -475,22 +509,11 @@ int launch_icp(dpgicp_slot *s, const Store &st, const Batch &b, const dpgicp_par
   return DPGICP_OK;
 }
 
-int finish_store(dpgicp_ctx *ctx, Store &st, int n_scans) {
-  /* counts back to the host (sizing of shared memory, argument validation) + range flag */
-  st.h_count.resize((size_t)n_scans);
-  int bad = 0;
-  CU_TRY(ctx, cudaMemcpyAsync(st.h_count.data(), st.count.p, sizeof(int32_t) * (size_t)n_scans,
-                              cudaMemcpyDeviceToHost, ctx->stream));
-  CU_TRY(ctx, cudaMemcpyAsync(&bad, ctx->d_bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-  CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  st.n_scans = n_scans;
-  st.max_count = 0;
-  for (int32_t c : st.h_count) st.max_count = std::max(st.max_count, c);
-  if (bad) {
-    st.n_scans = 0;
-    return fail(ctx, DPGICP_E_RANGE, "scan store holds a non-finite point or |coordinate| > DPGICP_MAX_ABS_COORD");
-  }
-  return mark_written(ctx);
+/* arguments of a range-scan write (dpgicp_upload_ranges, _upload_ranges_subset, _append_ranges, _convert_ranges_device) */
+int check_ranges(dpgicp_ctx *ctx, const float *ranges, int32_t n_scans, int32_t n_beams) {
+  if (n_scans < 0 || n_beams < 2 || (n_scans > 0 && !ranges)) return fail(ctx, DPGICP_E_INVALID, "bad range-scan arguments");
+  if (n_beams > DPGICP_MAX_POINTS) return fail(ctx, DPGICP_E_TOOBIG, "n_beams exceeds DPGICP_MAX_POINTS");
+  return DPGICP_OK;
 }
 
 /* arguments of a ragged cloud upload (dpgicp_upload_scans / dpgicp_append_scans): the largest scan and the point total */
@@ -511,32 +534,6 @@ int check_clouds(dpgicp_ctx *ctx, const void *points, size_t stride, const int64
   return DPGICP_OK;
 }
 
-int upload_scans_into(dpgicp_ctx *ctx, Store &st, const void *points, size_t stride, const int64_t *offsets,
-                      int32_t n_scans) {
-  int64_t maxc = 0, total = 0;
-  int rc = check_clouds(ctx, points, stride, offsets, n_scans, &maxc, &total);
-  if (rc) return rc;
-  const int pitch = (int)std::max<int64_t>(2, (maxc + 1) & ~(int64_t)1);
-  if ((rc = reserve(ctx, st.rows, sizeof(float2) * (size_t)pitch * (size_t)std::max(n_scans, 1)))) return rc;
-  if ((rc = reserve(ctx, st.count, sizeof(int32_t) * (size_t)std::max(n_scans, 1)))) return rc;
-  if ((rc = reserve(ctx, ctx->stage, (size_t)total * stride + 16))) return rc;
-  if ((rc = reserve(ctx, ctx->offsets, sizeof(int64_t) * ((size_t)n_scans + 1)))) return rc;
-  st.pitch = pitch;
-  st.n_scans = 0;
-  CU_TRY(ctx, cudaMemsetAsync(ctx->d_bad, 0, sizeof(int), ctx->stream));
-  if (n_scans == 0) { st.max_count = 0; st.h_count.clear(); return DPGICP_OK; }
-  if (total > 0)
-    CU_TRY(ctx, cudaMemcpyAsync(ctx->stage.p, points, (size_t)total * stride, cudaMemcpyHostToDevice, ctx->stream));
-  CU_TRY(ctx, cudaMemcpyAsync(ctx->offsets.p, offsets, sizeof(int64_t) * ((size_t)n_scans + 1),
-                              cudaMemcpyHostToDevice, ctx->stream));
-  pack_rows_kernel<<<n_scans, 256, 0, ctx->stream>>>((const unsigned char *)ctx->stage.p, stride,
-                                                     (const long long *)ctx->offsets.p, n_scans, pitch,
-                                                     (float2 *)st.rows.p, (int32_t *)st.count.p, ctx->d_bad);
-  ctx->launches++;
-  CU_TRY(ctx, cudaGetLastError());
-  return finish_store(ctx, st, n_scans);
-}
-
 int set_pairs_into(dpgicp_ctx *ctx, cudaStream_t stream, const Store &st, Batch &b, const int32_t *src, const int32_t *tgt,
                    const float *guess, const float *T_direct, int64_t n) {
   if (n < 0 || (n > 0 && (!src || !tgt || (!guess && !T_direct))))
@@ -545,13 +542,10 @@ int set_pairs_into(dpgicp_ctx *ctx, cudaStream_t stream, const Store &st, Batch 
   /* dpgicp_run is asynchronous: the previous list's H2D copy out of the pinned staging buffer may still be queued
    * behind a running kernel; wait for it before the buffer is rewritten (or freed) */
   if (b.h_tasks_free) CU_TRY(ctx, cudaEventSynchronize(b.h_tasks_free));
-  else CU_TRY(ctx, cudaEventCreateWithFlags(&b.h_tasks_free, cudaEventDisableTiming));
-  if ((size_t)n > b.h_tasks_cap) {
-    if (b.h_tasks) cudaFreeHost(b.h_tasks);
-    b.h_tasks = nullptr; b.h_tasks_cap = 0;
-    CU_TRY(ctx, cudaMallocHost((void **)&b.h_tasks, sizeof(PairTask) * (size_t)n));
-    b.h_tasks_cap = (size_t)n;
-  }
+  else CU_TRY(ctx, cudaEventCreateWithFlags(&b.h_tasks_free.h, cudaEventDisableTiming));
+  int rc;
+  if ((rc = reserve(ctx, b.h_tasks, sizeof(PairTask) * (size_t)n))) return rc;
+  PairTask *h_tasks = (PairTask *)b.h_tasks.p;
   /* host threads share the loop (the libm cos/sin of the guesses is the bulk of it); the first offending pair is
    * reported, as the serial loop would */
   int64_t bad_index = n, bad_guess = n;
@@ -569,16 +563,15 @@ int set_pairs_into(dpgicp_ctx *ctx, cudaStream_t stream, const Store &st, Batch 
       if (!std::isfinite(g0) || !std::isfinite(g1) || !std::isfinite(g2)) { if (k < bad_guess) bad_guess = k; continue; }
       t.c = (float)std::cos((double)g2); t.s = (float)std::sin((double)g2); t.tx = g0; t.ty = g1;
     }
-    b.h_tasks[k] = t;
+    h_tasks[k] = t;
   }
   if (bad_index < n && bad_index <= bad_guess)
     return fail(ctx, DPGICP_E_INVALID, "pair index out of range at pair " + std::to_string(bad_index));
   if (bad_guess < n) return fail(ctx, DPGICP_E_RANGE, "non-finite guess at pair " + std::to_string(bad_guess));
-  int rc;
   if ((rc = reserve(ctx, b.tasks, sizeof(PairTask) * (size_t)std::max<int64_t>(n, 1)))) return rc;
   if ((rc = reserve(ctx, b.results, sizeof(dpgicp_result) * (size_t)std::max<int64_t>(n, 1)))) return rc;
   if (n > 0)
-    CU_TRY(ctx, cudaMemcpyAsync(b.tasks.p, b.h_tasks, sizeof(PairTask) * (size_t)n, cudaMemcpyHostToDevice, stream));
+    CU_TRY(ctx, cudaMemcpyAsync(b.tasks.p, h_tasks, sizeof(PairTask) * (size_t)n, cudaMemcpyHostToDevice, stream));
   CU_TRY(ctx, cudaEventRecord(b.h_tasks_free, stream));
   b.n_pairs = n;
   b.has_order = false;
@@ -627,16 +620,11 @@ int two_cloud_store(dpgicp_ctx *ctx, const void *a, int na, const void *b, int n
   Store &st = ctx->scratch_store;
   const int pitch = std::max(2, (std::max(na, nb) + 1) & ~1);
   const size_t row_bytes = sizeof(float2) * (size_t)pitch, blob = 2 * row_bytes + 16;
-  if (blob > ctx->h_pair_cap) {
-    if (ctx->h_pair) { CU_TRY(ctx, cudaStreamSynchronize(ctx->stream)); cudaFreeHost(ctx->h_pair); }
-    ctx->h_pair = nullptr; ctx->h_pair_cap = 0;
-    CU_TRY(ctx, cudaMallocHost(&ctx->h_pair, blob));
-    ctx->h_pair_cap = blob;
-  } else {
-    CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));       /* a previous call's copy out of the buffer (already done: every
+  CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));         /* a previous call's copy out of the buffer (already done: every
                                                             * single-pair call ends with a synchronisation) */
-  }
-  float *rows = (float *)ctx->h_pair;
+  int rc;
+  if ((rc = reserve(ctx, ctx->h_pair, blob))) return rc;
+  float *rows = (float *)ctx->h_pair.p;
   const void *src[2] = {a, b};
   const int cnt[2] = {na, nb};
   for (int r = 0; r < 2; ++r) {
@@ -653,9 +641,8 @@ int two_cloud_store(dpgicp_ctx *ctx, const void *a, int na, const void *b, int n
     }
     std::memset(row + 2 * (size_t)cnt[r], 0, sizeof(float) * 2 * (size_t)(pitch - cnt[r]));
   }
-  int32_t *h_cnt = (int32_t *)((char *)ctx->h_pair + 2 * row_bytes);
+  int32_t *h_cnt = (int32_t *)((char *)ctx->h_pair.p + 2 * row_bytes);
   h_cnt[0] = na; h_cnt[1] = nb;
-  int rc;
   if ((rc = reserve(ctx, st.rows, 2 * row_bytes))) return rc;
   if ((rc = reserve(ctx, st.count, 2 * sizeof(int32_t)))) return rc;
   CU_TRY(ctx, cudaMemcpyAsync(st.rows.p, rows, 2 * row_bytes, cudaMemcpyHostToDevice, ctx->stream));
@@ -819,7 +806,7 @@ int fetch_pairs_from(dpgicp_ctx *ctx, cudaStream_t stream, const Batch &b, int32
 }
 
 /* Room for n_new more rows of at least need_pitch (even) points behind the rows of the store, every existing row kept
- * (the append path).  Rows and counts grow by doubling, so n one-scan appends copy O(n) rows in total; a scan longer
+ * (make_room of an append).  Rows and counts grow by doubling, so n one-scan appends copy O(n) rows in total; a scan longer
  * than the pitch re-pitches the kept rows on the device.  A buffer that moves is freed only after the context's stream
  * and every slot's stream have drained: the copy out of it, and any run enqueued before the append, read it.  On failure the store is as
  * it was. */
@@ -830,25 +817,17 @@ int grow_store(dpgicp_ctx *ctx, Store &st, int n_new, int need_pitch) {
   const size_t row_bytes = sizeof(float2) * (size_t)pitch;
   const bool move_rows = (n_old > 0 && pitch != st.pitch) || (size_t)rows * row_bytes > st.rows.cap;
   const bool move_count = (size_t)rows * sizeof(int32_t) > st.count.cap;
-  DevBuf nr, nc;
-  auto alloc = [&](DevBuf &b, size_t bytes) {
-    cudaError_t e = cudaMalloc(&b.p, bytes);
-    if (e != cudaSuccess) {
-      b.p = nullptr;
-      return fail(ctx, e == cudaErrorMemoryAllocation ? DPGICP_E_NOMEM : DPGICP_E_CUDA,
-                  std::string("cudaMalloc (scan store growth): ") + cudaGetErrorString(e));
-    }
-    b.cap = bytes;
-    return (int)DPGICP_OK;
-  };
+  DevBuf nr, nc;            /* on failure freed on return, after the context's stream has drained the copies into them */
   auto cuda = [&](cudaError_t e, const char *what) {
-    return e == cudaSuccess ? (int)DPGICP_OK : fail(ctx, DPGICP_E_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
+    return e == cudaSuccess ? (int)DPGICP_OK
+                            : fail(ctx, e == cudaErrorMemoryAllocation ? DPGICP_E_NOMEM : DPGICP_E_CUDA,
+                                   std::string(what) + ": " + cudaGetErrorString(e));
   };
   int rc = DPGICP_OK;
   if (move_rows) {
     int64_t cap = st.pitch > 0 ? (int64_t)(st.rows.cap / (sizeof(float2) * (size_t)st.pitch)) : 0;
     if (rows > cap) cap = std::max(rows, 2 * cap);
-    rc = alloc(nr, (size_t)cap * row_bytes);
+    rc = cuda(nr.alloc((size_t)cap * row_bytes), "cudaMalloc (scan store growth)");
     if (!rc && n_old > 0 && pitch == st.pitch)
       rc = cuda(cudaMemcpyAsync(nr.p, st.rows.p, (size_t)n_old * row_bytes, cudaMemcpyDeviceToDevice, ctx->stream),
                 "cudaMemcpyAsync (scan rows)");
@@ -861,7 +840,7 @@ int grow_store(dpgicp_ctx *ctx, Store &st, int n_new, int need_pitch) {
   }
   if (!rc && move_count) {
     const int64_t cap = std::max(rows, 2 * (int64_t)(st.count.cap / sizeof(int32_t)));
-    rc = alloc(nc, (size_t)cap * sizeof(int32_t));
+    rc = cuda(nc.alloc((size_t)cap * sizeof(int32_t)), "cudaMalloc (scan store growth)");
     if (!rc && n_old > 0)
       rc = cuda(cudaMemcpyAsync(nc.p, st.count.p, (size_t)n_old * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream),
                 "cudaMemcpyAsync (scan counts)");
@@ -870,60 +849,119 @@ int grow_store(dpgicp_ctx *ctx, Store &st, int n_new, int need_pitch) {
   if (!rc && (move_rows || move_count)) rc = drain_slots(ctx);
   if (rc) {
     cudaStreamSynchronize(ctx->stream);
-    release(nr); release(nc);
     return rc;
   }
-  if (move_rows) { release(st.rows); st.rows = nr; }
-  if (move_count) { release(st.count); st.count = nc; }
+  if (move_rows) st.rows = std::move(nr);       /* the old buffers go: nothing queued reads them any more */
+  if (move_count) st.count = std::move(nc);
   st.pitch = pitch;
   return DPGICP_OK;
 }
 
-/* the counts of the n_new rows just converted behind the store back to the host (only those) + the range flag; the
- * store takes them only when every point is in range */
-int finish_append(dpgicp_ctx *ctx, Store &st, int n_new) {
+/* ---- the write path of the scan store ---------------------------------------------------------------------------
+ * dpgicp_upload_scans, _upload_ranges, _upload_ranges_subset and _convert_ranges_device replace the store;
+ * dpgicp_append_ranges and _append_scans append to it.  Each one checks its arguments before it touches anything (store,
+ * batches, slots), then calls make_room, stages its input, converts into the rows behind n_scans (convert_ranges or
+ * pack_clouds) and calls commit_rows.  From make_room on, a replace that fails for any reason leaves an empty store and
+ * an append that fails leaves the store as it was. */
+
+/* the row pitch for scans of at most n points: even, so that every row is 16-byte aligned */
+int row_pitch(int64_t n) { return (int)std::max<int64_t>(2, (n + 1) & ~(int64_t)1); }
+
+/* Room for n rows of at least `pitch` points behind n_scans, and the range flag cleared.
+ * Replace: the slots drain and every batch empties (replace_store), and the store is emptied before any allocation.
+ * Rows and counts are then reserved at exactly the size needed, the old buffers freed first, so a re-upload never holds
+ * two copies of the store (3.5 GB at config 5).
+ * Append: the row count must fit int32; then grow_store.  An empty append touches nothing. */
+int make_room(dpgicp_ctx *ctx, bool append, int32_t n, int pitch) {
+  Store &st = ctx->store;
+  int rc;
+  if (append) {
+    if ((int64_t)st.n_scans + n > INT32_MAX) return fail(ctx, DPGICP_E_INVALID, "the store would hold more than 2^31 - 1 scans");
+    if (n == 0) return DPGICP_OK;
+    if ((rc = grow_store(ctx, st, n, pitch))) return rc;
+  } else {
+    if ((rc = replace_store(ctx))) return rc;
+    st.n_scans = 0;
+    st.max_count = 0;
+    st.h_count.clear();
+    if ((rc = reserve(ctx, st.rows, sizeof(float2) * (size_t)pitch * (size_t)std::max(n, 1)))) return rc;
+    if ((rc = reserve(ctx, st.count, sizeof(int32_t) * (size_t)std::max(n, 1)))) return rc;
+    st.pitch = pitch;
+  }
+  CU_TRY(ctx, cudaMemsetAsync(ctx->d_bad.p, 0, sizeof(int), ctx->stream));
+  return DPGICP_OK;
+}
+
+/* n range scans of n_beams beams in device memory -> the n rows behind n_scans (with d_ids: scan k is row d_ids[k] of
+ * d_in).  The conversion of createNode (dpg_slam.cc:488-513) + getCachedPointCloudFromNode (dpg_node.cc:8-26); every
+ * range-scan writer converts here, so an appended row is bit for bit the row one upload of the same scans holds. */
+int convert_ranges(dpgicp_ctx *ctx, const float *d_in, const int32_t *d_ids, int32_t n, int32_t n_beams, float angle_min,
+                   float angle_max, float range_max, float lx, float ly, float ltheta) {
+  /* createNode dpg_slam.cc:497: angle_inc = (max - min) / (n - 1.0), stored as float */
+  const float angle_inc = (float)(((double)(float)(angle_max - angle_min)) / ((double)n_beams - 1.0));
+  const float lc = cosf(ltheta), ls = sinf(ltheta);       /* Eigen::Rotation2Df(ltheta), host libm */
+  int rc;
+  if ((rc = ensure_trig(ctx, n_beams, angle_min, angle_inc))) return rc;
+  const Store &st = ctx->store;
+  const int threads = 128, warps_per_block = threads / 32;
+  const int blocks = (n + warps_per_block - 1) / warps_per_block;
+  ranges_to_rows_kernel<<<blocks, threads, 0, ctx->stream>>>(d_in, d_ids, n, n_beams, (const double2 *)ctx->trig.p, range_max,
+                                                            lx, ly, lc, ls, st.pitch, (float2 *)st.rows.p + (size_t)st.n_scans * st.pitch,
+                                                            (int32_t *)st.count.p + st.n_scans, (int *)ctx->d_bad.p);
+  ctx->launches++;
+  CU_TRY(ctx, cudaGetLastError());
+  return DPGICP_OK;
+}
+
+/* n ragged host clouds (the layout of dpgicp_upload_scans, `total` points) -> the n rows behind n_scans */
+int pack_clouds(dpgicp_ctx *ctx, const void *points, size_t stride, const int64_t *offsets, int32_t n, int64_t total) {
+  int rc;
+  if ((rc = reserve(ctx, ctx->stage, (size_t)total * stride + 16))) return rc;
+  if ((rc = reserve(ctx, ctx->offsets, sizeof(int64_t) * ((size_t)n + 1)))) return rc;
+  if (total > 0)
+    CU_TRY(ctx, cudaMemcpyAsync(ctx->stage.p, points, (size_t)total * stride, cudaMemcpyHostToDevice, ctx->stream));
+  CU_TRY(ctx, cudaMemcpyAsync(ctx->offsets.p, offsets, sizeof(int64_t) * ((size_t)n + 1), cudaMemcpyHostToDevice,
+                              ctx->stream));
+  const Store &st = ctx->store;
+  pack_rows_kernel<<<n, 256, 0, ctx->stream>>>((const unsigned char *)ctx->stage.p, stride, (const long long *)ctx->offsets.p,
+                                               n, st.pitch, (float2 *)st.rows.p + (size_t)st.n_scans * st.pitch,
+                                               (int32_t *)st.count.p + st.n_scans, (int *)ctx->d_bad.p);
+  ctx->launches++;
+  CU_TRY(ctx, cudaGetLastError());
+  return DPGICP_OK;
+}
+
+/* the counts of the n rows just written behind n_scans back to the host (only those) + the range flag.  The store takes
+ * the rows only when every point is in range; otherwise n_scans stays where make_room left it: an append keeps its old
+ * rows and count, a replace leaves an empty store. */
+int commit_rows(dpgicp_ctx *ctx, int32_t n) {
+  Store &st = ctx->store;
   const size_t first = (size_t)st.n_scans;
-  st.h_count.resize(first + (size_t)n_new);
+  st.h_count.resize(first + (size_t)n);
   int bad = 0;
-  CU_TRY(ctx, cudaMemcpyAsync(st.h_count.data() + first, (const int32_t *)st.count.p + first, sizeof(int32_t) * (size_t)n_new,
+  CU_TRY(ctx, cudaMemcpyAsync(st.h_count.data() + first, (const int32_t *)st.count.p + first, sizeof(int32_t) * (size_t)n,
                               cudaMemcpyDeviceToHost, ctx->stream));
-  CU_TRY(ctx, cudaMemcpyAsync(&bad, ctx->d_bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  CU_TRY(ctx, cudaMemcpyAsync(&bad, ctx->d_bad.p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
   CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
   if (bad) {
     st.h_count.resize(first);
-    return fail(ctx, DPGICP_E_RANGE, "appended scans hold a non-finite point or |coordinate| > DPGICP_MAX_ABS_COORD; "
-                                     "the store is unchanged");
+    return fail(ctx, DPGICP_E_RANGE, "the scans hold a non-finite point or |coordinate| > DPGICP_MAX_ABS_COORD and were not "
+                                     "stored (an append leaves the store as it was, a full upload leaves it empty)");
   }
-  if (first == 0) st.max_count = 0;
   for (size_t k = first; k < st.h_count.size(); ++k) st.max_count = std::max(st.max_count, st.h_count[k]);
   st.n_scans = (int32_t)st.h_count.size();
   return mark_written(ctx);
 }
 
-/* the device cells and events of a slot (own_stream: a stream of its own, else the context's) */
+/* the device cells and events of a slot (own_stream: a stream of its own, else the context's); on failure, deleting the
+ * slot frees what was made */
 cudaError_t slot_init(dpgicp_slot *s, dpgicp_ctx *ctx, bool own_stream) {
   s->ctx = ctx;
-  cudaError_t e = cudaMalloc((void **)&s->d_queue, 32 * sizeof(unsigned long long));
-  for (cudaEvent_t &ev : s->stage_ev)
-    if (e == cudaSuccess) e = cudaEventCreate(&ev);
-  if (e == cudaSuccess && own_stream) e = cudaStreamCreateWithFlags(&s->own, cudaStreamNonBlocking);
+  cudaError_t e = s->d_queue.alloc(32 * sizeof(unsigned long long));
+  for (Event &ev : s->stage_ev)
+    if (e == cudaSuccess) e = cudaEventCreate(&ev.h);
+  if (e == cudaSuccess && own_stream) e = cudaStreamCreateWithFlags(&s->own.h, cudaStreamNonBlocking);
   return e;
-}
-
-void release_batch(Batch &b) {
-  release(b.tasks); release(b.results); release(b.order);
-  if (b.h_tasks) cudaFreeHost(b.h_tasks);
-  if (b.h_tasks_free) cudaEventDestroy(b.h_tasks_free);
-  b.h_tasks = nullptr; b.h_tasks_free = nullptr;
-}
-
-/* after the slot's stream has drained */
-void slot_release(dpgicp_slot *s) {
-  release_batch(s->batch);
-  for (int k = 0; k < 2; ++k) { release(s->state[k]); release(s->susp[k]); }
-  if (s->d_queue) cudaFree(s->d_queue);
-  for (cudaEvent_t e : s->stage_ev) if (e) cudaEventDestroy(e);
-  if (s->own) cudaStreamDestroy(s->own);
 }
 
 /* slot handles a caller holds: a destroyed (or never created) handle is refused, not followed */
@@ -990,13 +1028,14 @@ int dpgicp_create(int device, dpgicp_ctx **out) {
     return fail(nullptr, DPGICP_E_NODEVICE, "device is not sm_100 class; this library is built for sm_100a only");
   }
   ctx->sm_count = prop.multiProcessorCount;
-  if ((e = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking)) != cudaSuccess ||
-      (e = cudaMalloc((void **)&ctx->d_bad, sizeof(int))) != cudaSuccess ||
-      (e = cudaEventCreateWithFlags(&ctx->written, cudaEventDisableTiming)) != cudaSuccess ||
+  if ((e = cudaStreamCreateWithFlags(&ctx->own_stream.h, cudaStreamNonBlocking)) != cudaSuccess ||
+      (e = ctx->d_bad.alloc(sizeof(int))) != cudaSuccess ||
+      (e = cudaEventCreateWithFlags(&ctx->written.h, cudaEventDisableTiming)) != cudaSuccess ||
       (e = slot_init(&ctx->main, ctx, false)) != cudaSuccess) {
-    delete ctx;
+    delete ctx;                               /* frees what was made */
     return fail(nullptr, DPGICP_E_CUDA, cudaGetErrorString(e));
   }
+  ctx->stream = ctx->own_stream;
   if (const char *w = std::getenv("DPGICP_WARPS")) ctx->force_warps = std::atoi(w);
   if (const char *c = std::getenv("DPGICP_CTAS_PER_SM")) ctx->force_ctas_per_sm = std::atoi(c);
   if (const char *c = std::getenv("DPGICP_HANDOVER")) {
@@ -1021,21 +1060,8 @@ void dpgicp_destroy(dpgicp_ctx *ctx) {
   if (!ctx) return;
   cudaSetDevice(ctx->device);
   while (!ctx->slots.empty()) dpgicp_slot_destroy(ctx->slots.back());
-  cudaStreamSynchronize(ctx->stream);
-  for (Store *s : {&ctx->store, &ctx->scratch_store}) { release(s->rows); release(s->count); }
-  release_batch(ctx->scratch_batch);
-  slot_release(&ctx->main);
-  if (ctx->written) cudaEventDestroy(ctx->written);
-  release(ctx->nodes.xy); release(ctx->nodes.aux); release(ctx->nodes.pass); release(ctx->nodes.boxes);
-  release(ctx->list_nodes.xy); release(ctx->list_nodes.aux); release(ctx->list_nodes.pass); release(ctx->list_nodes.boxes);
-  release(ctx->enum_cnt); release(ctx->enum_amb); release(ctx->d_pair);
-  if (ctx->h_pair) cudaFreeHost(ctx->h_pair);
+  cudaStreamSynchronize(ctx->stream);         /* the members, which the stream's work may read, go only after it drained */
   gather_close(ctx);
-  release(ctx->gather);
-  release(ctx->stage); release(ctx->offsets); release(ctx->misc); release(ctx->corr); release(ctx->trig);
-  if (ctx->d_bad) cudaFree(ctx->d_bad);
-  if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
-  if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
   delete ctx;
 }
 
@@ -1046,12 +1072,11 @@ int dpgicp_set_stream(dpgicp_ctx *ctx, void *stream) {
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
   if (stream) {
-    if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
+    ctx->own_stream.reset();                  /* the context's own stream goes; the caller's is never destroyed */
     ctx->stream = (cudaStream_t)stream;
-    ctx->own_stream = false;
   } else if (!ctx->own_stream) {
-    CU_TRY(ctx, cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
-    ctx->own_stream = true;
+    CU_TRY(ctx, cudaStreamCreateWithFlags(&ctx->own_stream.h, cudaStreamNonBlocking));
+    ctx->stream = ctx->own_stream;
   }
   return DPGICP_OK;
 }
@@ -1063,46 +1088,42 @@ int dpgicp_synchronize(dpgicp_ctx *ctx) {
   return DPGICP_OK;
 }
 
+/* the scan-store writers: argument checks, then the write path above */
+static int write_scans(dpgicp_ctx *ctx, bool append, const void *points, size_t stride, const int64_t *offsets,
+                       int32_t n_scans) {
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  int64_t maxc = 0, total = 0;
+  int rc = check_clouds(ctx, points, stride, offsets, n_scans, &maxc, &total);
+  if (rc || (rc = make_room(ctx, append, n_scans, row_pitch(maxc))) || n_scans == 0) return rc;
+  if ((rc = pack_clouds(ctx, points, stride, offsets, n_scans, total))) return rc;
+  return commit_rows(ctx, n_scans);
+}
+
+/* host ranges, converted on the device */
+static int write_ranges(dpgicp_ctx *ctx, bool append, const float *ranges, int32_t n_scans, int32_t n_beams,
+                        float angle_min, float angle_max, float range_max, float lx, float ly, float ltheta) {
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  int rc = check_ranges(ctx, ranges, n_scans, n_beams);
+  if (rc || (rc = make_room(ctx, append, n_scans, row_pitch(n_beams))) || n_scans == 0) return rc;
+  if ((rc = reserve(ctx, ctx->stage, sizeof(float) * (size_t)n_scans * (size_t)n_beams + 16))) return rc;
+  CU_TRY(ctx, cudaMemcpyAsync(ctx->stage.p, ranges, sizeof(float) * (size_t)n_scans * (size_t)n_beams,
+                              cudaMemcpyHostToDevice, ctx->stream));
+  if ((rc = convert_ranges(ctx, (const float *)ctx->stage.p, nullptr, n_scans, n_beams, angle_min, angle_max, range_max,
+                           lx, ly, ltheta)))
+    return rc;
+  return commit_rows(ctx, n_scans);
+}
+
 int dpgicp_upload_scans(dpgicp_ctx *ctx, const void *points, size_t stride, const int64_t *offsets, int32_t n_scans) {
   if (!ctx) return DPGICP_E_INVALID;
-  CU_TRY(ctx, cudaSetDevice(ctx->device));
-  int rc = replace_store(ctx);
-  if (rc) return rc;
-  return upload_scans_into(ctx, ctx->store, points, stride, offsets, n_scans);
+  return write_scans(ctx, false, points, stride, offsets, n_scans);
 }
 
 int dpgicp_upload_ranges(dpgicp_ctx *ctx, const float *ranges, int32_t n_scans, int32_t n_beams, float angle_min,
                          float angle_max, float range_max, float lx, float ly, float ltheta) {
   if (!ctx) return DPGICP_E_INVALID;
   NvtxRange range("dpgicp: upload ranges + scan->cloud");
-  CU_TRY(ctx, cudaSetDevice(ctx->device));
-  if (n_scans < 0 || n_beams < 2 || (n_scans > 0 && !ranges)) return fail(ctx, DPGICP_E_INVALID, "bad range-scan arguments");
-  if (n_beams > DPGICP_MAX_POINTS) return fail(ctx, DPGICP_E_TOOBIG, "n_beams exceeds DPGICP_MAX_POINTS");
-  Store &st = ctx->store;
-  int rc = replace_store(ctx);
-  if (rc) return rc;
-  const int pitch = (n_beams + 1) & ~1;
-  if ((rc = reserve(ctx, st.rows, sizeof(float2) * (size_t)pitch * (size_t)std::max(n_scans, 1)))) return rc;
-  if ((rc = reserve(ctx, st.count, sizeof(int32_t) * (size_t)std::max(n_scans, 1)))) return rc;
-  if ((rc = reserve(ctx, ctx->stage, sizeof(float) * (size_t)n_scans * (size_t)n_beams + 16))) return rc;
-  st.pitch = pitch;
-  st.n_scans = 0;
-  if (n_scans == 0) { st.max_count = 0; st.h_count.clear(); return DPGICP_OK; }
-  CU_TRY(ctx, cudaMemsetAsync(ctx->d_bad, 0, sizeof(int), ctx->stream));
-  CU_TRY(ctx, cudaMemcpyAsync(ctx->stage.p, ranges, sizeof(float) * (size_t)n_scans * (size_t)n_beams,
-                              cudaMemcpyHostToDevice, ctx->stream));
-  /* createNode dpg_slam.cc:497: angle_inc = (max - min) / (n - 1.0), stored as float */
-  const float angle_inc = (float)(((double)(float)(angle_max - angle_min)) / ((double)n_beams - 1.0));
-  const float lc = cosf(ltheta), ls = sinf(ltheta);       /* Eigen::Rotation2Df(ltheta), host libm */
-  const int threads = 128, warps_per_block = threads / 32;
-  const int blocks = (n_scans + warps_per_block - 1) / warps_per_block;
-  if ((rc = ensure_trig(ctx, n_beams, angle_min, angle_inc))) return rc;
-  ranges_to_rows_kernel<<<blocks, threads, 0, ctx->stream>>>((const float *)ctx->stage.p, nullptr, n_scans, n_beams,
-                                                            (const double2 *)ctx->trig.p, range_max, lx, ly, lc, ls, pitch,
-                                                            (float2 *)st.rows.p, (int32_t *)st.count.p, ctx->d_bad);
-  ctx->launches++;
-  CU_TRY(ctx, cudaGetLastError());
-  return finish_store(ctx, st, n_scans);
+  return write_ranges(ctx, false, ranges, n_scans, n_beams, angle_min, angle_max, range_max, lx, ly, ltheta);
 }
 
 int dpgicp_upload_ranges_subset(dpgicp_ctx *ctx, const float *ranges, int32_t n_scans_total, int32_t n_beams,
@@ -1110,22 +1131,13 @@ int dpgicp_upload_ranges_subset(dpgicp_ctx *ctx, const float *ranges, int32_t n_
                                 float lx, float ly, float ltheta) {
   if (!ctx) return DPGICP_E_INVALID;
   CU_TRY(ctx, cudaSetDevice(ctx->device));
-  if (n_scans_total < 0 || n_ids < 0 || n_beams < 2 || (n_ids > 0 && (!ranges || !scan_ids)))
-    return fail(ctx, DPGICP_E_INVALID, "bad range-scan arguments");
-  if (n_beams > DPGICP_MAX_POINTS) return fail(ctx, DPGICP_E_TOOBIG, "n_beams exceeds DPGICP_MAX_POINTS");
+  if (n_scans_total < 0 || (n_ids > 0 && !scan_ids)) return fail(ctx, DPGICP_E_INVALID, "bad range-scan arguments");
+  int rc = check_ranges(ctx, ranges, n_ids, n_beams);
+  if (rc) return rc;
   for (int32_t k = 0; k < n_ids; ++k)
     if (scan_ids[k] < 0 || scan_ids[k] >= n_scans_total)
       return fail(ctx, DPGICP_E_INVALID, "scan id out of range at position " + std::to_string(k));
-  Store &st = ctx->store;
-  int rc = replace_store(ctx);
-  if (rc) return rc;
-  const int pitch = (n_beams + 1) & ~1;
-  if ((rc = reserve(ctx, st.rows, sizeof(float2) * (size_t)pitch * (size_t)std::max(n_ids, 1)))) return rc;
-  if ((rc = reserve(ctx, st.count, sizeof(int32_t) * (size_t)std::max(n_ids, 1)))) return rc;
-  st.pitch = pitch;
-  st.n_scans = 0;
-  if (n_ids == 0) { st.max_count = 0; st.h_count.clear(); return DPGICP_OK; }
-  CU_TRY(ctx, cudaMemsetAsync(ctx->d_bad, 0, sizeof(int), ctx->stream));
+  if ((rc = make_room(ctx, false, n_ids, row_pitch(n_beams))) || n_ids == 0) return rc;
   /* page-locked input: the kernel reads the selected rows straight from host memory, so only they cross the
    * bus and nothing is staged; pageable input: gather the rows through a pinned buffer and copy them */
   cudaPointerAttributes attr;
@@ -1141,88 +1153,29 @@ int dpgicp_upload_ranges_subset(dpgicp_ctx *ctx, const float *ranges, int32_t n_
     d_ids = (const int32_t *)ctx->offsets.p;
   } else {
     const size_t bytes = sizeof(float) * (size_t)n_ids * (size_t)n_beams;
-    if (bytes > ctx->h_stage_cap) {
-      if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
-      ctx->h_stage = nullptr; ctx->h_stage_cap = 0;
-      CU_TRY(ctx, cudaMallocHost(&ctx->h_stage, bytes));
-      ctx->h_stage_cap = bytes;
-    }
     CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));       /* the buffer may still feed a previous copy */
+    if ((rc = reserve(ctx, ctx->h_stage, bytes))) return rc;
     for (int32_t k = 0; k < n_ids; ++k)
-      std::memcpy((float *)ctx->h_stage + (size_t)k * n_beams, ranges + (size_t)scan_ids[k] * n_beams, sizeof(float) * (size_t)n_beams);
+      std::memcpy((float *)ctx->h_stage.p + (size_t)k * n_beams, ranges + (size_t)scan_ids[k] * n_beams, sizeof(float) * (size_t)n_beams);
     if ((rc = reserve(ctx, ctx->stage, bytes + 16))) return rc;
-    CU_TRY(ctx, cudaMemcpyAsync(ctx->stage.p, ctx->h_stage, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    CU_TRY(ctx, cudaMemcpyAsync(ctx->stage.p, ctx->h_stage.p, bytes, cudaMemcpyHostToDevice, ctx->stream));
     d_in = (const float *)ctx->stage.p;
   }
-  const float angle_inc = (float)(((double)(float)(angle_max - angle_min)) / ((double)n_beams - 1.0));
-  const float lc = cosf(ltheta), ls = sinf(ltheta);
-  const int threads = 128, warps_per_block = threads / 32;
-  const int blocks = (n_ids + warps_per_block - 1) / warps_per_block;
-  if ((rc = ensure_trig(ctx, n_beams, angle_min, angle_inc))) return rc;
-  ranges_to_rows_kernel<<<blocks, threads, 0, ctx->stream>>>(d_in, d_ids, n_ids, n_beams, (const double2 *)ctx->trig.p, range_max,
-                                                            lx, ly, lc, ls, pitch, (float2 *)st.rows.p, (int32_t *)st.count.p, ctx->d_bad);
-  ctx->launches++;
-  CU_TRY(ctx, cudaGetLastError());
-  return finish_store(ctx, st, n_ids);
+  if ((rc = convert_ranges(ctx, d_in, d_ids, n_ids, n_beams, angle_min, angle_max, range_max, lx, ly, ltheta))) return rc;
+  return commit_rows(ctx, n_ids);
 }
 
 int dpgicp_append_ranges(dpgicp_ctx *ctx, const float *ranges, int32_t n_scans, int32_t n_beams, float angle_min,
                          float angle_max, float range_max, float lx, float ly, float ltheta) {
   if (!ctx) return DPGICP_E_INVALID;
   NvtxRange range("dpgicp: append ranges + scan->cloud");
-  CU_TRY(ctx, cudaSetDevice(ctx->device));
-  if (n_scans < 0 || n_beams < 2 || (n_scans > 0 && !ranges)) return fail(ctx, DPGICP_E_INVALID, "bad range-scan arguments");
-  if (n_beams > DPGICP_MAX_POINTS) return fail(ctx, DPGICP_E_TOOBIG, "n_beams exceeds DPGICP_MAX_POINTS");
-  Store &st = ctx->store;
-  if ((int64_t)st.n_scans + n_scans > INT32_MAX) return fail(ctx, DPGICP_E_INVALID, "the store would hold more than 2^31 - 1 scans");
-  if (n_scans == 0) return DPGICP_OK;
-  const int first = st.n_scans;
-  int rc;
-  if ((rc = grow_store(ctx, st, n_scans, (n_beams + 1) & ~1))) return rc;
-  if ((rc = reserve(ctx, ctx->stage, sizeof(float) * (size_t)n_scans * (size_t)n_beams + 16))) return rc;
-  CU_TRY(ctx, cudaMemsetAsync(ctx->d_bad, 0, sizeof(int), ctx->stream));
-  CU_TRY(ctx, cudaMemcpyAsync(ctx->stage.p, ranges, sizeof(float) * (size_t)n_scans * (size_t)n_beams,
-                              cudaMemcpyHostToDevice, ctx->stream));
-  /* the conversion of dpgicp_upload_ranges, writing rows first .. first + n_scans - 1 */
-  const float angle_inc = (float)(((double)(float)(angle_max - angle_min)) / ((double)n_beams - 1.0));
-  const float lc = cosf(ltheta), ls = sinf(ltheta);
-  const int threads = 128, warps_per_block = threads / 32;
-  const int blocks = (n_scans + warps_per_block - 1) / warps_per_block;
-  if ((rc = ensure_trig(ctx, n_beams, angle_min, angle_inc))) return rc;
-  ranges_to_rows_kernel<<<blocks, threads, 0, ctx->stream>>>((const float *)ctx->stage.p, nullptr, n_scans, n_beams,
-                                                            (const double2 *)ctx->trig.p, range_max, lx, ly, lc, ls, st.pitch,
-                                                            (float2 *)st.rows.p + (size_t)first * st.pitch,
-                                                            (int32_t *)st.count.p + first, ctx->d_bad);
-  ctx->launches++;
-  CU_TRY(ctx, cudaGetLastError());
-  return finish_append(ctx, st, n_scans);
+  return write_ranges(ctx, true, ranges, n_scans, n_beams, angle_min, angle_max, range_max, lx, ly, ltheta);
 }
 
 int dpgicp_append_scans(dpgicp_ctx *ctx, const void *points, size_t stride, const int64_t *offsets, int32_t n_scans) {
   if (!ctx) return DPGICP_E_INVALID;
   NvtxRange range("dpgicp: append clouds");
-  CU_TRY(ctx, cudaSetDevice(ctx->device));
-  int64_t maxc = 0, total = 0;
-  int rc = check_clouds(ctx, points, stride, offsets, n_scans, &maxc, &total);
-  if (rc) return rc;
-  Store &st = ctx->store;
-  if ((int64_t)st.n_scans + n_scans > INT32_MAX) return fail(ctx, DPGICP_E_INVALID, "the store would hold more than 2^31 - 1 scans");
-  if (n_scans == 0) return DPGICP_OK;
-  const int first = st.n_scans;
-  if ((rc = grow_store(ctx, st, n_scans, (int)std::max<int64_t>(2, (maxc + 1) & ~(int64_t)1)))) return rc;
-  if ((rc = reserve(ctx, ctx->stage, (size_t)total * stride + 16))) return rc;
-  if ((rc = reserve(ctx, ctx->offsets, sizeof(int64_t) * ((size_t)n_scans + 1)))) return rc;
-  CU_TRY(ctx, cudaMemsetAsync(ctx->d_bad, 0, sizeof(int), ctx->stream));
-  if (total > 0)
-    CU_TRY(ctx, cudaMemcpyAsync(ctx->stage.p, points, (size_t)total * stride, cudaMemcpyHostToDevice, ctx->stream));
-  CU_TRY(ctx, cudaMemcpyAsync(ctx->offsets.p, offsets, sizeof(int64_t) * ((size_t)n_scans + 1), cudaMemcpyHostToDevice,
-                              ctx->stream));
-  pack_rows_kernel<<<n_scans, 256, 0, ctx->stream>>>((const unsigned char *)ctx->stage.p, stride, (const long long *)ctx->offsets.p,
-                                                     n_scans, st.pitch, (float2 *)st.rows.p + (size_t)first * st.pitch,
-                                                     (int32_t *)st.count.p + first, ctx->d_bad);
-  ctx->launches++;
-  CU_TRY(ctx, cudaGetLastError());
-  return finish_append(ctx, st, n_scans);
+  return write_scans(ctx, true, points, stride, offsets, n_scans);
 }
 
 int dpgicp_scan_count(const dpgicp_ctx *ctx) { return ctx ? ctx->store.n_scans : DPGICP_E_INVALID; }
@@ -1387,7 +1340,7 @@ static int gather_export_impl(dpgicp_ctx *ctx, int64_t n_global, int64_t n_alloc
   if (ctx->gather_world > 0)
     return fail(ctx, DPGICP_E_STATE, "gather buffers are attached (peers may still store into this one): dpgicp_gather_detach on every rank first");
   /* a dedicated cudaMalloc allocation (IPC handles cover whole allocations) */
-  release(ctx->gather);
+  ctx->gather.release();
   int rc;
   if ((rc = reserve(ctx, ctx->gather, sizeof(dpgicp_result) * (size_t)std::max<int64_t>(n_alloc, 1)))) return rc;
   CU_TRY(ctx, cudaMemsetAsync(ctx->gather.p, 0, ctx->gather.cap, ctx->stream));
@@ -1447,7 +1400,7 @@ int dpgicp_gather_attach_local(dpgicp_ctx **ctxs, int32_t world, int64_t n_globa
     CU_TRY(ctx, cudaSetDevice(ctx->device));
     CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     gather_close(ctx);
-    release(ctx->gather);
+    ctx->gather.release();
     const int64_t want = (root_only && r > 0) ? 1 : std::max<int64_t>(n_global, 1);
     int rc;
     if ((rc = reserve(ctx, ctx->gather, sizeof(dpgicp_result) * (size_t)want))) return rc;
@@ -1512,7 +1465,7 @@ static int last_run_counters_slot(dpgicp_slot *s, uint64_t counters[8]) {
   dpgicp_ctx *ctx = s->ctx;
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   unsigned long long h[8];
-  CU_TRY(ctx, cudaMemcpyAsync(h, s->d_queue + 8, sizeof(h), cudaMemcpyDeviceToHost, stream_of(s)));
+  CU_TRY(ctx, cudaMemcpyAsync(h, (const unsigned long long *)s->d_queue.p + 8, sizeof(h), cudaMemcpyDeviceToHost, stream_of(s)));
   CU_TRY(ctx, cudaStreamSynchronize(stream_of(s)));
   for (int k = 0; k < 8; ++k) counters[k] = h[k];
   counters[4] = ctx->launches;
@@ -1528,7 +1481,7 @@ int dpgicp_last_run_counters(dpgicp_ctx *ctx, uint64_t counters[8]) {
 /* development builds only: cycles thread 0 spent in each phase of the pass loop, summed over pairs */
 int dpgicp_debug_phase_counters(dpgicp_ctx *ctx, uint64_t out[8]) {
   unsigned long long h[8];
-  CU_TRY(ctx, cudaMemcpyAsync(h, ctx->main.d_queue + 16, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+  CU_TRY(ctx, cudaMemcpyAsync(h, (const unsigned long long *)ctx->main.d_queue.p + 16, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
   CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
   for (int k = 0; k < 8; ++k) out[k] = h[k];
   return DPGICP_OK;
@@ -1684,9 +1637,9 @@ int dpgicp_cov_pairs(dpgicp_ctx *ctx, const int32_t *data_idx, const int32_t *mo
   CovItem *d_items = (CovItem *)(base + b_cov);
   uint32_t *d_status = (uint32_t *)(base + b_cov + b_items);
   CU_TRY(ctx, cudaMemcpyAsync(d_items, items.data(), b_items, cudaMemcpyHostToDevice, ctx->stream));
-  cudaEvent_t e0, e1;
-  CU_TRY(ctx, cudaEventCreate(&e0));
-  CU_TRY(ctx, cudaEventCreate(&e1));
+  Event e0, e1;
+  CU_TRY(ctx, cudaEventCreate(&e0.h));
+  CU_TRY(ctx, cudaEventCreate(&e1.h));
   CU_TRY(ctx, cudaEventRecord(e0, ctx->stream));
   /* one warp per item: no block reduction, the most independent items in flight (measured on B200 with a store larger
    * than L2: 82 % of the measured HBM copy bandwidth with 1 warp per item, 66 / 53 / 33 % with 2 / 4 / 8) */
@@ -1706,7 +1659,6 @@ int dpgicp_cov_pairs(dpgicp_ctx *ctx, const int32_t *data_idx, const int32_t *mo
   CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
   float ms = 0.f;
   cudaEventElapsedTime(&ms, e0, e1);
-  cudaEventDestroy(e0); cudaEventDestroy(e1);
   if (kernel_ms) *kernel_ms = ms;
   return DPGICP_OK;
 }
@@ -1783,29 +1735,10 @@ int dpgicp_convert_ranges_device(dpgicp_ctx *ctx, const float *d_ranges, int32_t
                                  float angle_max, float range_max, float lx, float ly, float ltheta) {
   if (!ctx) return DPGICP_E_INVALID;
   CU_TRY(ctx, cudaSetDevice(ctx->device));
-  if (n_scans < 0 || n_beams < 2 || (n_scans > 0 && !d_ranges)) return fail(ctx, DPGICP_E_INVALID, "bad range-scan arguments");
-  if (n_beams > DPGICP_MAX_POINTS) return fail(ctx, DPGICP_E_TOOBIG, "n_beams exceeds DPGICP_MAX_POINTS");
-  Store &st = ctx->store;
-  int rc = replace_store(ctx);
-  if (rc) return rc;
-  const int pitch = (n_beams + 1) & ~1;
-  if ((rc = reserve(ctx, st.rows, sizeof(float2) * (size_t)pitch * (size_t)std::max(n_scans, 1)))) return rc;
-  if ((rc = reserve(ctx, st.count, sizeof(int32_t) * (size_t)std::max(n_scans, 1)))) return rc;
-  st.pitch = pitch;
-  st.n_scans = 0;
-  if (n_scans == 0) { st.max_count = 0; st.h_count.clear(); return DPGICP_OK; }
-  CU_TRY(ctx, cudaMemsetAsync(ctx->d_bad, 0, sizeof(int), ctx->stream));
-  const float angle_inc = (float)(((double)(float)(angle_max - angle_min)) / ((double)n_beams - 1.0));
-  const float lc = cosf(ltheta), ls = sinf(ltheta);
-  const int threads = 128, warps_per_block = threads / 32;
-  const int blocks = (n_scans + warps_per_block - 1) / warps_per_block;
-  if ((rc = ensure_trig(ctx, n_beams, angle_min, angle_inc))) return rc;
-  ranges_to_rows_kernel<<<blocks, threads, 0, ctx->stream>>>(d_ranges, nullptr, n_scans, n_beams, (const double2 *)ctx->trig.p,
-                                                            range_max, lx, ly, lc, ls, pitch, (float2 *)st.rows.p,
-                                                            (int32_t *)st.count.p, ctx->d_bad);
-  ctx->launches++;
-  CU_TRY(ctx, cudaGetLastError());
-  return finish_store(ctx, st, n_scans);
+  int rc = check_ranges(ctx, d_ranges, n_scans, n_beams);
+  if (rc || (rc = make_room(ctx, false, n_scans, row_pitch(n_beams))) || n_scans == 0) return rc;
+  if ((rc = convert_ranges(ctx, d_ranges, nullptr, n_scans, n_beams, angle_min, angle_max, range_max, lx, ly, ltheta))) return rc;
+  return commit_rows(ctx, n_scans);
 }
 
 int dpgicp_enable_stage_timing(dpgicp_ctx *ctx, int32_t on) {
@@ -1832,9 +1765,9 @@ int dpgicp_fp32_probe(dpgicp_ctx *ctx, double *mul_add, double *fma) {
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   int rc;
   if ((rc = reserve(ctx, ctx->misc, 256))) return rc;
-  cudaEvent_t e0, e1;
-  CU_TRY(ctx, cudaEventCreate(&e0));
-  CU_TRY(ctx, cudaEventCreate(&e1));
+  Event e0, e1;
+  CU_TRY(ctx, cudaEventCreate(&e0.h));
+  CU_TRY(ctx, cudaEventCreate(&e1.h));
   const int iters = 1 << 14, blocks = ctx->sm_count * 8, threads = 256;
   double best[2] = {0.0, 0.0};
   for (int mode = 0; mode < 2; ++mode) {
@@ -1852,7 +1785,6 @@ int dpgicp_fp32_probe(dpgicp_ctx *ctx, double *mul_add, double *fma) {
       if (rep > 0 && ms > 0.f) best[mode] = std::max(best[mode], ops / (ms * 1e-3));
     }
   }
-  cudaEventDestroy(e0); cudaEventDestroy(e1);
   *mul_add = best[0]; *fma = best[1];
   return DPGICP_OK;
 }
@@ -1862,9 +1794,9 @@ int dpgicp_fp32x2_probe(dpgicp_ctx *ctx, double *mul_add_packed) {
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   int rc;
   if ((rc = reserve(ctx, ctx->misc, 256))) return rc;
-  cudaEvent_t e0, e1;
-  CU_TRY(ctx, cudaEventCreate(&e0));
-  CU_TRY(ctx, cudaEventCreate(&e1));
+  Event e0, e1;
+  CU_TRY(ctx, cudaEventCreate(&e0.h));
+  CU_TRY(ctx, cudaEventCreate(&e1.h));
   const int iters = 1 << 14, blocks = ctx->sm_count * 8, threads = 256;
   double best = 0.0;
   for (int rep = 0; rep < 4; ++rep) {             /* rep 0 warms up */
@@ -1879,7 +1811,6 @@ int dpgicp_fp32x2_probe(dpgicp_ctx *ctx, double *mul_add_packed) {
     const double ops = (double)blocks * threads * (double)iters * 8.0 * 4.0;   /* FMUL2 + packed sum = 2 instructions, 4 operations */
     if (rep > 0 && ms > 0.f) best = std::max(best, ops / (ms * 1e-3));
   }
-  cudaEventDestroy(e0); cudaEventDestroy(e1);
   *mul_add_packed = best;
   return DPGICP_OK;
 }
@@ -1894,7 +1825,6 @@ int dpgicp_slot_create(dpgicp_ctx *ctx, dpgicp_slot **out) {
   s->batch.n_pairs = -1;                     /* no pair list yet: a run is refused */
   cudaError_t e = slot_init(s, ctx, true);
   if (e != cudaSuccess) {
-    slot_release(s);
     delete s;
     return fail(ctx, e == cudaErrorMemoryAllocation ? DPGICP_E_NOMEM : DPGICP_E_CUDA, std::string("dpgicp_slot_create: ") + cudaGetErrorString(e));
   }
@@ -1916,9 +1846,8 @@ int dpgicp_slot_destroy(dpgicp_slot *slot) {
   }
   dpgicp_ctx *ctx = s->ctx;
   cudaSetDevice(ctx->device);
-  cudaStreamSynchronize(s->own);
+  cudaStreamSynchronize(s->own);              /* the members, which the slot's work may read, go only after it drained */
   ctx->slots.erase(std::find(ctx->slots.begin(), ctx->slots.end(), s));
-  slot_release(s);
   delete s;
   return DPGICP_OK;
 }

@@ -1,6 +1,7 @@
 """GPU (B200): the scan store grown one node at a time (dpgicp_append_ranges / dpgicp_append_scans) and the reference's
 online loop replayed on it.  An appended store holds the rows one upload of the same scans would hold, so every record
-is independent of how the store was built; a failed append leaves the store as it was; appends are stream-ordered
+is independent of how the store was built; a failed append leaves the store as it was; a store write refused for its
+arguments leaves the store and every batch as they were; appends are stream-ordered
 behind a run already enqueued; the online replay (append -> set_nodes -> enumerate ONLINE -> run, reoptimize at each
 pass boundary) equals the CPU oracle update by update, and the C++ runner's --replay writes the same records."""
 import json
@@ -171,6 +172,47 @@ def test_failed_append_leaves_the_store_as_it_was():
         sm.append_scans(*_csr([long_cloud]))
         assert sm.scan_count == 51 and sm.download_scan(50).tobytes() == long_cloud.tobytes()
         _assert_rows_equal(_rows(sm, 50), before, "after the next append")
+
+
+def test_refused_store_writes_touch_nothing():
+    """every store writer refuses bad arguments before it touches the store, the batches or the slots"""
+    wl = synth.config_corridor(n_pairs=600, seed=38)
+    sc = wl.scanner
+    p = Params.defaults(downsample_divisor=1, cov_mode=COV_CENSI_CORR)
+    half = len(wl.src_idx) // 2
+    with ScanMatcher(0) as sm:
+        sm.upload_ranges(wl.ranges, sc)
+        row = sm.download_scan(7)
+        slot = sm.slot()
+        sm.set_pairs(wl.src_idx[:half], wl.tgt_idx[:half], wl.guess[:half])
+        slot.set_pairs(wl.src_idx[half:], wl.tgt_idx[half:], wl.guess[half:])
+        sm.run(p)
+        slot.run(p)
+        want = sm.fetch_results(), slot.fetch_results()
+        lib, h = sm._lib, sm._h
+        geo = (sc.angle_min, sc.angle_max, sc.range_max, 0.2, 0.0, 0.0)
+        pts, off = np.zeros((4, 2), np.float32), np.array([0, 4], np.int64)
+        wide = np.ones((1, 8193), np.float32)
+        ids = np.array([0, 1], np.int32)                             # scan 1 of a one-scan array: out of range
+        off_wide = np.array([0, 8193], np.int64)
+        attempts = [
+            ("upload_scans", E_INVALID, lambda: lib.dpgicp_upload_scans(h, pts.ctypes.data, 6, off.ctypes.data, 1)),
+            ("upload_ranges", E_TOOBIG, lambda: lib.dpgicp_upload_ranges(h, wide.ctypes.data, 1, 8193, *geo)),
+            ("upload_ranges_subset", E_INVALID,
+             lambda: lib.dpgicp_upload_ranges_subset(h, wl.ranges.ctypes.data, 1, wl.ranges.shape[1], ids.ctypes.data, 2,
+                                                     *geo)),
+            ("convert_ranges_device", E_INVALID, lambda: lib.dpgicp_convert_ranges_device(h, None, 1, 1081, *geo)),
+            ("append_ranges", E_INVALID, lambda: lib.dpgicp_append_ranges(h, wide.ctypes.data, 1, 1, *geo)),
+            ("append_scans", E_TOOBIG, lambda: lib.dpgicp_append_scans(h, wide.ctypes.data, 8, off_wide.ctypes.data, 1)),
+        ]
+        for name, code, call in attempts:
+            assert call() == code, name
+            assert sm.scan_count == wl.n_scans, name
+            assert sm.download_scan(7).tobytes() == row.tobytes(), name
+            sm.run(p)
+            slot.run(p)
+            assert sm.fetch_results().tobytes() == want[0].tobytes(), name
+            assert slot.fetch_results().tobytes() == want[1].tobytes(), name
 
 
 # ---- 4. an append is stream-ordered behind a run already enqueued ----------------------------------------------------
