@@ -121,7 +121,7 @@ EXPORTS = [
     "dpgicp_slot_create", "dpgicp_slot_destroy", "dpgicp_slot_set_pairs", "dpgicp_slot_set_pair_cost_hints",
     "dpgicp_slot_run", "dpgicp_slot_run_range", "dpgicp_slot_fetch_results", "dpgicp_slot_fetch_results_range",
     "dpgicp_slot_fetch_factors", "dpgicp_slot_fetch_pairs", "dpgicp_slot_last_run_counters", "dpgicp_slot_synchronize",
-    "dpgicp_slot_query", "dpgicp_slot_enumerate_pairs_device",
+    "dpgicp_slot_query", "dpgicp_slot_enumerate_pairs_device", "dpgicp_update_nodes",
 ]
 
 _lib = None
@@ -185,6 +185,7 @@ def load_library() -> C.CDLL:
                                               C.POINTER(i64)]),
         "dpgicp_correspondences_seeded": (C.c_int, [vp, vp, i32, vp, i32, sz, vp, PP, vp, vp, vp, vp]),
         "dpgicp_set_nodes": (C.c_int, [vp, vp, vp, i32]),
+        "dpgicp_update_nodes": (C.c_int, [vp, i32, vp, vp, vp, i32]),
         "dpgicp_enumerate_pairs_device": (C.c_int, [vp, i32, C.c_float, C.c_float, i32, i32, C.POINTER(i64), C.POINTER(i64)]),
         "dpgicp_fetch_pairs": (C.c_int, [vp, vp, vp, vp, i64]),
         "dpgicp_convert_ranges_device": (C.c_int, [vp, vp, i32, i32] + [C.c_float] * 6),

@@ -25,6 +25,9 @@
  * --inflight K (K >= 2) enumerates the pair list into K batch slots of one context and runs it in batches of
  * --batch-pairs pairs with K batches in flight (batch b on slot b % K, launched once that slot's previous batch is
  * fetched).  The CSV is identical to --inflight 1.
+ * --nodes full|sync (with --replay) chooses how each alignment batch brings the node table up to date: full sends the
+ * whole table (dpgicp_set_nodes), sync sends the estimates that changed since the last batch and the new node
+ * (ScanMatcher::syncNodes -> dpgicp_update_nodes).  The CSV is identical for both.
  */
 #include <algorithm>
 #include <chrono>
@@ -172,9 +175,11 @@ double percentile(std::vector<double> v, double q) {      /* nearest rank */
  *     if k > 0 and pass[k] != pass[k-1]:   reoptimize() over nodes 0..k-1   (incrementPassNumber, slam.cc:25-33)
  *     append scan k                        (createNode, dpg_slam.cc:462-513)
  *     if k >= 1: pairs of node k           (updatePoseGraphObsConstraints, dpg_slam.cc:255-314)
- * Each alignment batch is set_nodes -> enumerate on the device -> run -> records + factors back (the hand-off to
- * addObservationConstraint).  Node estimates are the log's; a pose-graph optimiser would update them in between. */
-int replay(const ScanLog &L, const dpgicp_params &params, float r_same, float r_other, int device, const std::string &csv_out) {
+ * Each alignment batch is node table -> enumerate on the device -> run -> records + factors back (the hand-off to
+ * addObservationConstraint).  Node estimates are the log's; a pose-graph optimiser would update them in between.  The
+ * node table goes whole (set_nodes) or as the rows that changed (sync_nodes). */
+int replay(const ScanLog &L, const dpgicp_params &params, float r_same, float r_other, int device, bool sync_nodes,
+           const std::string &csv_out) {
   dpgicp_shim::ScanMatcher sm(device);
   dpgicp_ctx *ctx = sm.ctx();
   auto check = [&](int rc, const char *what) {
@@ -194,7 +199,8 @@ int replay(const ScanLog &L, const dpgicp_params &params, float r_same, float r_
   /* one alignment batch over nodes 0..n_nodes-1; returns the set_nodes and the enumerate + run + fetch times */
   auto align = [&](int n_nodes, int mode, int update, double *dt_nodes, double *dt_erf) {
     const double t0 = now_s();
-    check(dpgicp_set_nodes(ctx, pose.data(), L.pass.data(), n_nodes), "dpgicp_set_nodes");
+    if (sync_nodes) sm.syncNodes(L.est.data(), L.pass.data(), n_nodes);
+    else check(dpgicp_set_nodes(ctx, pose.data(), L.pass.data(), n_nodes), "dpgicp_set_nodes");
     const double t1 = now_s();
     int64_t n = 0;
     check(dpgicp_enumerate_pairs_device(ctx, mode, r_same, r_other, 0, 1, &n, nullptr), "dpgicp_enumerate_pairs_device");
@@ -235,12 +241,12 @@ int replay(const ScanLog &L, const dpgicp_params &params, float r_same, float r_
     std::fclose(f);
   }
   auto ms = [](const std::vector<double> &v, double q) { return 1e3 * percentile(v, q); };
-  std::printf("{\"mode\": \"replay\", \"scans\": %d, \"beams\": %d, \"online_updates\": %d, \"reoptimize_batches\": %d, "
+  std::printf("{\"mode\": \"replay\", \"nodes\": \"%s\", \"scans\": %d, \"beams\": %d, \"online_updates\": %d, \"reoptimize_batches\": %d, "
               "\"pairs\": %zu, \"online_pairs\": %zu, "
               "\"update_ms_median\": {\"append\": %.4f, \"set_nodes\": %.4f, \"enumerate_run_fetch\": %.4f, \"total\": %.4f}, "
               "\"update_ms_p90\": {\"append\": %.4f, \"set_nodes\": %.4f, \"enumerate_run_fetch\": %.4f, \"total\": %.4f}, "
               "\"replay_s\": %.6f}\n",
-              L.n_scans, L.n_beams, n_online, n_reopt, rows.size(), online_pairs,
+              sync_nodes ? "sync" : "full", L.n_scans, L.n_beams, n_online, n_reopt, rows.size(), online_pairs,
               ms(t_append, 0.5), ms(t_nodes, 0.5), ms(t_erf, 0.5), ms(t_total, 0.5),
               ms(t_append, 0.9), ms(t_nodes, 0.9), ms(t_erf, 0.9), ms(t_total, 0.9), replay_s);
   return 0;
@@ -254,6 +260,7 @@ int main(int argc, char **argv) {
   std::vector<int> devices;
   int32_t caller = DPGICP_ENUM_REOPTIMIZE;
   bool successive_only = false, replay_log = false;
+  std::string nodes = "full";
   int inflight = 1;
   int64_t batch_pairs = 5000;
   uint64_t seed = 2;
@@ -292,6 +299,7 @@ int main(int argc, char **argv) {
     else if (a == "--other-pass-radius") r_other = (float)std::atof(next("--other-pass-radius"));
     else if (a == "--successive-only") successive_only = true;
     else if (a == "--replay") replay_log = true;
+    else if (a == "--nodes") nodes = next("--nodes");
     else if (a == "--inflight") inflight = std::atoi(next("--inflight"));
     else if (a == "--batch-pairs") batch_pairs = std::atoll(next("--batch-pairs"));
     else {
@@ -300,7 +308,7 @@ int main(int argc, char **argv) {
                    "         [--seed S] [--divisor D] [--cov-mode 0|1|2] [--metric 0|1] [--search 0|1|2] [--window W] [--successive-only]\n"
                    "         [--same-pass-radius R] [--other-pass-radius R] [--write-log FILE] [--out FILE.csv] [--device K]\n"
                    "         [--gpus N | --devices a,b,...] [--caller reoptimize|online] [--outlier-mode 0|1|2 --outlier-param X]\n"
-                   "         [--replay] [--inflight K [--batch-pairs N]]\n");
+                   "         [--replay [--nodes full|sync]] [--inflight K [--batch-pairs N]]\n");
       return a == "--help" ? 0 : 2;
     }
   }
@@ -319,6 +327,10 @@ int main(int argc, char **argv) {
                          "supported with --replay, --successive-only, --gpus or --devices\n");
     return 2;
   }
+  if (nodes != "full" && (nodes != "sync" || !replay_log)) {
+    std::fprintf(stderr, "dpg_batch_runner: --nodes is full or sync, and sync applies to --replay only\n");
+    return 2;
+  }
   if (replay_log && !devices.empty()) {
     std::fprintf(stderr, "dpg_batch_runner: --replay runs on one device (--device K); --gpus / --devices are not supported "
                          "with it (online batches are tens of pairs)\n");
@@ -326,7 +338,7 @@ int main(int argc, char **argv) {
   }
 
   try {
-    if (replay_log) return replay(L, params, r_same, r_other, device, csv_out);
+    if (replay_log) return replay(L, params, r_same, r_other, device, nodes == "sync", csv_out);
     std::vector<int32_t> src, tgt;
     std::vector<dpgicp_result> res;
     double t0, t1, t2, t3;

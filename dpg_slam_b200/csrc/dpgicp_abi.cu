@@ -98,12 +98,15 @@ struct Batch {
   int32_t max_scan = -1;         /* device-enumerated lists: highest scan (= node) index used; -1 = validated on the host */
 };
 
-struct Nodes {                   /* pose-graph node estimates on the device (dpgicp_set_nodes) */
+struct Nodes {                   /* pose-graph node estimates on the device (dpgicp_set_nodes, dpgicp_update_nodes) */
   DevBuf xy, aux, pass;          /* float2 (x, y); float4 (theta, cosf(-theta), sinf(-theta), 0); int32 pass */
-  DevBuf boxes;                  /* index-order box hierarchy, all levels back to back */
-  int32_t n = 0;
-  int levels = 0;
+  DevBuf boxes;                  /* index-order box hierarchy, levels back to back, each sized for `cap` nodes */
+  int32_t n = 0, cap = 0;        /* nodes in the table; nodes the buffers hold (grows by doubling) */
+  int levels = 0;                /* levels and level_cnt follow n; level_off follows cap, so growth below cap moves no level */
   int64_t level_off[8] = {0}, level_cnt[8] = {0};
+  HostBuf h_rows;                /* dpgicp_update_nodes: the listed rows and dirty leaves, staged for one copy */
+  DevBuf d_rows;
+  Event rows_free;               /* recorded after the last kernel that reads d_rows: both staging buffers may be rewritten */
 };
 
 }  // namespace
@@ -654,50 +657,181 @@ int two_cloud_store(dpgicp_ctx *ctx, const void *a, int na, const void *b, int n
   return DPGICP_OK;
 }
 
+/* box levels over n >= 1 nodes: L = 1 boxes of 32 nodes, L + 1 boxes of 32 level-L boxes, until one warp can test the
+ * top level at once; cnt[L - 1] = boxes of level L */
+struct Levels {
+  int levels = 0;
+  int64_t cnt[kEnumMaxLevels] = {0};
+};
+Levels box_levels(int64_t n) {
+  Levels lv;
+  int64_t c = n;
+  do {
+    c = (c + kEnumFan - 1) / kEnumFan;
+    lv.cnt[lv.levels++] = c;
+  } while (c > kEnumFan && lv.levels < kEnumMaxLevels);
+  return lv;
+}
+
+void set_levels(Nodes &N, const Levels &lv) {
+  N.levels = lv.levels;
+  for (int L = 0; L < lv.levels; ++L) N.level_cnt[L] = lv.cnt[L];
+}
+
+/* every box level above the leaves, from the leaves up (at most n / 1024 boxes), in the layout `off` */
+void refit_upper_levels(dpgicp_ctx *ctx, NodeBox *bx, const int64_t *off, const Levels &lv) {
+  for (int L = 1; L < lv.levels; ++L) {
+    const int nb = (int)lv.cnt[L], blocks = (nb + 3) / 4;
+    node_boxes_up_kernel<<<blocks, 128, 0, ctx->stream>>>(bx + off[L - 1], (int)lv.cnt[L - 1], bx + off[L], nb);
+    ctx->launches++;
+  }
+}
+
+/* the node row of one estimate: position, and theta with the cos / sin of -theta from the host's libm
+ * (Eigen::Rotation2Df(-theta_1), math_utils.cc:28), which the enumeration's guesses take bit for bit */
+inline void node_row(float x, float y, float th, float2 &xy, float4 &aux) {
+  const float ang = -th;
+  xy = make_float2(x, y);
+  aux = make_float4(th, cosf(ang), sinf(ang), 0.f);
+}
+
+/* Room for n nodes in N.  Capacity grows by doubling and the box levels are laid out for the capacity, so a table that
+ * grows one node at a time reallocates O(log n) times and keeps every level in place in between.  keep: the current
+ * N.n nodes move to the new buffers (rows and leaf boxes device to device, upper levels refit in the new layout), so
+ * the grown table is complete for N.n; the old buffers are freed only after the context's stream has drained.  The
+ * level counts stay those of N.n: the caller sets them with the new count.  On failure N is as it was. */
+int node_room(dpgicp_ctx *ctx, Nodes &N, int32_t n, bool keep) {
+  const Levels lv = box_levels(n);
+  if (lv.cnt[lv.levels - 1] > kEnumFan) return fail(ctx, DPGICP_E_TOOBIG, "too many nodes");
+  if (n <= N.cap) return DPGICP_OK;
+  const int32_t cap = (int32_t)std::min<int64_t>(INT32_MAX, std::max<int64_t>(n, 2 * (int64_t)N.cap));
+  const Levels cap_lv = box_levels(cap);
+  int64_t off[8] = {0}, total = 0;
+  for (int L = 0; L < cap_lv.levels; ++L) { off[L] = total; total += cap_lv.cnt[L]; }
+  DevBuf xy, aux, pass, boxes;
+  CU_TRY(ctx, xy.alloc(sizeof(float2) * (size_t)cap));
+  CU_TRY(ctx, aux.alloc(sizeof(float4) * (size_t)cap));
+  CU_TRY(ctx, pass.alloc(sizeof(int32_t) * (size_t)cap));
+  CU_TRY(ctx, boxes.alloc(sizeof(NodeBox) * (size_t)total));
+  cudaError_t e = cudaSuccess;
+  if (keep && N.n > 0) {
+    const size_t m = (size_t)N.n;
+    Levels old;
+    old.levels = N.levels;
+    for (int L = 0; L < N.levels; ++L) old.cnt[L] = N.level_cnt[L];
+    e = cudaMemcpyAsync(xy.p, N.xy.p, sizeof(float2) * m, cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(aux.p, N.aux.p, sizeof(float4) * m, cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(pass.p, N.pass.p, sizeof(int32_t) * m, cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e == cudaSuccess)
+      e = cudaMemcpyAsync(boxes.p, N.boxes.p, sizeof(NodeBox) * (size_t)old.cnt[0], cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e == cudaSuccess) {
+      refit_upper_levels(ctx, (NodeBox *)boxes.p, off, old);
+      e = cudaGetLastError();
+    }
+  }
+  const cudaError_t s = cudaStreamSynchronize(ctx->stream);   /* before the new buffers or the old ones are freed: an
+                                                               * enqueued kernel may still read the old ones */
+  CU_TRY(ctx, e);
+  CU_TRY(ctx, s);
+  N.xy = std::move(xy); N.aux = std::move(aux); N.pass = std::move(pass); N.boxes = std::move(boxes);
+  N.cap = cap;
+  for (int L = 0; L < 8; ++L) N.level_off[L] = off[L];
+  return DPGICP_OK;
+}
+
 /* node estimates -> node table N on the device, plus the index-order box hierarchy the enumeration walks */
 int set_nodes_impl(dpgicp_ctx *ctx, Nodes &N, const float *pose, const int32_t *pass, int32_t n, bool pose_is_xy) {
   N.n = 0;
   if (n == 0) return DPGICP_OK;
-  std::vector<float> xy((size_t)n * 2), aux((size_t)n * 4);
+  std::vector<float2> xy((size_t)n);
+  std::vector<float4> aux((size_t)n);
   const int stride = pose_is_xy ? 2 : 3;
   for (int32_t k = 0; k < n; ++k) {
     const float x = pose[(size_t)stride * k], y = pose[(size_t)stride * k + 1], th = pose_is_xy ? 0.0f : pose[(size_t)stride * k + 2];
     if (!std::isfinite(x) || !std::isfinite(y) || !std::isfinite(th))
       return fail(ctx, DPGICP_E_RANGE, "non-finite node estimate at node " + std::to_string(k));
-    xy[2 * (size_t)k] = x; xy[2 * (size_t)k + 1] = y;
-    const float ang = -th;                            /* Eigen::Rotation2Df(-theta_1), math_utils.cc:28 */
-    aux[4 * (size_t)k] = th; aux[4 * (size_t)k + 1] = cosf(ang); aux[4 * (size_t)k + 2] = sinf(ang); aux[4 * (size_t)k + 3] = 0.f;
+    node_row(x, y, th, xy[(size_t)k], aux[(size_t)k]);
   }
   int rc;
-  if ((rc = reserve(ctx, N.xy, sizeof(float) * 2 * (size_t)n))) return rc;
-  if ((rc = reserve(ctx, N.aux, sizeof(float) * 4 * (size_t)n))) return rc;
-  if ((rc = reserve(ctx, N.pass, sizeof(int32_t) * (size_t)n))) return rc;
-  /* levels: L = 1 boxes of 32 nodes, L + 1 boxes of 32 level-L boxes, until one warp can test the top level at once */
-  N.levels = 0;
-  int64_t total = 0, cnt = n;
-  do {
-    cnt = (cnt + kEnumFan - 1) / kEnumFan;
-    if (N.levels >= kEnumMaxLevels) return fail(ctx, DPGICP_E_TOOBIG, "too many nodes");
-    N.level_off[N.levels] = total; N.level_cnt[N.levels] = cnt;
-    total += cnt; ++N.levels;
-  } while (cnt > kEnumFan);
-  if ((rc = reserve(ctx, N.boxes, sizeof(NodeBox) * (size_t)total))) return rc;
-  CU_TRY(ctx, cudaMemcpyAsync(N.xy.p, xy.data(), sizeof(float) * 2 * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-  CU_TRY(ctx, cudaMemcpyAsync(N.aux.p, aux.data(), sizeof(float) * 4 * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+  if ((rc = node_room(ctx, N, n, false))) return rc;
+  const Levels lv = box_levels(n);
+  CU_TRY(ctx, cudaMemcpyAsync(N.xy.p, xy.data(), sizeof(float2) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+  CU_TRY(ctx, cudaMemcpyAsync(N.aux.p, aux.data(), sizeof(float4) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
   CU_TRY(ctx, cudaMemcpyAsync(N.pass.p, pass, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-  NodeBox *bx = (NodeBox *)N.boxes.p;
   {
-    const int nb = (int)N.level_cnt[0], blocks = (nb + 3) / 4;
-    node_boxes_leaf_kernel<<<blocks, 128, 0, ctx->stream>>>((const float2 *)N.xy.p, (const int32_t *)N.pass.p, n, bx, nb);
+    const int nb = (int)lv.cnt[0], blocks = (nb + 3) / 4;
+    node_boxes_leaf_kernel<<<blocks, 128, 0, ctx->stream>>>((const float2 *)N.xy.p, (const int32_t *)N.pass.p, n,
+                                                            (NodeBox *)N.boxes.p, nb);
     ctx->launches++;
   }
-  for (int L = 1; L < N.levels; ++L) {
-    const int nb = (int)N.level_cnt[L], blocks = (nb + 3) / 4;
-    node_boxes_up_kernel<<<blocks, 128, 0, ctx->stream>>>(bx + N.level_off[L - 1], (int)N.level_cnt[L - 1], bx + N.level_off[L], nb);
-    ctx->launches++;
-  }
+  refit_upper_levels(ctx, (NodeBox *)N.boxes.p, N.level_off, lv);
   CU_TRY(ctx, cudaGetLastError());
   CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));         /* the host staging vectors go out of scope */
+  set_levels(N, lv);
+  N.n = n;
+  return DPGICP_OK;
+}
+
+/* dpgicp_update_nodes on the context's table: the listed rows and the leaf boxes that hold them, then the upper levels.
+ * Everything is checked on the host before the first device write; host work and copies scale with n_ids.  A CUDA
+ * error once the device work has been enqueued empties the table, as a failed set_nodes_impl does. */
+int update_nodes_impl(dpgicp_ctx *ctx, Nodes &N, int32_t n, const int32_t *ids, const float *pose, const int32_t *pass,
+                      int32_t n_ids) {
+  if (n_ids < 0 || (n_ids > 0 && (!ids || !pose || !pass))) return fail(ctx, DPGICP_E_INVALID, "bad node arguments");
+  if (n < N.n) return fail(ctx, DPGICP_E_INVALID, "n_nodes is below the current node count: the table does not shrink");
+  if (n_ids == 0 && n == N.n) return DPGICP_OK;
+  std::vector<int32_t> copy;                /* ascending ids (what a diff of the estimate vector gives) are used as they are */
+  const int32_t *sorted = ids, *sorted_end = ids + n_ids;
+  if (!std::is_sorted(ids, ids + n_ids)) {
+    copy.assign(ids, ids + n_ids);
+    std::sort(copy.begin(), copy.end());
+    sorted = copy.data(); sorted_end = sorted + n_ids;
+  }
+  if (n_ids > 0 && (sorted[0] < 0 || sorted_end[-1] >= n))
+    return fail(ctx, DPGICP_E_INVALID, "node id out of range [0, n_nodes)");
+  if (std::adjacent_find(sorted, sorted_end) != sorted_end) return fail(ctx, DPGICP_E_INVALID, "duplicate node id");
+  const int64_t listed_new = sorted_end - std::lower_bound(sorted, sorted_end, N.n);
+  if (listed_new != (int64_t)n - N.n) return fail(ctx, DPGICP_E_INVALID, "every new node id in [old count, n_nodes) must be listed");
+  for (int32_t k = 0; k < n_ids; ++k)
+    if (!std::isfinite(pose[3 * (size_t)k]) || !std::isfinite(pose[3 * (size_t)k + 1]) || !std::isfinite(pose[3 * (size_t)k + 2]))
+      return fail(ctx, DPGICP_E_RANGE, "non-finite node estimate at node " + std::to_string(ids[k]));
+  /* dirty leaves: the leaf of every listed id, ascending, once each */
+  std::vector<int32_t> leaves;
+  for (const int32_t *q = sorted; q != sorted_end; ++q)
+    if (leaves.empty() || leaves.back() != *q / kEnumFan) leaves.push_back(*q / kEnumFan);
+  /* staging: aux (float4) | xy (float2) | ids | pass | leaves */
+  const size_t m = (size_t)n_ids, bytes = 32 * m + 4 * leaves.size();
+  if (N.rows_free) CU_TRY(ctx, cudaEventSynchronize(N.rows_free));
+  else CU_TRY(ctx, cudaEventCreateWithFlags(&N.rows_free.h, cudaEventDisableTiming));
+  int rc;
+  if ((rc = reserve(ctx, N.h_rows, std::max(bytes, bytes > N.h_rows.cap ? 2 * N.h_rows.cap : 0)))) return rc;
+  if ((rc = reserve(ctx, N.d_rows, std::max(bytes, bytes > N.d_rows.cap ? 2 * N.d_rows.cap : 0)))) return rc;
+  if ((rc = node_room(ctx, N, n, true))) return rc;
+  const Levels lv = box_levels(n);
+  char *h = (char *)N.h_rows.p;
+  float4 *h_aux = (float4 *)h;
+  float2 *h_xy = (float2 *)(h + 16 * m);
+  std::memcpy(h + 24 * m, ids, 4 * m);
+  std::memcpy(h + 28 * m, pass, 4 * m);
+  std::memcpy(h + 32 * m, leaves.data(), 4 * leaves.size());
+  for (size_t k = 0; k < m; ++k) node_row(pose[3 * k], pose[3 * k + 1], pose[3 * k + 2], h_xy[k], h_aux[k]);
+  const char *d = (const char *)N.d_rows.p;
+  cudaError_t e = cudaMemcpyAsync(N.d_rows.p, h, bytes, cudaMemcpyHostToDevice, ctx->stream);
+  if (e == cudaSuccess) {
+    node_rows_scatter_kernel<<<(n_ids + 127) / 128, 128, 0, ctx->stream>>>(
+        (const int32_t *)(d + 24 * m), (const float2 *)(d + 16 * m), (const float4 *)d, (const int32_t *)(d + 28 * m), n_ids,
+        (float2 *)N.xy.p, (float4 *)N.aux.p, (int32_t *)N.pass.p);
+    const int nl = (int)leaves.size();
+    node_boxes_refit_kernel<<<(nl + 3) / 4, 128, 0, ctx->stream>>>((const float2 *)N.xy.p, (const int32_t *)N.pass.p, n,
+                                                                   (const int32_t *)(d + 32 * m), nl, (NodeBox *)N.boxes.p);
+    ctx->launches += 2;
+    refit_upper_levels(ctx, (NodeBox *)N.boxes.p, N.level_off, lv);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) e = cudaEventRecord(N.rows_free, ctx->stream);
+  if (e != cudaSuccess) N.n = 0;
+  CU_TRY(ctx, e);
+  set_levels(N, lv);
   N.n = n;
   return DPGICP_OK;
 }
@@ -1695,6 +1829,14 @@ int dpgicp_set_nodes(dpgicp_ctx *ctx, const float *pose, const int32_t *pass, in
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   if (n < 0 || (n > 0 && (!pose || !pass))) return fail(ctx, DPGICP_E_INVALID, "bad node arguments");
   return set_nodes_impl(ctx, ctx->nodes, pose, pass, n, false);
+}
+
+int dpgicp_update_nodes(dpgicp_ctx *ctx, int32_t n_nodes, const int32_t *ids, const float *pose, const int32_t *pass,
+                        int32_t n_ids) {
+  if (!ctx) return DPGICP_E_INVALID;
+  NvtxRange range("dpgicp: update nodes");
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  return update_nodes_impl(ctx, ctx->nodes, n_nodes, ids, pose, pass, n_ids);
 }
 
 /* enumeration into slot s: on the context's stream (synchronous, as the host re-derives guesses), after the slot's own

@@ -1848,11 +1848,10 @@ __device__ __forceinline__ bool box_may_pass(const NodeBox bx, float2 q, int pq,
   return lb <= r;                                                 /* empty boxes have lb = +inf / NaN   */
 }
 
-/* leaf boxes: one warp per box of kEnumFan consecutive nodes */
-__global__ void node_boxes_leaf_kernel(const float2 *__restrict__ xy, const int32_t *__restrict__ pass, int n,
-                                       NodeBox *__restrict__ out, int n_boxes) {
-  const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-  if (b >= n_boxes) return;
+/* leaf box b (nodes b * kEnumFan .. + kEnumFan - 1 below n), one warp; node_boxes_leaf_kernel and
+ * node_boxes_refit_kernel share it, so a refit box is bit for bit the rebuilt one */
+__device__ __forceinline__ void node_leaf_box(const float2 *__restrict__ xy, const int32_t *__restrict__ pass, int n, int b,
+                                              int lane, NodeBox *__restrict__ out) {
   const int k = b * kEnumFan + lane;
   const float inf = __int_as_float(0x7f800000);
   float lox = inf, loy = inf, hix = -inf, hiy = -inf;
@@ -1861,6 +1860,34 @@ __global__ void node_boxes_leaf_kernel(const float2 *__restrict__ xy, const int3
   lox = warp_min(lox); loy = warp_min(loy); hix = warp_max(hix); hiy = warp_max(hiy);
   plo = __reduce_min_sync(0xffffffffu, plo); phi = __reduce_max_sync(0xffffffffu, phi);
   if (lane == 0) { NodeBox o = {lox, loy, hix, hiy, plo, phi, 0, 0}; out[b] = o; }
+}
+
+/* leaf boxes: one warp per box of kEnumFan consecutive nodes */
+__global__ void node_boxes_leaf_kernel(const float2 *__restrict__ xy, const int32_t *__restrict__ pass, int n,
+                                       NodeBox *__restrict__ out, int n_boxes) {
+  const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  if (b >= n_boxes) return;
+  node_leaf_box(xy, pass, n, b, lane, out);
+}
+
+/* dpgicp_update_nodes: the listed leaf boxes only (the leaves that hold a changed or new node), one warp per leaf */
+__global__ void node_boxes_refit_kernel(const float2 *__restrict__ xy, const int32_t *__restrict__ pass, int n,
+                                        const int32_t *__restrict__ leaves, int n_leaves, NodeBox *__restrict__ out) {
+  const int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  if (w >= n_leaves) return;
+  node_leaf_box(xy, pass, n, leaves[w], lane, out);
+}
+
+/* dpgicp_update_nodes: node ids[k] takes row k of the staged estimates (one thread per listed node) */
+__global__ void node_rows_scatter_kernel(const int32_t *__restrict__ ids, const float2 *__restrict__ xy_in,
+                                         const float4 *__restrict__ aux_in, const int32_t *__restrict__ pass_in, int n_ids,
+                                         float2 *__restrict__ xy, float4 *__restrict__ aux, int32_t *__restrict__ pass) {
+  const int k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= n_ids) return;
+  const int i = ids[k];
+  xy[i] = xy_in[k];
+  aux[i] = aux_in[k];
+  pass[i] = pass_in[k];
 }
 
 /* parent boxes: one warp per box of kEnumFan consecutive child boxes */

@@ -354,6 +354,28 @@ int  dpgicp_enumerate_pairs(dpgicp_ctx *ctx, const float *node_xy, const int32_t
 #define DPGICP_ENUM_REOPTIMIZE 0
 #define DPGICP_ENUM_ONLINE     1
 int  dpgicp_set_nodes(dpgicp_ctx *ctx, const float *node_pose_xytheta, const int32_t *node_pass, int32_t n_nodes);
+/* Change part of the node table of dpgicp_set_nodes and/or grow it.  After the call the table holds n_nodes nodes;
+ * node ids[k] takes the estimate pose_xytheta[3k..3k+2] and pass[k]; every other node keeps what it had.
+ *   Result: the table is bit for bit what one dpgicp_set_nodes of the equivalent full arrays holds (positions, theta
+ *     and its host-libm cosf / sinf, pass numbers, every box level), so enumerated lists, guesses, records and factors
+ *     are identical too, whatever changed (a node that moves away and shrinks its box, a change of pass range).
+ *   Size: n_nodes >= the current count (a table never set counts as 0, so this call may start one); every id in
+ *     [current count, n_nodes) is listed; ids are distinct and in [0, n_nodes).  n_ids = 0 with an unchanged n_nodes
+ *     does nothing.
+ *   Errors leave the table as it was: DPGICP_E_INVALID for a shrinking n_nodes, a new id not listed, a duplicate or
+ *     out-of-range id, or NULL arrays with n_ids > 0; DPGICP_E_RANGE for a non-finite estimate.  Both are found on the
+ *     host before any device write.  DPGICP_E_NOMEM from the capacity growth also leaves the table as it was; a CUDA
+ *     error (DPGICP_E_CUDA) once the device work has been enqueued empties the table, as a failed dpgicp_set_nodes
+ *     does.
+ *   Cost: host work and the host-to-device copy scale with n_ids, not n_nodes: the listed rows are scattered and only
+ *     the leaf boxes (32 nodes each) that hold a listed node are refit, then the upper levels (at most n_nodes / 1024
+ *     boxes).  Capacity grows by doubling, so appending one node per call is amortised O(1).
+ *   Ordering: as dpgicp_set_nodes.  The table is per context and the enumeration reads it synchronously; a run
+ *     already enqueued in any slot keeps the guesses its batch was enumerated with.  The call returns once its work is
+ *     enqueued on the context's stream.  dpgicp_set_nodes still replaces the whole table and may be mixed with this
+ *     call in any order; dpgicp_enumerate_pairs (host list) uses a table of its own and is unaffected.             */
+int  dpgicp_update_nodes(dpgicp_ctx *ctx, int32_t n_nodes, const int32_t *ids, const float *pose_xytheta,
+                         const int32_t *pass, int32_t n_ids);
 int  dpgicp_enumerate_pairs_device(dpgicp_ctx *ctx, int32_t mode, float same_pass_radius, float other_pass_radius,
                                    int32_t shard_rank, int32_t shard_world, int64_t *n_pairs_total,
                                    int64_t *n_pairs_local);
@@ -409,7 +431,8 @@ int  dpgicp_fp32x2_probe(dpgicp_ctx *ctx, double *ops_per_s_mul_add_packed);
  *     for every slot's enqueued work and empty every slot's batch.  dpgicp_append_* writes only rows no enqueued run
  *     reads and does not wait, unless the store has to move (growth, re-pitch): the old buffers are then freed only
  *     after every slot's stream has drained;
- *   - dpgicp_set_nodes does not wait: no run reads the node table (the enumeration does, and it is synchronous);
+ *   - dpgicp_set_nodes and dpgicp_update_nodes do not wait: no run reads the node table (the enumeration does, and it
+ *     is synchronous);
  *   - dpgicp_slot_enumerate_pairs_device runs on the context's stream and returns when the list is on the device, as
  *     dpgicp_enumerate_pairs_device does; it first waits for the slot's own enqueued work;
  *   - the fused multi-GPU gather (dpgicp_gather_attach*) applies to the default slot only: a slot's run writes its

@@ -17,7 +17,9 @@
 #ifndef DPGICP_SHIM_HPP
 #define DPGICP_SHIM_HPP
 
+#include <algorithm>
 #include <cstdint>
+#include <cstring>
 #include <functional>
 #include <stdexcept>
 #include <string>
@@ -43,6 +45,61 @@ struct IcpResults {             /* the reference's pair<pair<Vector2f,float>, Ma
   double cov[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
   dpgicp_result record{};
 };
+
+/* The node table a context was last sent by syncNodes.  diff() lists the rows of a new estimate vector whose bits
+ * differ from it, then the new rows; it asks for the whole table instead (returns true) when there is no table yet,
+ * the vector is shorter, or more than kFullShare of its rows would go. */
+class NodeMirror {
+ public:
+  /* update_nodes costs host work per listed row, set_nodes per node; at 50 000 nodes on an NVIDIA B200 (1000 W,
+   * 1965 MHz) update_nodes takes 0.37 ms for 25 % of the rows and 0.65 ms for 50 % against 0.47-0.49 ms for set_nodes
+   * (profiles/online_nodes.json, "share": measured through the Python wrapper, which has the same threshold) */
+  static constexpr double kFullShare = 0.3;
+  bool diff(const Pose2f *poses, const int32_t *pass, int32_t n, std::vector<int32_t> &ids, std::vector<float> &flat,
+            std::vector<int32_t> &ids_pass) const {
+    ids.clear(); flat.clear(); ids_pass.clear();
+    if (!valid_ || (size_t)n < pose_.size()) return true;
+    const int32_t m = (int32_t)pose_.size();
+    auto same = [&](int32_t i, int32_t k) {      /* rows i .. i + k - 1, bit for bit */
+      return i + k <= m && std::memcmp(&poses[i], &pose_[(size_t)i], sizeof(Pose2f) * (size_t)k) == 0 &&
+             std::memcmp(&pass[i], &pass_[(size_t)i], sizeof(int32_t) * (size_t)k) == 0;
+    };
+    for (int32_t b = 0; b < n; b += 256) {      /* whole blocks first: an unchanged block costs two memcmp */
+      const int32_t e = std::min(n, b + 256);
+      if (same(b, e - b)) continue;
+      for (int32_t i = b; i < e; ++i) {
+        if (same(i, 1)) continue;
+        ids.push_back(i);
+        if ((double)ids.size() > kFullShare * n) return true;
+        flat.insert(flat.end(), {poses[i].x, poses[i].y, poses[i].theta});
+        ids_pass.push_back(pass[i]);
+      }
+    }
+    return false;
+  }
+  /* after the table was sent: the whole vector (full) or the rows diff() listed */
+  void commit(const Pose2f *poses, const int32_t *pass, int32_t n, bool full, const std::vector<int32_t> &ids) {
+    if (full) {
+      pose_.assign(poses, poses + n); pass_.assign(pass, pass + n);
+    } else {
+      pose_.resize((size_t)n); pass_.resize((size_t)n);
+      for (int32_t i : ids) { pose_[(size_t)i] = poses[i]; pass_[(size_t)i] = pass[i]; }
+    }
+    valid_ = true;
+  }
+  void clear() { valid_ = false; pose_.clear(); pass_.clear(); }
+
+ private:
+  bool valid_ = false;
+  std::vector<Pose2f> pose_;
+  std::vector<int32_t> pass_;
+};
+
+inline std::vector<float> flatten(const Pose2f *poses, size_t n) {
+  std::vector<float> flat(n * 3);
+  for (size_t i = 0; i < n; ++i) { flat[3 * i] = poses[i].x; flat[3 * i + 1] = poses[i].y; flat[3 * i + 2] = poses[i].theta; }
+  return flat;
+}
 
 class ScanMatcher {
  public:
@@ -120,6 +177,37 @@ class ScanMatcher {
     for (const Cloud &c : clouds) { all.insert(all.end(), c.begin(), c.end()); off.push_back((int64_t)all.size()); }
     check(dpgicp_append_scans(ctx_, all.data(), sizeof(PointXYZ), off.data(), (int32_t)clouds.size()),
           "dpgicp_append_scans");
+  }
+  /* node ids[k] takes poses[k] and pass[k]; the table then holds n_nodes nodes (dpgicp_update_nodes) */
+  void updateNodes(int32_t n_nodes, const std::vector<int32_t> &ids, const std::vector<Pose2f> &poses,
+                   const std::vector<int32_t> &pass) {
+    if (poses.size() != ids.size() || pass.size() != ids.size()) throw std::runtime_error("updateNodes: length mismatch");
+    mirror_.clear();
+    const std::vector<float> flat = flatten(poses.data(), poses.size());
+    check(dpgicp_update_nodes(ctx_, n_nodes, ids.data(), flat.data(), pass.data(), (int32_t)ids.size()), "dpgicp_update_nodes");
+  }
+  /* the whole estimate vector after calculateEstimate(): only the rows that changed since the last syncNodes, and the
+   * new ones, go to the device; the first call, or one where most rows changed, sends the whole table.  The diff is
+   * taken against what the last syncNodes sent, so syncNodes (or updateNodes, after which the next syncNodes sends
+   * everything) must be the only writer of the table: dpgicp_set_nodes / dpgicp_update_nodes called on ctx()
+   * directly are not seen, and the next syncNodes would diff against a stale table. */
+  void syncNodes(const Pose2f *poses, const int32_t *pass, int32_t n_nodes) {
+    std::vector<int32_t> ids, ids_pass;
+    std::vector<float> flat;
+    const bool full = mirror_.diff(poses, pass, n_nodes, ids, flat, ids_pass);
+    mirror_.clear();
+    if (full) {
+      const std::vector<float> all = flatten(poses, (size_t)n_nodes);
+      check(dpgicp_set_nodes(ctx_, all.data(), pass, n_nodes), "dpgicp_set_nodes");
+    } else {
+      check(dpgicp_update_nodes(ctx_, n_nodes, ids.data(), flat.data(), ids_pass.data(), (int32_t)ids.size()),
+            "dpgicp_update_nodes");
+    }
+    mirror_.commit(poses, pass, n_nodes, full, ids);
+  }
+  void syncNodes(const std::vector<Pose2f> &poses, const std::vector<int32_t> &pass) {
+    if (pass.size() != poses.size()) throw std::runtime_error("syncNodes: length mismatch");
+    syncNodes(poses.data(), pass.data(), (int32_t)poses.size());
   }
   /* node poses -> (source, target) list of one reoptimize() */
   void enumeratePairs(const std::vector<Pose2f> &poses, const std::vector<int32_t> &pass, float same_pass_radius,
@@ -212,6 +300,7 @@ class ScanMatcher {
   }
   dpgicp_ctx *ctx_ = nullptr;
   dpgicp_params params_{};
+  NodeMirror mirror_;
 };
 
 /* ------------------------------------------------------------------------------------------------
@@ -258,9 +347,34 @@ class MultiGpuScanMatcher {
   }
   /* node estimates (DpgNode::getEstimatedPosition) and pass numbers; node k owns scan k */
   void setNodes(const std::vector<Pose2f> &poses, const std::vector<int32_t> &pass) {
-    std::vector<float> flat(poses.size() * 3);
-    for (size_t i = 0; i < poses.size(); ++i) { flat[3 * i] = poses[i].x; flat[3 * i + 1] = poses[i].y; flat[3 * i + 2] = poses[i].theta; }
+    mirror_.clear();
+    const std::vector<float> flat = flatten(poses.data(), poses.size());
     each([&](int r) { return dpgicp_set_nodes(ctx_[(size_t)r], flat.data(), pass.data(), (int32_t)poses.size()); }, "dpgicp_set_nodes");
+  }
+  /* ScanMatcher::updateNodes / syncNodes on every context (syncNodes: the same only-writer rule, for every ctx(r)) */
+  void updateNodes(int32_t n_nodes, const std::vector<int32_t> &ids, const std::vector<Pose2f> &poses,
+                   const std::vector<int32_t> &pass) {
+    if (poses.size() != ids.size() || pass.size() != ids.size()) throw std::runtime_error("updateNodes: length mismatch");
+    mirror_.clear();
+    const std::vector<float> flat = flatten(poses.data(), poses.size());
+    each([&](int r) { return dpgicp_update_nodes(ctx_[(size_t)r], n_nodes, ids.data(), flat.data(), pass.data(), (int32_t)ids.size()); },
+         "dpgicp_update_nodes");
+  }
+  void syncNodes(const std::vector<Pose2f> &poses, const std::vector<int32_t> &pass) {
+    if (pass.size() != poses.size()) throw std::runtime_error("syncNodes: length mismatch");
+    const int32_t n = (int32_t)poses.size();
+    std::vector<int32_t> ids, ids_pass;
+    std::vector<float> flat;
+    const bool full = mirror_.diff(poses.data(), pass.data(), n, ids, flat, ids_pass);
+    mirror_.clear();
+    if (full) {
+      flat = flatten(poses.data(), poses.size());
+      each([&](int r) { return dpgicp_set_nodes(ctx_[(size_t)r], flat.data(), pass.data(), n); }, "dpgicp_set_nodes");
+    } else {
+      each([&](int r) { return dpgicp_update_nodes(ctx_[(size_t)r], n, ids.data(), flat.data(), ids_pass.data(), (int32_t)ids.size()); },
+           "dpgicp_update_nodes");
+    }
+    mirror_.commit(poses.data(), pass.data(), n, full, ids);
   }
   /* the caller's pair list (DPGICP_ENUM_REOPTIMIZE / _ONLINE) built on every device; returns the global pair count */
   int64_t enumeratePairs(int32_t mode, float same_pass_radius, float other_pass_radius) {
@@ -321,6 +435,7 @@ class MultiGpuScanMatcher {
   std::vector<int64_t> local_;
   int64_t n_total_ = 0;
   dpgicp_params params_{};
+  NodeMirror mirror_;
 };
 
 }  // namespace dpgicp_shim
