@@ -98,6 +98,8 @@ struct Batch {
   int32_t max_scan = -1;         /* device-enumerated lists: highest scan (= node) index used; -1 = validated on the host */
 };
 
+struct StageTarget { int warps, csize; };      /* of the stage chain: warps per CTA, CTAs per cluster */
+
 struct Nodes {                   /* pose-graph node estimates on the device (dpgicp_set_nodes, dpgicp_update_nodes) */
   DevBuf xy, aux, pass;          /* float2 (x, y); float4 (theta, cosf(-theta), sinf(-theta), 0); int32 pass */
   DevBuf boxes;                  /* index-order box hierarchy, levels back to back, each sized for `cap` nodes */
@@ -153,14 +155,12 @@ struct dpgicp_ctx {
   int64_t gather_n = 0;
   int gather_world = 0, gather_rank = 0;
   void *gather_peer[DPGICP_MAX_GATHER_RANKS] = {nullptr};
-  int max_stages = 5;
-  std::vector<int> chain, chain_cluster;     /* DPGICP_CHAIN: target warps (and "x<cluster size>") per stage (development knob) */
+  StageTarget chain[5];                      /* DPGICP_CHAIN: target warps (and "x<cluster size>") per stage (development knob) */
+  int n_chain = 0;
   DevBuf d_bad;                              /* int: range flag of the store writes */
   HostBuf h_stage;                           /* staging for subset uploads from pageable memory */
   double handover_factor = 2.0;              /* DPGICP_HANDOVER="f[,fc]": a stage hands over once at most f x (CTAs of the next stage) pairs are */
   double handover_cluster = 1.0;             /* left; fc x (clusters) when the next stage runs clusters (development knob; 0 = plain queue-dry rule) */
-  int force_warps = 0;
-  int force_ctas_per_sm = 0;
   uint64_t launches = 0;
   std::string err;
 };
@@ -255,88 +255,95 @@ float gate_threshold(const dpgicp_params *p) {
   return f;
 }
 
-template <int WARPS, int SEARCH, int CSIZE>
-int launch_icp_t(dpgicp_ctx *ctx, cudaStream_t stream, const KernelParams &kp, size_t smem, int64_t max_items, int nw, int *grid_out) {
-  auto kern = icp_pairs_kernel<WARPS, SEARCH, CSIZE>;
-  const void *kfn = reinterpret_cast<const void *>(kern);
-  /* the dynamic shared-memory opt-in and the occupancy of a shape do not change between runs: set / query once */
+using IcpKernel = void (*)(KernelParams);
+
+/* the icp_pairs_kernel instantiation of a stage: nw warps per CTA run on the one with the next power-of-two register
+ * budget; clusters (the last stage only) use the 16-warp budget */
+template <int SEARCH>
+IcpKernel icp_kernel_w(int nw, int csize, bool resume) {
+  /* first stage of large scans: 12 warps with the 80-register budget so that two CTAs share an SM */
+  if (csize == 1 && !resume && nw > 8 && nw <= 12) return icp_pairs_kernel<12, SEARCH, 1>;
+  if (csize == 2) return icp_pairs_kernel<16, SEARCH, 2>;
+  if (csize == 4) return icp_pairs_kernel<16, SEARCH, 4>;
+  if (nw <= 1) return icp_pairs_kernel<1, SEARCH, 1>;
+  if (nw <= 2) return icp_pairs_kernel<2, SEARCH, 1>;
+  if (nw <= 4) return icp_pairs_kernel<4, SEARCH, 1>;
+  if (nw <= 8) return icp_pairs_kernel<8, SEARCH, 1>;
+  return icp_pairs_kernel<16, SEARCH, 1>;
+}
+
+IcpKernel icp_kernel(int search, int nw, int csize, bool resume) {
+  if (search == DPGICP_SEARCH_PROJECTIVE) return icp_kernel_w<DPGICP_SEARCH_PROJECTIVE>(nw, csize, resume);
+  if (search == DPGICP_SEARCH_PRUNED) return icp_kernel_w<DPGICP_SEARCH_PRUNED>(nw, csize, resume);
+  if (search == kSearchPrunedFlat) return icp_kernel_w<kSearchPrunedFlat>(nw, csize, resume);
+  if (search == kSearchPrunedStock) return icp_kernel_w<kSearchPrunedStock>(nw, csize, resume);
+  if (search == kSearchPrunedFlatStock) return icp_kernel_w<kSearchPrunedFlatStock>(nw, csize, resume);
+  return icp_kernel_w<DPGICP_SEARCH_BRUTE>(nw, csize, resume);
+}
+
+/* one stage of the chain: a persistent grid of `units` CTAs (csize 1) or clusters of csize CTAs, `warps` warps each */
+struct Stage {
+  IcpKernel kern;
+  int warps, csize;
+  size_t smem;
+  int64_t units;
+  long long handover;      /* KernelParams::handover (0 on the last stage, which never suspends) */
+};
+
+cudaLaunchConfig_t launch_config(const Stage &s, int64_t grid, cudaStream_t stream, cudaLaunchAttribute *cluster) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3((unsigned)grid, 1, 1);
+  cfg.blockDim = dim3((unsigned)s.warps * 32, 1, 1);
+  cfg.dynamicSmemBytes = s.smem;
+  cfg.stream = stream;
+  cluster->id = cudaLaunchAttributeClusterDimension;
+  cluster->val.clusterDim.x = s.csize; cluster->val.clusterDim.y = 1; cluster->val.clusterDim.z = 1;
+  cfg.attrs = cluster;
+  cfg.numAttrs = s.csize > 1 ? 1 : 0;
+  return cfg;
+}
+
+/* resident CTAs (csize 1) or clusters of stage s's kernel on the whole device.  The dynamic shared-memory opt-in and the
+ * occupancy of a shape do not change between runs: set / queried once. */
+int units(dpgicp_ctx *ctx, const Stage &s, int64_t *out) {
+  const void *kfn = reinterpret_cast<const void *>(s.kern);
   {
     /* the attribute belongs to (device, function), not to a context: several contexts of one process share it, so it is
      * tracked process-wide and only ever raised */
     std::lock_guard<std::mutex> lock(g_optin_mutex);
     size_t &have = g_smem_optin[std::make_pair(ctx->device, kfn)];
-    if (have < smem) {
-      CU_TRY(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      have = smem;
+    if (have < s.smem) {
+      CU_TRY(ctx, cudaFuncSetAttribute(s.kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s.smem));
+      have = s.smem;
     }
   }
-  cudaLaunchConfig_t cfg = {};
-  cfg.blockDim = dim3((unsigned)nw * 32, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CSIZE; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = CSIZE > 1 ? 1 : 0;
-  int64_t units = 0;                        /* resident CTAs (CSIZE == 1) or clusters on the whole device */
-  const auto key = std::make_tuple(kfn, nw, smem);
+  const auto key = std::make_tuple(kfn, s.warps, s.smem);
   auto occ = ctx->occupancy.find(key);
-  if (occ != ctx->occupancy.end()) {
-    units = occ->second;
-  } else if (CSIZE > 1) {
-    cfg.gridDim = dim3((unsigned)(ctx->sm_count / CSIZE) * CSIZE, 1, 1);
-    int n_clusters = 0;
-    CU_TRY(ctx, cudaOccupancyMaxActiveClusters(&n_clusters, kern, &cfg));
-    if (n_clusters < 1) return fail(ctx, DPGICP_E_TOOBIG, "no cluster of this shape fits the device");
-    units = n_clusters;
-    ctx->occupancy[key] = n_clusters;
-  } else {
-    int per_sm = 0;
-    CU_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, nw * 32, smem));
-    if (per_sm < 1) return fail(ctx, DPGICP_E_TOOBIG, "scan too large for one CTA's shared memory");
-    units = (int64_t)ctx->sm_count * per_sm;
-    ctx->occupancy[key] = (int)units;
+  if (occ == ctx->occupancy.end()) {
+    int n = 0;
+    if (s.csize > 1) {
+      cudaLaunchAttribute cluster;
+      const cudaLaunchConfig_t cfg = launch_config(s, (ctx->sm_count / s.csize) * s.csize, nullptr, &cluster);
+      CU_TRY(ctx, cudaOccupancyMaxActiveClusters(&n, s.kern, &cfg));
+      if (n < 1) return fail(ctx, DPGICP_E_TOOBIG, "no cluster of this shape fits the device");
+    } else {
+      CU_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, s.kern, s.warps * 32, s.smem));
+      if (n < 1) return fail(ctx, DPGICP_E_TOOBIG, "scan too large for one CTA's shared memory");
+      n *= ctx->sm_count;
+    }
+    occ = ctx->occupancy.emplace(key, n).first;
   }
-  if (CSIZE == 1 && ctx->force_ctas_per_sm > 0) units = std::min<int64_t>(units, (int64_t)ctx->sm_count * ctx->force_ctas_per_sm);
-  /* persistent grid: a whole number of resident CTAs per SM (or clusters), never more than work items */
-  if (units > max_items) units = max_items;
-  if (units < 1) units = 1;
-  const int64_t grid = units * CSIZE;
-  if (grid_out) {
-    if (*grid_out < 0) { *grid_out = (int)units; return DPGICP_OK; }      /* query only */
-    *grid_out = (int)units;
-  }
-  cfg.gridDim = dim3((unsigned)grid, 1, 1);
-  CU_TRY(ctx, cudaLaunchKernelEx(&cfg, kern, kp));
-  ctx->launches++;
-  CU_TRY(ctx, cudaGetLastError());
+  *out = occ->second;
   return DPGICP_OK;
 }
 
-/* nw warps per CTA run on the instantiation with the next power-of-two register budget; clusters (the last
- * stage only) use the 16-warp budget */
-template <int SEARCH>
-int launch_icp_w(dpgicp_ctx *ctx, cudaStream_t stream, int nw, int csize, const KernelParams &kp, size_t smem, int64_t n, int *grid_out) {
-  nw = std::max(1, std::min(nw, 16));
-  /* first stage of large scans: 12 warps with the 80-register budget so that two CTAs share an SM */
-  if (csize == 1 && !kp.resume && nw > 8 && nw <= 12) return launch_icp_t<12, SEARCH, 1>(ctx, stream, kp, smem, n, nw, grid_out);
-  if (csize == 2) return launch_icp_t<16, SEARCH, 2>(ctx, stream, kp, smem, n, nw, grid_out);
-  if (csize == 4) return launch_icp_t<16, SEARCH, 4>(ctx, stream, kp, smem, n, nw, grid_out);
-  if (nw <= 1) return launch_icp_t<1, SEARCH, 1>(ctx, stream, kp, smem, n, 1, grid_out);
-  if (nw <= 2) return launch_icp_t<2, SEARCH, 1>(ctx, stream, kp, smem, n, nw, grid_out);
-  if (nw <= 4) return launch_icp_t<4, SEARCH, 1>(ctx, stream, kp, smem, n, nw, grid_out);
-  if (nw <= 8) return launch_icp_t<8, SEARCH, 1>(ctx, stream, kp, smem, n, nw, grid_out);
-  return launch_icp_t<16, SEARCH, 1>(ctx, stream, kp, smem, n, nw, grid_out);
-}
-
-int launch_stage(dpgicp_ctx *ctx, cudaStream_t stream, int search, int nw, int csize, const KernelParams &kp, size_t smem, int64_t n, int *grid_out) {
-  if (search == DPGICP_SEARCH_PROJECTIVE) return launch_icp_w<DPGICP_SEARCH_PROJECTIVE>(ctx, stream, nw, csize, kp, smem, n, grid_out);
-  if (search == DPGICP_SEARCH_PRUNED) return launch_icp_w<DPGICP_SEARCH_PRUNED>(ctx, stream, nw, csize, kp, smem, n, grid_out);
-  if (search == kSearchPrunedFlat) return launch_icp_w<kSearchPrunedFlat>(ctx, stream, nw, csize, kp, smem, n, grid_out);
-  if (search == kSearchPrunedStock) return launch_icp_w<kSearchPrunedStock>(ctx, stream, nw, csize, kp, smem, n, grid_out);
-  if (search == kSearchPrunedFlatStock) return launch_icp_w<kSearchPrunedFlatStock>(ctx, stream, nw, csize, kp, smem, n, grid_out);
-  return launch_icp_w<DPGICP_SEARCH_BRUTE>(ctx, stream, nw, csize, kp, smem, n, grid_out);
+int launch(dpgicp_ctx *ctx, cudaStream_t stream, const Stage &s, const KernelParams &kp) {
+  cudaLaunchAttribute cluster;
+  const cudaLaunchConfig_t cfg = launch_config(s, s.units * s.csize, stream, &cluster);
+  CU_TRY(ctx, cudaLaunchKernelEx(&cfg, s.kern, kp));
+  ctx->launches++;
+  CU_TRY(ctx, cudaGetLastError());
+  return DPGICP_OK;
 }
 
 /* warps per CTA close to `target` that split `tiles` 32-point tiles evenly (every warp gets
@@ -347,6 +354,54 @@ int balanced_warps(int tiles, int target, int csize = 1) {
   const int per_warp = (tiles + slots - 1) / slots;
   const int warps_total = (tiles + per_warp - 1) / per_warp;
   return std::max(1, (warps_total + csize - 1) / csize);
+}
+
+/* st[0 .. *n_stages) = the stage chain of `count` pairs of n_cap-point clouds.  trim: a rejector runs (its block-wide
+ * select does not span a cluster); one_stage: the correspondences hook. */
+int plan_stages(dpgicp_ctx *ctx, int search, int n_cap, int64_t count, bool trim, bool one_stage, Stage (&st)[5],
+                int *n_stages) {
+  const int tiles = n_cap / kTile;
+  /* 34 tiles (1081 beams) -> 4, 7, 12 warps per CTA, then clusters of 4 CTAs x 9 warps (one tile per warp on four
+   * SMs) for the last pairs: measured per-pass latency of one pair 28.7 / 17.9 / 11.4 / 6.3 us */
+  const int w0 = n_cap <= 512 ? 2 : (n_cap <= 2048 ? 4 : 12);
+  const StageTarget defaults[4] = {{w0, 1}, {std::min(16, 2 * w0), 1}, {16, 1}, {16, 4}};
+  const StageTarget *targets = ctx->n_chain ? ctx->chain : defaults;
+  const int n_targets = ctx->n_chain ? ctx->n_chain : (tiles >= 16 && !trim) ? 4 : 3;
+  /* widths balanced against the tile count, a cluster only on the last stage (it never suspends), each wider than the
+   * one before: narrow CTAs for the bulk of the batch, wider ones for the pairs still running when a queue runs dry */
+  int n = 0;
+  for (int k = 0; k < (one_stage ? 1 : n_targets); ++k) {
+    const int cs = k > 0 && k + 1 == n_targets && !trim ? targets[k].csize : 1;
+    const int w = balanced_warps(tiles, targets[k].warps, cs);
+    if (n == 0 || w * cs > st[n - 1].warps * st[n - 1].csize)
+      st[n++] = {icp_kernel(search, w, cs, k > 0), w, cs, smem_bytes(n_cap, search == DPGICP_SEARCH_PROJECTIVE, trim, w), 0, 0};
+  }
+  /* the hand-over bound towards stage s of cap units: DPGICP_HANDOVER's factor x its clusters (default 1) or CTAs
+   * (default 2; the next stage's own queue-dry rule then takes over).  Factor 0: the plain queue-dry rule, no drop. */
+  const auto bound = [&](const Stage &s, int64_t cap) {
+    if (ctx->handover_factor <= 0.0) return (long long)1 << 40;
+    return (long long)std::ceil((s.csize > 1 ? ctx->handover_cluster : ctx->handover_factor) * (double)cap);
+  };
+  int64_t cap;
+  /* Small batches (the online caller's handful of pairs, a single runIcp-shaped call): a stage whose WHOLE batch is within
+   * the hand-over bound towards the next stage would see its queue dry at once and suspend every pair after its first
+   * pass — a launch, a state round trip through HBM and a re-staging for nothing.  Start the chain at the first stage that
+   * would keep its pairs (the last one at the latest). */
+  while (n > 1 && ctx->handover_factor > 0.0) {
+    if (const int rc = units(ctx, st[1], &cap)) return rc;
+    if (count > bound(st[1], cap)) break;
+    std::copy(st + 1, st + n, st);
+    --n;
+  }
+  st[0].kern = icp_kernel(search, st[0].warps, st[0].csize, false);      /* the first stage takes fresh pairs */
+  /* persistent grids, never more than work items: stage 0's pairs, then the pairs the stage before can suspend */
+  for (int k = 0; k < n; ++k) {
+    if (const int rc = units(ctx, st[k], &cap)) return rc;
+    if (k > 0) st[k - 1].handover = bound(st[k], cap);
+    st[k].units = std::max<int64_t>(1, std::min(cap, k > 0 ? st[k - 1].units : count));
+  }
+  *n_stages = n;
+  return DPGICP_OK;
 }
 
 /* the stage chain of batch b over store st, on slot s's stream with s's queue cells and state buffers (b is s's batch, or
@@ -409,8 +464,6 @@ int launch_icp(dpgicp_slot *s, const Store &st, const Batch &b, const dpgicp_par
   kp.sensor_x = p->sensor_x;
   kp.sensor_y = p->sensor_y;
   const bool trim = p->outlier_mode != DPGICP_OUTLIER_NONE;
-  /* shared memory of a stage: the reduction scratch grows with the CTA width */
-  auto smem_of = [&](int warps) { return smem_bytes(n_cap, p->search == DPGICP_SEARCH_PROJECTIVE, trim, warps); };
   /* clouds of at most 32 groups: the pruned search's flat instantiation (one candidate round, no upper box level) */
   int search = p->search;
   if (search == DPGICP_SEARCH_PRUNED) {
@@ -419,62 +472,20 @@ int launch_icp(dpgicp_slot *s, const Store &st, const Batch &b, const dpgicp_par
     const bool flat = n_cap / kGroup <= kFlatMaxGroups;
     search = stock ? (flat ? kSearchPrunedFlatStock : kSearchPrunedStock) : (flat ? kSearchPrunedFlat : DPGICP_SEARCH_PRUNED);
   }
-
-  /* stage widths (warps per pair): narrow CTAs for the bulk of the batch, wider ones for the pairs
-   * still running when a stage's queue runs dry; each width is balanced against the tile count */
-  const int tiles = n_cap / kTile;
-  int w0 = ctx->force_warps;
-  if (w0 <= 0) w0 = n_cap <= 512 ? 2 : (n_cap <= 2048 ? 4 : 12);
-  struct StageShape { int warps, csize; };
-  /* 34 tiles (1081 beams) -> 4, 7, 12 warps per CTA, then clusters of 4 CTAs x 9 warps (one tile per warp on four
-   * SMs) for the last pairs: measured per-pass latency of one pair 28.7 / 17.9 / 11.4 / 6.3 us */
-  StageShape targets[5] = {{w0, 1}, {std::min(16, 2 * w0), 1}, {16, 1}, {16, 4}, {16, 1}};
-  int n_targets = (tiles >= 16 && !trim) ? 4 : 3;      /* the rejector's block-wide select does not span a cluster */
-  if (!ctx->chain.empty()) {
-    n_targets = 0;
-    for (size_t k = 0; k < ctx->chain.size() && n_targets < 5; ++k)
-      targets[n_targets++] = {ctx->chain[k], trim ? 1 : ctx->chain_cluster[k]};
-  }
-  StageShape shapes[5] = {{balanced_warps(tiles, targets[0].warps), 1}, {0, 1}, {0, 1}, {0, 1}, {0, 1}};
-  int n_stages = 1;
-  if (corr_out == nullptr) {
-    for (int k = 1; k < n_targets && n_stages < ctx->max_stages; ++k) {
-      /* a cluster of CTAs per pair is only used for the last stage (it never suspends) */
-      const int cs = (k + 1 == n_targets || n_stages + 1 == ctx->max_stages) ? targets[k].csize : 1;
-      const int w = balanced_warps(tiles, targets[k].warps, cs);
-      if (w * cs <= shapes[n_stages - 1].warps * shapes[n_stages - 1].csize) continue;
-      shapes[n_stages++] = {w, cs};
-    }
-  }
-  /* Small batches (the online caller's handful of pairs, a single runIcp-shaped call): a stage whose WHOLE batch is within
-   * the hand-over bound towards the next stage would see its queue dry at once and suspend every pair after its first
-   * pass — a launch, a state round trip through HBM and a re-staging for nothing.  Start the chain at the first stage that
-   * would keep its pairs (the last one at the latest). */
-  while (n_stages > 1 && ctx->handover_factor > 0.0) {
-    int next_units = -1;
-    KernelParams kq = kp;
-    kq.resume = 1;
-    int rcq = launch_stage(ctx, stream, search, shapes[1].warps, shapes[1].csize, kq, smem_of(shapes[1].warps), (int64_t)1 << 40, &next_units);
-    if (rcq) return rcq;
-    const long long bound = (long long)std::ceil((shapes[1].csize > 1 ? ctx->handover_cluster : ctx->handover_factor) * (double)next_units);
-    if (count > bound) break;
-    for (int k = 1; k < n_stages; ++k) shapes[k - 1] = shapes[k];
-    --n_stages;
-  }
+  Stage stages[5];
+  int n_stages = 0;
+  int rc = plan_stages(ctx, search, n_cap, count, trim, corr_out != nullptr, stages, &n_stages);
+  if (rc) return rc;
   CU_TRY(ctx, cudaMemsetAsync(q, 0, 32 * sizeof(unsigned long long), stream));
-  int grid_prev = 0;
   const bool timing = s->stage_timing && corr_out == nullptr;
   if (timing) { s->last_stages = n_stages; CU_TRY(ctx, cudaEventRecord(s->stage_ev[0], stream)); }
   if (n_stages > 1) {
     /* every stage can suspend at most one pair per CTA: size the state slots for stage 0's grid */
-    int g0 = -1;
-    int rc = launch_stage(ctx, stream, search, shapes[0].warps, shapes[0].csize, kp, smem_of(shapes[0].warps), count, &g0);
-    if (rc) return rc;
+    kp.slot_cap = stages[0].units;
     for (int k = 0; k < 2; ++k) {
-      if ((rc = reserve(ctx, s->state[k], (size_t)g0 * (size_t)kp.slot_bytes))) return rc;
-      if ((rc = reserve(ctx, s->susp[k], (size_t)g0 * sizeof(long long)))) return rc;
+      if ((rc = reserve(ctx, s->state[k], (size_t)kp.slot_cap * (size_t)kp.slot_bytes))) return rc;
+      if ((rc = reserve(ctx, s->susp[k], (size_t)kp.slot_cap * sizeof(long long)))) return rc;
     }
-    kp.slot_cap = g0;
   }
   for (int sidx = 0; sidx < n_stages; ++sidx) {
     KernelParams ks = kp;
@@ -486,27 +497,15 @@ int launch_icp(dpgicp_slot *s, const Store &st, const Batch &b, const dpgicp_par
       ks.state_in = (const unsigned char *)s->state[(sidx - 1) & 1].p;
     }
     ks.finished = q + 24 + sidx;
+    ks.handover = stages[sidx].handover;
     if (sidx + 1 < n_stages) {
-      /* hand over once the next stage could run all that is left at once (clusters: exactly; CTAs: a third more,
-       * the next stage's own queue-dry rule then takes over) */
-      int next_units = -1;
-      KernelParams kq = kp;
-      kq.resume = 1;                        /* occupancy query for the shape the next stage will really use */
-      int rcq = launch_stage(ctx, stream, search, shapes[sidx + 1].warps, shapes[sidx + 1].csize, kq, smem_of(shapes[sidx + 1].warps), (int64_t)1 << 40, &next_units);
-      if (rcq) return rcq;
-      ks.handover = (long long)std::ceil((shapes[sidx + 1].csize > 1 ? ctx->handover_cluster : ctx->handover_factor) * (double)next_units);
-      if (ctx->handover_factor <= 0.0) ks.handover = (long long)1 << 40;      /* development: the plain queue-dry rule */
       ks.out_count = reinterpret_cast<unsigned int *>(q + 6 + (sidx & 1));
       ks.susp_out = (long long *)s->susp[sidx & 1].p;
       ks.state_out = (unsigned char *)s->state[sidx & 1].p;
       if (sidx >= 2)      /* the count cell is reused by stage sidx: clear it after stage sidx-1 consumed it */
         CU_TRY(ctx, cudaMemsetAsync(q + 6 + (sidx & 1), 0, sizeof(unsigned long long), stream));
     }
-    int grid = 0;
-    const int64_t max_items = sidx == 0 ? count : (int64_t)grid_prev;
-    int rc = launch_stage(ctx, stream, search, shapes[sidx].warps, shapes[sidx].csize, ks, smem_of(shapes[sidx].warps), max_items, &grid);
-    if (rc) return rc;
-    grid_prev = grid;
+    if ((rc = launch(ctx, stream, stages[sidx], ks))) return rc;
     if (timing) CU_TRY(ctx, cudaEventRecord(s->stage_ev[sidx + 1], stream));
   }
   return DPGICP_OK;
@@ -1170,19 +1169,16 @@ int dpgicp_create(int device, dpgicp_ctx **out) {
     return fail(nullptr, DPGICP_E_CUDA, cudaGetErrorString(e));
   }
   ctx->stream = ctx->own_stream;
-  if (const char *w = std::getenv("DPGICP_WARPS")) ctx->force_warps = std::atoi(w);
-  if (const char *c = std::getenv("DPGICP_CTAS_PER_SM")) ctx->force_ctas_per_sm = std::atoi(c);
   if (const char *c = std::getenv("DPGICP_HANDOVER")) {
     ctx->handover_factor = std::max(0.0, std::atof(c));
     if (const char *q = std::strchr(c, ',')) ctx->handover_cluster = std::max(0.0, std::atof(q + 1));
   }
-  if (const char *c = std::getenv("DPGICP_STAGES")) ctx->max_stages = std::max(1, std::min(5, std::atoi(c)));
   if (const char *c = std::getenv("DPGICP_CHAIN")) {
-    for (const char *q = c; *q;) {            /* e.g. "4,8,16,9x2": the last stage as clusters of 2 CTAs x 9 warps */
-      ctx->chain.push_back(std::max(1, std::atoi(q)));
+    for (const char *q = c; *q && ctx->n_chain < 5;) {      /* e.g. "4,8,16,9x2": the last stage as clusters of 2 CTAs x 9 warps */
+      const int w = std::max(1, std::atoi(q));
       int cs = 1;
       while (*q && *q != ',') { if (*q == 'x') cs = std::atoi(q + 1); ++q; }
-      ctx->chain_cluster.push_back(cs == 2 || cs == 4 ? cs : 1);
+      ctx->chain[ctx->n_chain++] = {w, cs == 2 || cs == 4 ? cs : 1};
       if (*q == ',') ++q;
     }
   }

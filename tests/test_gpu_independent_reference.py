@@ -102,18 +102,13 @@ def test_rejector_whole_runs_under_forced_chains_equal_oracle(gpu_matcher, monke
     runs = [Params.defaults(downsample_divisor=1, search=SEARCH_PRUNED, cov_mode=COV_CENSI_CORR, max_iterations=60,
                             outlier_mode=m, outlier_param=q) for m, q in ((OUTLIER_TRIMMED, 0.8), (OUTLIER_MEDIAN, 0.5), (OUTLIER_MEDIAN, 1.5))]
     refs = [O.run_batch(pts, off, src, tgt, guess, p, fast=1, threads=0)[0] for p in runs]
-    for stages, warps, chain in ((1, 1, None), (1, 32, None), (2, 0, "1,32"), (4, 0, "4,8,16,9x4"), (2, 0, "2,5x2")):
-        monkeypatch.setenv("DPGICP_STAGES", str(stages))
-        monkeypatch.setenv("DPGICP_WARPS", str(warps))
-        if chain:
-            monkeypatch.setenv("DPGICP_CHAIN", chain)
-        else:
-            monkeypatch.delenv("DPGICP_CHAIN", raising=False)
+    for chain in ("1", "32", "1,32", "4,8,16,9x4", "2,5x2"):
+        monkeypatch.setenv("DPGICP_CHAIN", chain)
         with ScanMatcher(0) as sm:
             sm.upload_scans(pts, off)
             for p, ref in zip(runs, refs):
                 got = sm.submit_pairs(src, tgt, guess, p)
-                assert_records_match(got, ref, f"chain {stages}/{warps}/{chain} outlier {p.outlier_mode}/{p.outlier_param}")
+                assert_records_match(got, ref, f"chain {chain} outlier {p.outlier_mode}/{p.outlier_param}")
 
 
 # ---- one pass against the float64 step -----------------------------------------------------------------------------------

@@ -658,27 +658,19 @@ def test_staged_chain_equals_single_stage(gpu_matcher, monkeypatch):
     p = Params.defaults(downsample_divisor=1, cov_mode=COV_CENSI_CORR)
     gpu_matcher.upload_ranges(wl.ranges, wl.scanner)
     want = gpu_matcher.submit_pairs(wl.src_idx, wl.tgt_idx, wl.guess, p)
-    for stages, warps, chain in ((1, 4, None), (2, 2, None), (3, 1, None), (3, 8, None), (1, 16, None), (4, 0, "3,5,11,32"),
-                                 (4, 0, "4,8,16,32"), (2, 0, "1,32"), (1, 32, None),
-                                 # last stage as thread-block clusters: 2 or 4 CTAs (SMs) per pair, partial sums through DSMEM
-                                 (4, 0, "4,8,16,9x2"), (3, 0, "4,8,9x4"), (2, 0, "2,5x2"), (2, 0, "4,16x4")):
-        monkeypatch.setenv("DPGICP_STAGES", str(stages))
-        monkeypatch.setenv("DPGICP_WARPS", str(warps))
-        if chain:
-            monkeypatch.setenv("DPGICP_CHAIN", chain)
-        else:
-            monkeypatch.delenv("DPGICP_CHAIN", raising=False)
+    for chain in ("4", "2,4", "1,2,16", "8,16,16x4", "16", "3,5,11,32", "4,8,16,32", "1,32", "32",
+                  # last stage as thread-block clusters: 2 or 4 CTAs (SMs) per pair, partial sums through DSMEM
+                  "4,8,16,9x2", "4,8,9x4", "2,5x2", "4,16x4"):
+        monkeypatch.setenv("DPGICP_CHAIN", chain)
         with ScanMatcher(0) as sm:
             sm.upload_ranges(wl.ranges, wl.scanner)
             got = sm.submit_pairs(wl.src_idx, wl.tgt_idx, wl.guess, p)
-            assert got.tobytes() == want.tobytes(), (stages, warps)
+            assert got.tobytes() == want.tobytes(), chain
             c = sm.last_run_counters()
             assert c["iterations"] == int(got["iterations"].sum())
     # the hand-over rule (a stage suspends its pairs once its queue is dry AND few enough are left for the next stage)
     # only moves the moment of suspension
-    monkeypatch.setenv("DPGICP_STAGES", "5")
-    monkeypatch.setenv("DPGICP_WARPS", "0")
-    monkeypatch.delenv("DPGICP_CHAIN", raising=False)
+    monkeypatch.delenv("DPGICP_CHAIN")
     for handover in ("0", "0.5,0.5", "1.0,3.0", "4"):
         monkeypatch.setenv("DPGICP_HANDOVER", handover)
         with ScanMatcher(0) as sm:
@@ -688,15 +680,11 @@ def test_staged_chain_equals_single_stage(gpu_matcher, monkeypatch):
     # down-sampled clouds take the gather path when fresh and the contiguous path when resumed
     p5 = p.copy(downsample_divisor=5)
     want5 = gpu_matcher.submit_pairs(wl.src_idx, wl.tgt_idx, wl.guess, p5)
-    monkeypatch.delenv("DPGICP_CHAIN", raising=False)
-    monkeypatch.setenv("DPGICP_STAGES", "1")
-    monkeypatch.setenv("DPGICP_WARPS", "2")
+    monkeypatch.setenv("DPGICP_CHAIN", "2")
     with ScanMatcher(0) as sm:
         sm.upload_ranges(wl.ranges, wl.scanner)
         assert sm.submit_pairs(wl.src_idx, wl.tgt_idx, wl.guess, p5).tobytes() == want5.tobytes()
     # clusters with every covariance mode and metric, ragged and empty scans, small batches (all pairs reach the cluster stage)
-    monkeypatch.setenv("DPGICP_STAGES", "4")
-    monkeypatch.setenv("DPGICP_WARPS", "0")
     wl2 = synth.config_corridor(n_pairs=40, n_beams=721, seed=12)
     wl2.ranges[2, :] = 40.0
     wl2.ranges[4, 2:] = 40.0

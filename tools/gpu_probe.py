@@ -38,26 +38,27 @@ def main():
     else:
         wl = synth.config_loop_closure(n_pairs=n_pairs, n_scans=2000, seed=3)
     out = {}
-    combos = [(st, w, c) for st in (1, 2, 3) for w in (0, 2, 4, 8) for c in (0,)] + [(3, 4, 4), (3, 4, 3), (1, 4, 6)]
-    for stages, warps, ctas in combos:
-        os.environ["DPGICP_STAGES"] = str(stages)
-        os.environ["DPGICP_WARPS"] = str(warps)
-        os.environ["DPGICP_CTAS_PER_SM"] = str(ctas)
+    # DPGICP_CHAIN values: target warps per stage, "xC" = the last stage as clusters of C CTAs; "default" = the library's
+    for chain in ("default", "2", "4", "8", "16", "2,4", "4,8", "8,16", "2,4,16", "4,8,16", "8,16,16x4"):
+        if chain == "default":
+            os.environ.pop("DPGICP_CHAIN", None)
+        else:
+            os.environ["DPGICP_CHAIN"] = chain
         with ScanMatcher(0) as sm:
             sm.upload_ranges(wl.ranges, wl.scanner)
             sm.set_pairs(wl.src_idx, wl.tgt_idx, wl.guess)
             for search in (1, 0):
                 for div in (1, 5):
-                    if search == 0 and (stages != 3 or warps != 0):
+                    if search == 0 and chain != "default":
                         continue
                     p = Params.defaults(downsample_divisor=div, cov_mode=COV_CENSI_CORR, search=search)
                     try:
                         best, med = time_run(sm, p)
                     except Exception as e:
-                        print("ERR", stages, warps, ctas, search, div, e, flush=True)
+                        print("ERR", chain, search, div, e, flush=True)
                         continue
                     c = sm.last_run_counters()
-                    key = f"st{stages}_w{warps}_c{ctas}_s{search}_d{div}"
+                    key = f"chain{chain}_s{search}_d{div}"
                     out[key] = dict(ms=best, med=med, pairs_per_s=wl.n_pairs / best * 1e3, evals=c["distance_evals"],
                                     tests=c["box_tests"])
                     print(key, json.dumps(out[key]), flush=True)
